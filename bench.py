@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- CoMap hot path on B200: site-pairs scored per second, mapping + null included.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[3], SURVEY.md s8d "config 4"): synthetic 5,000-site x
@@ -346,6 +346,21 @@ def table_checksum(cols, n):
         return int(h.sum(dtype=np.uint64))
 
 
+DUMP_PAIR_ROWS = 1 << 19        # 9 float64 columns of 4 MB each + the 8 MB null: 44 MB of the 64 MB allowed
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy in float64 (the integer columns are exact in it)."""
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("bench.py: %d bytes of outputs exceed the %d-byte dump limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args, cfg):
     import torch
     import torch.distributed as dist
@@ -354,6 +369,8 @@ def run_ours(args, cfg):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs needs one process (each rank holds only its shard of the pair table)")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device; comap_b200 has no CPU fallback")
     torch.cuda.set_device(local)
@@ -434,6 +451,8 @@ def run_ours(args, cfg):
         for _ in range(max(3, args.warmup)):
             n_rows = step_resident()
         step_e2e()
+        if args.dump_outputs:
+            dump_rows = np.sort(np.random.default_rng(0).choice(n_rows, min(n_rows, DUMP_PAIR_ROWS), replace=False))
 
         sampler = ClockSampler(local)
         if rank == 0:
@@ -441,6 +460,16 @@ def run_ours(args, cfg):
         l0 = ctx.launch_count()
         ms = timed(step_resident, args.steps)              # the timed region: no per-kernel events inside
         launches = ctx.launch_count() - l0
+        if args.dump_outputs:
+            # what the last timed step left on the device: the pair table (sampled rows, in the reference's order)
+            # and the binned null distribution; written once the measurements are over
+            for k in range(len(api.Context.COLS)):
+                ctx.pairs_fetch(k, cols_pin[k])
+            ctx.sync()
+            g = ctx.null_get()
+            dumped = {"pairs_" + c: cols_pin[k][dump_rows] for k, c in enumerate(api.Context.COLS)}
+            dumped.update(pairs_row=dump_rows, null_sorted=g["sorted"], null_bin_offsets=g["bin_offsets"],
+                          null_nmax=np.array([g["nmax"]]))
         ms_e2e = timed(step_e2e, args.steps)
         clocks = sampler.stop() if rank == 0 else None
         # per-kernel device time: the same steps again with CUDA events around every kernel family
@@ -550,6 +579,8 @@ def run_ours(args, cfg):
                                             validation=cpu_validation(cfg, w, one["fit"]))
             print(json.dumps(line), flush=True)
         ctx.close()
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -825,9 +856,15 @@ def main():
                          "configs[1]-shaped; clustering = configs[4]; mica = the permutation test of "
                          "examples/RNA/BacteriaSSU/options_perm.mica (all three N = 1, ours only)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64): a fixed "
+                         "seeded sample of the pair table's rows (pairs_<column>, pairs_row = their row numbers) and the "
+                         "binned null (null_sorted, null_bin_offsets, null_nmax); default workload, one process")
     for k in ("sites", "taxa", "rep_cpu", "rep_ram"):
         ap.add_argument("--" + k.replace("_", "-"), type=int, default=None)
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "nucleotides"):
+        ap.error("--dump-outputs is implemented for the default workload (--impl ours --workload nucleotides)")
     cfg = dict(CFG)
     for k in ("sites", "taxa", "rep_cpu", "rep_ram"):
         if getattr(args, k) is not None:

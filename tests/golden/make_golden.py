@@ -1,13 +1,16 @@
-"""Regenerates tests/golden/*.npz from the reference tree (run in the build container only).
+"""Regenerates tests/golden/*.npz from a checkout of the reference (CoMap's source tree).
+
+    python tests/golden/make_golden.py <path to the CoMap source tree>
 
 The reference ships exactly one set of numerical outputs for the hot path
 (examples/Proteins/Benchmark/CoMap/Myo_*.vec + Myo.infos, SURVEY.md s4/s8c).  They and the
 inputs that produced them (Myoglobin alignment + tree) are packed into one .npz so the
-tests can run on the GPU box, where /root/reference does not exist.  The RNA example's
-inputs are packed too (no expected outputs exist for it).
+tests need nothing outside this repository.  The .vec tables are stored as tab-separated
+text with the reference's 6 significant digits (tests/helpers.py golden() parses them back),
+which keeps the file under 1 MB.  The RNA example's inputs are packed too (no expected
+outputs exist for it).
 """
 import numpy as np, os, sys
-REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 def load_vec(p):
@@ -31,7 +34,8 @@ def main():
     out = {}
     for k in ("unif", "decomp", "naive", "laplace", "unif_grantham", "decomp_grantham", "naive_grantham"):
         coords, mean, M = load_vec(bm + "Myo_%s.vec" % k)
-        out["vec_" + k] = M            # [branch][site], 6 significant digits
+        txt = "".join("\t".join("%.6g" % v for v in row) + "\n" for row in M)   # [branch][site], 6 significant digits
+        out["vec_" + k] = np.frombuffer(txt.encode(), dtype=np.uint8)
     out["vec_coords"] = coords
     out["vec_brlen"] = mean
     inf = [l.split("\t") for l in open(bm + "Myo.infos").read().strip().split("\n")[1:]]
@@ -57,4 +61,5 @@ def main():
         dnd=np.frombuffer(open(s + "SRK.dnd", "rb").read(), dtype=np.uint8))
 
 if __name__ == "__main__":
+    REF = sys.argv[1]
     main()

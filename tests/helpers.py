@@ -10,7 +10,11 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def golden(name):
-    return np.load(os.path.join(GOLDEN, name + ".npz"))
+    """The arrays of tests/golden/<name>.npz.  The reference's .vec tables are stored as their text (tab-separated,
+    6 significant digits, one row per branch), which keeps the file small; they come back as float64 [branch][site]."""
+    with np.load(os.path.join(GOLDEN, name + ".npz")) as z:
+        return {k: np.loadtxt(io.StringIO(text(z[k])), delimiter="\t", ndmin=2) if k.startswith("vec_") and z[k].dtype == np.uint8
+                else z[k] for k in z.files}
 
 
 def text(arr):
