@@ -91,8 +91,12 @@ void Context::ensure_streams() {
     down_stream.upload(os, stream);
     if (A == 4) build_up_mma_stream(os, tree, tables); // tensor-core up pass (k1_mma.cu)
     else if (protein_mma) build_up_mma20_stream(os, tree, tables, kChunkSites20);
-    else build_up_stream(os, tree, tables, 0, C);
+    else build_up_stream(os, tree, tables, 0, std::min(C, kScalarUpClasses));
     up_stream.upload(os, stream);
+    if (A == 20 && !protein_mma && C > kScalarUpClasses) { // the rest of the classes, a second up launch
+      build_up_stream(os, tree, tables, kScalarUpClasses, C - kScalarUpClasses);
+      up_stream_hi.upload(os, stream);
+    }
   }
   {
     OpStream os;
@@ -271,6 +275,10 @@ void Context::run_map(const MapBuffers& b, bool simulated, bool states_only, boo
     part.reserve(sizeof(double) * (size_t)m.C * m.B * b.n_pad);
     if (!launch_map_up_mma20(m, b, up_stream, part.as<double>(), stream)) fail("mapping up pass: no launch shape fits shared memory for A = 20, C = %d", m.C);
     prof_end(2);
+  } else if (m.A == 20 && m.C > kScalarUpClasses) {
+    launch_map_up(m, b, up_stream, stream, 0, kScalarUpClasses);
+    launch_map_up(m, b, up_stream_hi, stream, kScalarUpClasses, m.C - kScalarUpClasses);
+    prof_end(2);
   } else {
     launch_map_up(m, b, up_stream, stream);
     prof_end(1);
@@ -363,6 +371,7 @@ int cmb_ctx_destroy(cmb_ctx* ctx) {
   for (DevBuf* b : bufs) b->release();
   c.down_stream.release();
   c.up_stream.release();
+  c.up_stream_hi.release();
   c.sim_stream.release();
   if (c.own_stream) cudaStreamDestroy(c.stream);
   delete ctx;

@@ -43,6 +43,7 @@ struct Context {
   // device-resident model + op streams
   DevBuf d_code_mask, d_pi, d_rates, d_probs;
   DevStream down_stream, up_stream, sim_stream;
+  DevStream up_stream_hi; // scalar protein up pass above kScalarUpClasses classes: classes [kScalarUpClasses, C)
   int cont_kind = 0;             // continuous-rate simulation (cmb_set_continuous_rates)
   double cont_alpha = 1., cont_pinv = 0.;
   DevBuf d_spec;                 // ev | R | L | brlen for it

@@ -403,6 +403,9 @@ struct UpParams {
   int groups;           // G
   int n_blocks, n_tips; // stage ring depth (n_tips unused)
   uint32_t block_bytes; // C*A*SG*8
+  // class block [c0, c0 + C) of a mapping with d_rows / A classes: the stored partials are rows c0*A.. of the
+  // d_rows-row blocks of b.D, and a block after the first adds its terms to b.out instead of writing them
+  int d_rows, d_row0, accumulate;
 };
 constexpr int kMaxBlocks = 8; // stage ring depth
 
@@ -481,12 +484,12 @@ __global__ void __launch_bounds__(MAXT, MINB) k1_up(MapModel m, MapBuffers b, Up
       }
       __syncwarp();
       if (ina) {
-        const double* src = b.D + d_block(site0 >> 8, h0.y, m.n_slots, rows) + (site0 & (kDSites - 1));
+        const double* src = b.D + d_block(site0 >> 8, h0.y, m.n_slots, up.d_rows) + (size_t)up.d_row0 * kDSites + (site0 & (kDSites - 1));
         for (int r = lane; r < rows; r += 32)
           tma_bulk_g2s(st + tip_slot + (size_t)r * row_bytes, src + (size_t)r * kDSites, row_bytes, &stg_full[s]);
       }
       if (inb) {
-        const double* src = b.D + d_block(site0 >> 8, h0.z, m.n_slots, rows) + (site0 & (kDSites - 1));
+        const double* src = b.D + d_block(site0 >> 8, h0.z, m.n_slots, up.d_rows) + (size_t)up.d_row0 * kDSites + (site0 & (kDSites - 1));
         for (int r = lane; r < rows; r += 32)
           tma_bulk_g2s(st + tip_slot + up.block_bytes + (size_t)r * row_bytes, src + (size_t)r * kDSites, row_bytes, &stg_full[s]);
       }
@@ -719,7 +722,8 @@ __global__ void __launch_bounds__(MAXT, MINB) k1_up(MapModel m, MapBuffers b, Up
           const double* src = rb + (size_t)(g * C * 2 + ab) * SW + k * 32 + lane;
           double t = 0.;
           for (int cc = 0; cc < C; cc++) t += src[(size_t)cc * 2 * SW];
-          b.out[(size_t)ob * n_pad + site0 + lsite + k * 32] = t * invL[k];
+          double* o = b.out + (size_t)ob * n_pad + site0 + lsite + k * 32;
+          *o = up.accumulate ? *o + t * invL[k] : t * invL[k];
         }
       }
       // ---- messages for the children that are expanded later
@@ -807,7 +811,7 @@ bool up_shape(int C, uint32_t cap, int max_smem, int max_warps, UpShape& sh) {
 }
 
 template <int A, int NS, int MAXT, int MINB, int CT = 0, int GT = 0>
-bool try_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st) {
+bool try_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st, int c0 = 0, int c_total = 0) {
   int dev = 0, max_smem = 0;
   CMB_CUDA(cudaGetDevice(&dev));
   CMB_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
@@ -826,6 +830,9 @@ bool try_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStre
   up.n_blocks = sh.n_blocks;
   up.n_tips = sh.n_tips;
   up.block_bytes = sh.block_bytes;
+  up.d_rows = (c_total > 0 ? c_total : m.C) * A;
+  up.d_row0 = c0 * A;
+  up.accumulate = c0 > 0;
   CMB_CUDA(cudaFuncSetAttribute(k1_up<A, NS, MAXT, MINB, CT, GT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh.smem));
   k1_up<A, NS, MAXT, MINB, CT, GT><<<(unsigned)(b.n_pad / SG), 32 * (sh.groups * m.C + 2), sh.smem, st>>>(m, b, up);
   CMB_CUDA(cudaGetLastError());
@@ -833,12 +840,14 @@ bool try_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStre
 }
 
 template <int A>
-void run_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st) {
+void run_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st, int c0, int c_total) {
   if constexpr (A == 4) return launch_map_up_mma(m, b, s, st);
   // proteins: one site group per CTA (C class warps + 2 producers, <= 255 registers).  Two groups
   // (320 threads, 168 registers) spill 1 KB per thread of the five live 20-vectors: 12.3 vs 4.9 ms
-  // per 20 000 sites at config 5.
-  else if (!try_up<A, 1, 192, 1>(m, b, s, st) && !try_up<A, 1, 320, 1>(m, b, s, st))
+  // per 20 000 sites at config 5.  More than kScalarUpClasses classes do not fit shared memory (two
+  // record chunks of 3.2 KB x 4 x C plus two stages of C stored partials: 236 KB at C = 5 on a B200's
+  // 227 KB), so the caller runs those in class blocks (Context::ensure_streams, run_map).
+  else if (!try_up<A, 1, 192, 1>(m, b, s, st, c0, c_total))
     fail("mapping up pass: no launch shape fits shared memory for A = %d, C = %d", A, m.C);
 }
 
@@ -856,9 +865,13 @@ void launch_map_down(const MapModel& m, const MapBuffers& b, const DevStream& s,
   else if (m.A == 20) run_down<20>(m, b, s, st);
   else fail("no mapping kernel for A = %d", m.A);
 }
-void launch_map_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st) {
-  if (m.A == 4) run_up<4>(m, b, s, st);
-  else if (m.A == 20) run_up<20>(m, b, s, st);
+void launch_map_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st, int c0, int cb) {
+  if (c0 < 0 || cb < 0 || c0 + cb > m.C || (c0 > 0 && cb == 0)) fail("internal: bad class block %d + %d of %d", c0, cb, m.C);
+  if (cb > 0 && (m.A != 20 || cb > kScalarUpClasses)) fail("internal: class blocks are for the scalar protein up pass (<= %d classes)", kScalarUpClasses);
+  MapModel mb = m;
+  if (cb > 0) mb.C = cb;
+  if (m.A == 4) run_up<4>(mb, b, s, st, c0, m.C);
+  else if (m.A == 20) run_up<20>(mb, b, s, st, c0, m.C);
   else fail("no mapping kernel for A = %d", m.A);
 }
 void launch_map_finish(const MapModel& m, const MapBuffers& b, cudaStream_t st) {

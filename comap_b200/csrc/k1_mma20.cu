@@ -492,7 +492,9 @@ bool try_down20(const MapModel& m, const MapBuffers& b, const DevStream& s, cuda
 
 } // namespace
 
-// false: no launch shape fits (deep stack / many classes) -- the caller falls back to the scalar kernels
+// false: no launch shape fits.  cmb_map reports that as an error: it does not fall back to the scalar kernels.
+// Context::ensure_streams sends trees deeper than 12 levels there up front, and on a B200 (227 KB per CTA)
+// one CTA per SM holds a 12-level stack (120 KB) with 8 stages, so the error is not reached there.
 bool launch_map_down_mma20(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st) {
   if (m.A != 20 || b.n_pad % SG) return false;
   if (m.states_only) return try_down20<2, true>(m, b, s, st) || try_down20<1, true>(m, b, s, st);

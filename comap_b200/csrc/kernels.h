@@ -54,7 +54,10 @@ struct MapModel {            // device-resident model constants
 void check_map_support(int A, int C); // throws when no kernel is built for (A, C)
 void launch_map_down(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st);
 void launch_map_finish(const MapModel& m, const MapBuffers& b, cudaStream_t st);
-void launch_map_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st);
+// cb > 0: only classes [c0, c0 + cb) of the m.C, from an up stream built for them (build_up_stream(.., c0, cb));
+// the first block writes b.out, later ones add to it.  Scalar protein kernels only, cb <= kScalarUpClasses.
+constexpr int kScalarUpClasses = 4;
+void launch_map_up(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st, int c0 = 0, int cb = 0);
 // A = 4: tensor-core up pass (k1_mma.cu); the stream is build_up_mma_stream's
 void launch_map_up_mma(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st);
 void launch_map_down_mma(const MapModel& m, const MapBuffers& b, const DevStream& s, cudaStream_t st);

@@ -42,7 +42,7 @@ def test_map_dna_vs_oracle(ctx, T, S, seed, amb):
     _check(r, q)
 
 
-@pytest.mark.parametrize("C", [1, 2, 3, 6, 8])
+@pytest.mark.parametrize("C", [1, 2, 3, 6, 7, 8])
 def test_map_dna_class_counts(ctx, C):
     """Every rate-class count the tensor-core kernels are instantiated for (1..8), with gaps."""
     c = H.random_dna_case(17, 260, 10 + C, C=C, ambiguity=0.05)
