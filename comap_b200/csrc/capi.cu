@@ -13,7 +13,7 @@ thread_local std::string g_last_error;
 void DevBuf::reserve(size_t bytes) {
   if (bytes <= cap) return;
   release();
-  size_t want = (bytes + 255) & ~size_t(255);
+  size_t want = align256(bytes);
   cudaError_t e = cudaMalloc(&p, want);
   if (e != cudaSuccess) {
     p = nullptr;
@@ -47,9 +47,6 @@ void DevStream::upload(const OpStream& s, cudaStream_t st) {
     CMB_CUDA(cudaMemcpyAsync(aux.p, s.aux.data(), sizeof(int32_t) * s.aux.size(), cudaMemcpyHostToDevice, st));
   }
   CMB_CUDA(cudaStreamSynchronize(st)); // host vectors may go away
-}
-void DevStream::release() {
-  bytes.release(); off.release(); nbytes.release(); nrec.release(); aux.release();
 }
 
 // Site counts are padded to whole 256-site blocks, and to an ODD number of them: the row stride
@@ -200,8 +197,9 @@ void Context::prof_collect() {
   prof.pending.clear();
 }
 
-void Context::wait_map() {
+void Context::cancel_map() {
   if (map_pending) CMB_CUDA(cudaEventSynchronize(map_done));
+  map_pending = false;
 }
 
 // max(norm) for the null's Domain and the saturated-site check of a finished mapping (host copies are in place)
@@ -258,6 +256,32 @@ VariantTables Context::variant_tables() {
   return vt;
 }
 
+MapBuffers Context::sim_buffers(int k, int64_t n, int64_t n_pad) {
+  const int B = tree.B, T = tree.n_leaves;
+  s_tips[k].reserve((size_t)T * n_pad);
+  s_D.reserve(sizeof(double) * (size_t)tree.n_slots * C * A * n_pad);
+  s_Lc.reserve(sizeof(double) * (size_t)C * n_pad);
+  s_invL.reserve(sizeof(double) * n_pad);
+  s_loglik.reserve(sizeof(double) * n_pad);
+  s_pr[k].reserve(sizeof(double) * n_pad);
+  s_rc[k].reserve(sizeof(int32_t) * n_pad);
+  s_out[k].reserve(sizeof(double) * (size_t)B * n_pad);
+  MapBuffers b;
+  b.n = n; b.n_pad = n_pad;
+  b.tips = s_tips[k].as<uint8_t>();
+  b.D = s_D.as<double>(); b.Lc = s_Lc.as<double>(); b.invL = s_invL.as<double>();
+  b.loglik = s_loglik.as<double>(); b.post_rate = s_pr[k].as<double>(); b.rate_class = s_rc[k].as<int32_t>();
+  b.out = s_out[k].as<double>();
+  return b;
+}
+
+void Context::clear_sim_tip_padding(int64_t n, int64_t n_pad) {
+  uint8_t* tips = s_tips[0].as<uint8_t>();
+  if (s_tips_ptr == tips && s_tips_pad == n_pad && s_tips_n == n) return;
+  CMB_CUDA(cudaMemsetAsync(tips, 0, (size_t)tree.n_leaves * n_pad, stream));
+  s_tips_ptr = tips; s_tips_pad = n_pad; s_tips_n = n;
+}
+
 // Down pass for every class block, site likelihoods, then up pass + contraction.
 void Context::run_map(const MapBuffers& b, bool simulated, bool states_only, bool variants) {
   MapModel m = map_model();
@@ -294,21 +318,6 @@ void Context::run_map(const MapBuffers& b, bool simulated, bool states_only, boo
 } // namespace cmb
 
 using namespace cmb;
-
-#define CMB_TRY try {
-#define CMB_CATCH                                   \
-  }                                                 \
-  catch (const std::exception& e) {                 \
-    g_last_error = e.what();                        \
-    return 1;                                       \
-  }                                                 \
-  catch (...) {                                     \
-    g_last_error = "unknown error";                 \
-    return 1;                                       \
-  }                                                 \
-  return 0;
-
-struct cmb_ctx { Context c; };
 
 extern "C" {
 
@@ -359,22 +368,8 @@ int cmb_ctx_destroy(cmb_ctx* ctx) {
   if (c.copy_stream) { cudaStreamSynchronize(c.copy_stream); cudaStreamDestroy(c.copy_stream); }
   if (c.copy_event) cudaEventDestroy(c.copy_event);
   for (auto& t : c.prof.pending) { cudaEventDestroy(std::get<1>(t)); cudaEventDestroy(std::get<2>(t)); }
-  DevBuf* bufs[] = {&c.d_code_mask, &c.d_pi, &c.d_rates, &c.d_probs, &c.d_tips, &c.d_D, &c.d_Lc, &c.d_invL,
-                    &c.d_loglik, &c.d_pr, &c.d_rc, &c.d_out, &c.d_sum, &c.d_sumsq, &c.s_tips[0], &c.s_tips[1],
-                    &c.s_D, &c.s_Lc, &c.s_invL, &c.s_loglik, &c.s_pr[0], &c.s_pr[1], &c.s_rc[0], &c.s_rc[1],
-                    &c.s_out[0], &c.s_out[1], &c.s_sum[0], &c.s_sum[1], &c.s_sumsq[0], &c.s_sumsq[1], &c.s_cls,
-                    &c.d_identity_mask, &c.null.stat, &c.null.nmin, &c.null.sorted, &c.null.bin_off_dev,
-                    &c.d_dist, &c.scratch, &c.scratch2, &c.staging, &c.pair_table, &c.pairs_mean, &c.pairs_sd, &c.pairs_norm,
-                    &c.d_meanvec, &c.corr_mean, &c.corr_sd, &c.mi_count, &c.gather_send, &c.gather_recv, &c.k1_part, &c.k1_part_obs, &c.var_tree, &c.var_tabs, &c.var_scratch, &c.var_scratch_obs, &c.mica_sites, &c.mica_table, &c.d_spec, &c.dist_tiles, &c.s_cols, &c.s_counts, &c.cn_mean, &c.cn_sd, &c.cn_norm, &c.cn_staging,
-                    &c.cn_dists[0], &c.cn_dists[1], &c.cn_dists[2], &c.cn_dists[3], &c.cn_works[0], &c.cn_works[1], &c.cn_works[2],
-                    &c.cn_works[3], &c.cn_outs[0], &c.cn_outs[1], &c.cn_outs[2], &c.cn_outs[3]};
-  for (DevBuf* b : bufs) b->release();
-  c.down_stream.release();
-  c.up_stream.release();
-  c.up_stream_hi.release();
-  c.sim_stream.release();
   if (c.own_stream) cudaStreamDestroy(c.stream);
-  delete ctx;
+  delete ctx; // device buffers free themselves
   CMB_CATCH
 }
 
@@ -390,7 +385,7 @@ int cmb_set_tree(cmb_ctx* ctx, int32_t n_nodes, const int32_t* parent, const dou
   CMB_TRY
   Context& c = ctx->c;
   CMB_CUDA(cudaSetDevice(c.device));
-  c.wait_map(); c.map_pending = false;
+  c.cancel_map();
   build_tree(c.tree, n_nodes, parent, brlen);
   c.have_tree = true;
   c.streams_ready = false;
@@ -408,7 +403,7 @@ int cmb_set_model(cmb_ctx* ctx, int32_t A, const double* Q, const double* pi, in
   if (A < 2 || A > 32) fail("cmb_set_model: A must be in 2..32 (got %d)", A);
   if (C < 1 || C > 32) fail("cmb_set_model: C must be in 1..32 (got %d)", C);
   check_map_support(A, C);
-  c.wait_map(); c.map_pending = false;
+  c.cancel_map();
   c.A = A; c.C = C; c.count_method = count_method;
   c.Q.assign(Q, Q + (size_t)A * A);
   c.pi.assign(pi, pi + A);
@@ -432,7 +427,7 @@ int cmb_set_alignment(cmb_ctx* ctx, int64_t S, const uint8_t* codes, int32_t n_c
   if (S < 1) fail("cmb_set_alignment: empty alignment");
   if (n_codes < 1 || n_codes > 256) fail("cmb_set_alignment: n_codes must be in 1..256");
   const int T = c.tree.n_leaves;
-  c.wait_map(); c.map_pending = false;
+  c.cancel_map();
   {
     uint8_t worst = 0; // branch-free max over the T*S codes (vectorises); the slow scan only names the culprit
     for (int64_t i = 0; i < (int64_t)T * S; i++) worst = codes[i] > worst ? codes[i] : worst;
@@ -461,9 +456,9 @@ int cmb_set_alignment(cmb_ctx* ctx, int64_t S, const uint8_t* codes, int32_t n_c
 int cmb_set_map_mode(cmb_ctx* ctx, int32_t average, int32_t joint) {
   CMB_TRY
   Context& c = ctx->c;
-  c.wait_map(); c.map_pending = false;
+  c.cancel_map();
   const int mode = (average ? 0 : 2) + (joint ? 0 : 1);
-  if (mode != c.map_mode) { c.mapped = false; c.null.ready = false; c.pairs_rows = -1; c.have_dist = false; }
+  if (mode != c.map_mode) { c.mapped = false; c.null.ready = false; c.drop_pair_table(); c.have_dist = false; }
   c.map_mode = mode;
   CMB_CATCH
 }
@@ -492,8 +487,7 @@ int cmb_map(cmb_ctx* ctx, double* n_out, double* norm, double* post_rate, int32_
   Context& c = ctx->c;
   CMB_CUDA(cudaSetDevice(c.device));
   if (!c.have_alignment) fail("cmb_map: call cmb_set_alignment first");
-  c.wait_map();
-  c.map_pending = false;
+  c.cancel_map();
   c.mapped = false;
   c.ensure_streams();
   const int64_t S = c.S, Sp = c.S_pad;
@@ -555,8 +549,7 @@ int cmb_map(cmb_ctx* ctx, double* n_out, double* norm, double* post_rate, int32_
   if (rate_class) CMB_CUDA(cudaMemcpyAsync(rate_class, c.d_rc.p, sizeof(int32_t) * S, cudaMemcpyDeviceToHost, c.stream));
   CMB_CUDA(cudaMemcpyAsync(c.h_loglik, c.d_loglik.p, sizeof(double) * S, cudaMemcpyDeviceToHost, c.stream));
   c.have_dist = false;
-  c.pairs_rows = -1; // resident pair columns belong to the previous mapping
-  for (auto& o : c.pairs_col_off) o = -1;
+  c.drop_pair_table(); // resident pair columns belong to the previous mapping
   if (c.null.nmax_from_map) c.null.ready = false; // binned with the previous mapping's max(norm)
   if (deferred) {
     CMB_CUDA(cudaEventRecord(c.map_done, c.map_stream));
@@ -597,16 +590,14 @@ int cmb_load_vectors(cmb_ctx* ctx, const double* n_in, double* norm) {
   if (norm) std::memcpy(norm, c.h_norm, sizeof(double) * S);
   c.have_dist = false;
   c.null.ready = false;
-  c.pairs_rows = -1;
-  for (auto& o : c.pairs_col_off) o = -1;
+  c.drop_pair_table();
   CMB_CATCH
 }
 
 int cmb_set_mi_threshold(cmb_ctx* ctx, double threshold) {
   ctx->c.mi_threshold = threshold;
   ctx->c.have_mi_count = false;
-  ctx->c.pairs_rows = -1; // resident Stat columns were scored with the previous threshold
-  for (auto& o : ctx->c.pairs_col_off) o = -1;
+  ctx->c.drop_pair_table(); // resident Stat columns were scored with the previous threshold
   return 0;
 }
 

@@ -15,22 +15,7 @@
 #include <cmath>
 #include <cstring>
 
-namespace cmb { extern thread_local std::string g_last_error; }
 using namespace cmb;
-struct cmb_ctx { Context c; };
-
-#define CMB_TRY try {
-#define CMB_CATCH                                   \
-  }                                                 \
-  catch (const std::exception& e) {                 \
-    g_last_error = e.what();                        \
-    return 1;                                       \
-  }                                                 \
-  catch (...) {                                     \
-    g_last_error = "unknown error";                 \
-    return 1;                                       \
-  }                                                 \
-  return 0;
 
 namespace {
 
@@ -52,25 +37,6 @@ void order_after(cudaStream_t later, cudaStream_t earlier) {
   CMB_CUDA(cudaEventDestroy(e));
 }
 
-MapBuffers sim_buffers0(Context& c, int64_t n, int64_t n_pad) {
-  const int A = c.A, C = c.C, B = c.tree.B, T = c.tree.n_leaves;
-  c.s_tips[0].reserve((size_t)T * n_pad);
-  c.s_D.reserve(sizeof(double) * (size_t)c.tree.n_slots * C * A * n_pad);
-  c.s_Lc.reserve(sizeof(double) * (size_t)C * n_pad);
-  c.s_invL.reserve(sizeof(double) * n_pad);
-  c.s_loglik.reserve(sizeof(double) * n_pad);
-  c.s_pr[0].reserve(sizeof(double) * n_pad);
-  c.s_rc[0].reserve(sizeof(int32_t) * n_pad);
-  c.s_out[0].reserve(sizeof(double) * (size_t)B * n_pad);
-  MapBuffers b;
-  b.n = n; b.n_pad = n_pad;
-  b.tips = c.s_tips[0].as<uint8_t>();
-  b.D = c.s_D.as<double>(); b.Lc = c.s_Lc.as<double>(); b.invL = c.s_invL.as<double>();
-  b.loglik = c.s_loglik.as<double>(); b.post_rate = c.s_pr[0].as<double>(); b.rate_class = c.s_rc[0].as<int32_t>();
-  b.out = c.s_out[0].as<double>();
-  return b;
-}
-
 } // namespace
 
 extern "C" {
@@ -83,7 +49,7 @@ int cmb_pairs_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, const cmb_fil
   Context& c = ctx1->c;
   Context& d = ctx2->c;
   CMB_CUDA(cudaSetDevice(c.device));
-  if (stat_id < 0 || stat_id > CMB_STAT_MI_LABEL) fail("unknown statistic id %d", stat_id);
+  check_stat(stat_id);
   check_pair(c, d, "cmb_pairs_inter");
   c.finish_map(); d.finish_map();
   if (!c.mapped || !d.mapped) fail("cmb_pairs_inter: call cmb_map on both data sets first");
@@ -94,22 +60,19 @@ int cmb_pairs_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, const cmb_fil
   const double* mv1 = corrected ? c.mean_vector() : nullptr;
   const double* mv2 = corrected ? d.mean_vector() : nullptr;
   order_after(c.stream, d.stream); // the second data set's mapping (and mean vector) is complete
-  const bool any_filter = (f && (f->min_rate_class > 0 || f->min_rate > 0. || f->max_rate_class_diff >= 0 ||
-                                 f->max_rate_diff >= 0. || f->min_stat > 0.)) || min_rate_class2 > 0 || min_rate2 > 0.;
-  auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
+  const bool filtered = any_filter(f) || min_rate_class2 > 0 || min_rate2 > 0.;
   const int64_t total = independent ? S1 : S1 * S2;
   if (total > 0x7fffffff) fail("cmb_pairs_inter: %lld pairs exceed the 2^31 - 1 rows one call scores", (long long)total);
   // dense columns i j stat rcmin prmin nmin | keep | compacted copies
   const size_t elt[6] = {4, 4, 8, 4, 8, 8};
   size_t off[6], off2[6], cur = 0;
-  for (int k = 0; k < 6; k++) { off[k] = cur; cur = al(cur + elt[k] * (size_t)total); }
+  for (int k = 0; k < 6; k++) { off[k] = cur; cur = align256(cur + elt[k] * (size_t)total); }
   const size_t o_keep = cur;
-  cur = al(cur + (size_t)total);
-  for (int k = 0; k < 6; k++) { off2[k] = cur; cur = al(cur + (any_filter ? elt[k] * (size_t)total : 0)); }
+  cur = align256(cur + (size_t)total);
+  for (int k = 0; k < 6; k++) { off2[k] = cur; cur = align256(cur + (filtered ? elt[k] * (size_t)total : 0)); }
   if (c.copy_stream) CMB_CUDA(cudaStreamSynchronize(c.copy_stream));
   c.pair_table.reserve(cur + 256);
-  for (auto& o : c.pairs_col_off) o = -1; // the resident intra table is gone
-  c.pairs_rows = -1;
+  c.drop_pair_table(); // the resident intra table is gone
   unsigned char* sb = c.pair_table.as<unsigned char>();
   int32_t* o_i = (int32_t*)(sb + off[0]); int32_t* o_j = (int32_t*)(sb + off[1]); double* o_stat = (double*)(sb + off[2]);
   int32_t* o_rc = (int32_t*)(sb + off[3]); double* o_pr = (double*)(sb + off[4]); double* o_nm = (double*)(sb + off[5]);
@@ -137,7 +100,7 @@ int cmb_pairs_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, const cmb_fil
     L.min_rate = f->min_rate; L.max_rate_diff = f->max_rate_diff; L.min_stat = f->min_stat;
   }
   L.min_rate_class2 = min_rate_class2; L.min_rate2 = min_rate2;
-  L.any_filter = any_filter; L.nmin_by_row = nmin_by_row;
+  L.any_filter = filtered; L.nmin_by_row = nmin_by_row;
   L.o_i = o_i; L.o_j = o_j; L.o_stat = o_stat; L.o_rcmin = o_rc; L.o_prmin = o_pr; L.o_nmin = o_nm; L.o_keep = o_keep_p;
   c.prof_begin("pairs");
   int nl = 0;
@@ -157,17 +120,15 @@ int cmb_pairs_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, const cmb_fil
   }
   c.prof_end(nl);
   int64_t kept = total;
-  if (any_filter && total > 0) {
+  if (filtered && total > 0) {
     int64_t* pos = nullptr;
     kept = compact_positions(total, o_keep_p, c.scratch2, &pos, c.stream);
-    compact_column<int32_t>(total, o_keep_p, pos, o_i, (int32_t*)(sb + off2[0]), c.stream);
-    compact_column<int32_t>(total, o_keep_p, pos, o_j, (int32_t*)(sb + off2[1]), c.stream);
-    compact_column<double>(total, o_keep_p, pos, o_stat, (double*)(sb + off2[2]), c.stream);
-    compact_column<int32_t>(total, o_keep_p, pos, o_rc, (int32_t*)(sb + off2[3]), c.stream);
-    compact_column<double>(total, o_keep_p, pos, o_pr, (double*)(sb + off2[4]), c.stream);
-    compact_column<double>(total, o_keep_p, pos, o_nm, (double*)(sb + off2[5]), c.stream);
-    c.prof.total_launches += 6;
-    for (int k = 0; k < 6; k++) off[k] = off2[k];
+    for (int k = 0; k < 6; k++) {
+      if (elt[k] == 4) compact_column<int32_t>(total, o_keep_p, pos, (int32_t*)(sb + off[k]), (int32_t*)(sb + off2[k]), c.stream);
+      else compact_column<double>(total, o_keep_p, pos, (double*)(sb + off[k]), (double*)(sb + off2[k]), c.stream);
+      off[k] = off2[k];
+      c.prof.total_launches += 1;
+    }
   }
   if (kept > capacity) fail("cmb_pairs_inter: capacity %lld < %lld rows", (long long)capacity, (long long)kept);
   void* host[6] = {out_i, out_j, out_stat, out_rcmin, out_prmin, out_nmin};
@@ -185,7 +146,7 @@ int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed,
   Context& c = ctx1->c;
   Context& d = ctx2->c;
   CMB_CUDA(cudaSetDevice(c.device));
-  if (stat_id < 0 || stat_id > CMB_STAT_MI_LABEL) fail("unknown statistic id %d", stat_id);
+  check_stat(stat_id);
   if (rep_ram < 1 || rep_cpu < 0) fail("cmb_null_inter: bad replicate counts");
   if (!raw) fail("cmb_null_inter: raw output buffer required");
   check_pair(c, d, "cmb_null_inter");
@@ -196,17 +157,12 @@ int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed,
   const double* mv2 = corrected ? d.mean_vector() : nullptr;
   const int B = c.tree.B;
   const int64_t R = rep_ram, total = (int64_t)rep_cpu * R;
-  c.null.ready = false;
-  c.null.stat.reserve(sizeof(double) * (size_t)std::max<int64_t>(total, 1));
-  c.null.nmin.reserve(sizeof(double) * (size_t)std::max<int64_t>(total, 1));
+  c.null.begin(total);
   // batch outer replicates: the two data sets' partials are alive at the same time
   size_t freeb = 0, totalb = 0;
   CMB_CUDA(cudaMemGetInfo(&freeb, &totalb));
-  auto per_site = [](const Context& x) {
-    return (size_t)x.tree.n_slots * x.C * x.A * 8 + (size_t)x.tree.B * 8 + (size_t)x.tree.n_leaves + (size_t)x.C * 8 + 64;
-  };
   const size_t held = c.s_D.cap + c.s_out[0].cap + d.s_D.cap + d.s_out[0].cap;
-  int64_t max_sites = (int64_t)((double)(freeb + held) * 0.6 / (double)(per_site(c) + per_site(d)));
+  int64_t max_sites = (int64_t)((double)(freeb + held) * 0.6 / (double)(null_bytes_per_site(c) + null_bytes_per_site(d)));
   max_sites = std::min<int64_t>(std::max<int64_t>(max_sites, R), (int64_t)1 << 20);
   const int64_t rpb = std::max<int64_t>(1, max_sites / R);
   // the second simulator draws from its own stream of the same counter-based generator
@@ -216,7 +172,7 @@ int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed,
   for (int64_t r0 = 0; r0 < rep_cpu; r0 += rpb) {
     const int64_t nb = std::min<int64_t>(rpb, rep_cpu - r0), n = nb * R;
     const int64_t np1 = pad_sites(n), np2 = pad_sites(n);
-    MapBuffers b1 = sim_buffers0(c, n, np1), b2 = sim_buffers0(d, n, np2);
+    MapBuffers b1 = c.sim_buffers(0, n, np1), b2 = d.sim_buffers(0, n, np2);
     c.prof_begin("simulate");
     launch_simulate(m1, c.sim_stream, seed, r0 * R, R, R, n, np1, weighted_classes, c.tree.n_nodes - 1,
                     c.s_tips[0].as<uint8_t>(), nullptr, c.stream);
@@ -240,7 +196,6 @@ int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed,
     CMB_CUDA(cudaStreamSynchronize(c.stream));
     off += n;
   }
-  c.null.n_samples = total;
   CMB_CATCH
 }
 
@@ -307,8 +262,7 @@ void group_stats(Context& c, int stat_id, const double* out, int64_t n_pad, cons
       for (int64_t col : j.cols) members.push_back((int32_t)col);
       offsets.push_back((int64_t)members.size());
     }
-    auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
-    const size_t o_off = al(members.size() * 4), o_stat = al(o_off + offsets.size() * 8);
+    const size_t o_off = align256(members.size() * 4), o_stat = align256(o_off + offsets.size() * 8);
     c.scratch2.reserve(o_stat + jobs.size() * 8 + 256);
     unsigned char* sb = c.scratch2.as<unsigned char>();
     CMB_CUDA(cudaMemcpyAsync(sb, members.data(), members.size() * 4, cudaMemcpyHostToDevice, c.stream));
@@ -325,8 +279,7 @@ void group_stats(Context& c, int stat_id, const double* out, int64_t n_pad, cons
     for (size_t a = 1; a < j.cols.size(); a++)
       for (size_t b = 0; b < a; b++) pairs.push_back(make_int2((int)j.cols[a], (int)j.cols[b])); // getValueForPair(v[i], v[j])
   std::vector<double> vals(pairs.size());
-  auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
-  const size_t o_stat = al(pairs.size() * sizeof(int2));
+  const size_t o_stat = align256(pairs.size() * sizeof(int2));
   c.scratch2.reserve(o_stat + pairs.size() * 8 + 256);
   unsigned char* sb = c.scratch2.as<unsigned char>();
   if (!pairs.empty()) {
@@ -360,7 +313,7 @@ extern "C" int cmb_candidates(cmb_ctx* ctx, int32_t stat_id, int32_t n_groups, c
   CMB_TRY
   Context& c = ctx->c;
   CMB_CUDA(cudaSetDevice(c.device));
-  if (stat_id < 0 || stat_id > CMB_STAT_MI_LABEL) fail("unknown statistic id %d", stat_id);
+  check_stat(stat_id);
   c.finish_map();
   if (!c.mapped) fail("cmb_candidates: call cmb_map first");
   if (n_groups < 1) fail("ERROR!!! No group can be tested!"); // CoMap.cpp:679-680
@@ -401,7 +354,7 @@ extern "C" int cmb_candidates(cmb_ctx* ctx, int32_t stat_id, int32_t n_groups, c
   int64_t batch = 0;
   bool test = true;
   while (test) { // CoETools::computePValuesForCandidateGroups, CoETools.cpp:1053-1086
-    MapBuffers b = sim_buffers0(c, R, n_pad);
+    MapBuffers b = c.sim_buffers(0, R, n_pad);
     c.prof_begin("simulate");
     launch_simulate(m, c.sim_stream, seed, batch * R, R, R, R, n_pad, weighted_classes, c.tree.n_nodes - 1,
                     c.s_tips[0].as<uint8_t>(), nullptr, c.stream);

@@ -7,32 +7,9 @@
 #include <algorithm>
 #include <cstring>
 
-namespace cmb {
-extern thread_local std::string g_last_error;
-MapBuffers sim_batch_buffers(Context& c, int64_t n, int64_t n_pad);                                                   // capi_stats.cu
-void load_null_distribution(Context& c, const double* stat_dev, const double* key_dev, int64_t n, int K, double kmax); // capi_stats.cu
-} // namespace cmb
-
 using namespace cmb;
 
-#define CMB_TRY try {
-#define CMB_CATCH                                   \
-  }                                                 \
-  catch (const std::exception& e) {                 \
-    g_last_error = e.what();                        \
-    return 1;                                       \
-  }                                                 \
-  catch (...) {                                     \
-    g_last_error = "unknown error";                 \
-    return 1;                                       \
-  }                                                 \
-  return 0;
-
-struct cmb_ctx { Context c; };
-
 namespace {
-
-inline size_t al(size_t x) { return (x + 255) & ~size_t(255); }
 
 // dense columns of the pair table in c.mica_table: MI | Hjoint | Hmin | Nmin | PValue | i | j | Nsim
 struct MicaTable {
@@ -42,7 +19,7 @@ struct MicaTable {
 };
 MicaTable mica_table(Context& c) {
   const int64_t n = c.S * (c.S - 1) / 2;
-  const size_t d = al(sizeof(double) * (size_t)std::max<int64_t>(n, 1)), w = al(sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1));
+  const size_t d = align256(sizeof(double) * (size_t)std::max<int64_t>(n, 1)), w = align256(sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1));
   c.mica_table.reserve(5 * d + 3 * w);
   unsigned char* b = c.mica_table.as<unsigned char>();
   MicaTable t;
@@ -122,7 +99,7 @@ int cmb_mica_pair_list(cmb_ctx* ctx, int64_t n, const int32_t* site1, const int3
   if (n < 0 || !site1 || !site2 || !mi) fail("cmb_mica_pair_list: bad arguments");
   for (int64_t r = 0; r < n; r++)
     if (site1[r] < 0 || site1[r] >= c.S || site2[r] < 0 || site2[r] >= c.S) fail("cmb_mica_pair_list: site index out of range at %lld", (long long)r);
-  const size_t w = al(sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1)), d = al(sizeof(double) * (size_t)std::max<int64_t>(n, 1));
+  const size_t w = align256(sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1)), d = align256(sizeof(double) * (size_t)std::max<int64_t>(n, 1));
   c.scratch.reserve(2 * w + 2 * d);
   unsigned char* b = c.scratch.as<unsigned char>();
   CMB_CUDA(cudaMemcpyAsync(b, site1, sizeof(int32_t) * n, cudaMemcpyHostToDevice, c.stream));
@@ -148,7 +125,7 @@ int cmb_mica_permutations(cmb_ctx* ctx, uint64_t seed, int32_t max_permutations,
   if (max_permutations < 1) fail("Permutation number should be greater than 0!"); // Mica.cpp:611-614
   const int64_t n = c.S * (c.S - 1) / 2;
   if (capacity < n) fail("cmb_mica_permutations: capacity %lld < %lld pairs", (long long)capacity, (long long)n);
-  const size_t d = al(sizeof(double) * (size_t)n), w = al(sizeof(int32_t) * (size_t)n);
+  const size_t d = align256(sizeof(double) * (size_t)n), w = align256(sizeof(int32_t) * (size_t)n);
   c.scratch.reserve(d + w + 256);
   double* pv = c.scratch.as<double>();
   int32_t* np = (int32_t*)(c.scratch.as<unsigned char>() + d);
@@ -174,22 +151,16 @@ int cmb_mica_null_parametric(cmb_ctx* ctx, uint64_t seed, int32_t rep_cpu, int32
   const int B = c.tree.B, T = c.tree.n_leaves;
   const int64_t R = rep_ram, total = (int64_t)rep_cpu * R;
   NullState& ns = c.null;
-  ns.ready = false;
-  ns.stat.reserve(sizeof(double) * (size_t)total);
-  ns.nmin.reserve(sizeof(double) * (size_t)total);
-  ns.n_samples = total;
+  ns.begin(total);
   MapModel m = c.map_model();
   const uint32_t* ident = c.d_identity_mask.as<uint32_t>();
   // Mica.cpp:505-541, one outer replicate at a time: two simulated alignments of rep_ram sites, their mappings for the
   // norms (computeSubstitutionVectors, whatever nijt.average says), MI and joint entropy of site j with site j
   const int64_t half = (R + 255) / 256 * 256, n_pad = pad_sites(half + R);
   for (int64_t r = 0; r < rep_cpu; r++) {
-    MapBuffers bb = sim_batch_buffers(c, half + R, n_pad);
+    MapBuffers bb = c.sim_buffers(0, half + R, n_pad);
     uint8_t* tips = c.s_tips[0].as<uint8_t>();
-    if (c.s_tips_ptr != tips || c.s_tips_pad != n_pad || c.s_tips_n != R) {
-      CMB_CUDA(cudaMemsetAsync(tips, 0, (size_t)T * n_pad, c.stream));
-      c.s_tips_ptr = tips; c.s_tips_pad = n_pad; c.s_tips_n = R;
-    }
+    c.clear_sim_tip_padding(R, n_pad);
     c.prof_begin("simulate");
     launch_simulate(m, c.sim_stream, seed, 2 * r * R, R, 2 * R, 2 * R, n_pad, weighted_classes, c.tree.n_nodes - 1, tips, nullptr,
                     c.stream, R, half, R);
@@ -213,7 +184,7 @@ int cmb_mica_null_parametric(cmb_ctx* ctx, uint64_t seed, int32_t rep_cpu, int32
     }
     c.prof.sites_simulated += 2 * R;
   }
-  if (K > 0) load_null_distribution(c, ns.stat.as<double>(), ns.nmin.as<double>(), total, K, nmax);
+  if (K > 0) null_load(c, ns.stat.as<double>(), ns.nmin.as<double>(), total, K, nmax);
   else CMB_CUDA(cudaStreamSynchronize(c.stream));
   CMB_CATCH
 }
@@ -224,13 +195,10 @@ int cmb_null_load(cmb_ctx* ctx, const double* stat, const double* key, int64_t n
   CMB_CUDA(cudaSetDevice(c.device));
   if (n < 0 || (n > 0 && (!stat || !key))) fail("cmb_null_load: bad arguments");
   NullState& ns = c.null;
-  ns.ready = false;
-  ns.stat.reserve(sizeof(double) * (size_t)std::max<int64_t>(n, 1));
-  ns.nmin.reserve(sizeof(double) * (size_t)std::max<int64_t>(n, 1));
-  ns.n_samples = n;
+  ns.begin(n);
   CMB_CUDA(cudaMemcpyAsync(ns.stat.p, stat, sizeof(double) * n, cudaMemcpyHostToDevice, c.stream));
   CMB_CUDA(cudaMemcpyAsync(ns.nmin.p, key, sizeof(double) * n, cudaMemcpyHostToDevice, c.stream));
-  load_null_distribution(c, ns.stat.as<double>(), ns.nmin.as<double>(), n, K, kmax);
+  null_load(c, ns.stat.as<double>(), ns.nmin.as<double>(), n, K, kmax);
   CMB_CATCH
 }
 

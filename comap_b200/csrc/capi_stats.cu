@@ -5,55 +5,16 @@
 #include <cmath>
 #include <cstring>
 
-namespace cmb { extern thread_local std::string g_last_error; }
 using namespace cmb;
-struct cmb_ctx { Context c; };
 
-#define CMB_TRY try {
-#define CMB_CATCH                                   \
-  }                                                 \
-  catch (const std::exception& e) {                 \
-    g_last_error = e.what();                        \
-    return 1;                                       \
-  }                                                 \
-  catch (...) {                                     \
-    g_last_error = "unknown error";                 \
-    return 1;                                       \
-  }                                                 \
-  return 0;
+namespace cmb {
 
-namespace {
-
-void check_stat(int stat_id) {
-  if (stat_id < 0 || stat_id > CMB_STAT_MI_LABEL) fail("unknown statistic id %d", stat_id);
-}
-
-// Bytes of device memory one simulated site needs through simulate -> map x2 -> paired.
 size_t null_bytes_per_site(const Context& c) {
   size_t D = (size_t)c.tree.n_slots * c.C * c.A * 8;
   size_t out = (size_t)c.tree.B * 8 * 2;
   size_t tips = (size_t)c.tree.n_leaves * 2;
   const size_t part = c.protein_mma ? (size_t)c.C * c.tree.B * 8 : 0; // per-class partial outputs of k1_mma20.cu
   return D + out + tips + part + (size_t)c.C * 8 + 16 * 8;
-}
-
-MapBuffers sim_buffers(Context& c, int k, int64_t n, int64_t n_pad) {
-  const int A = c.A, C = c.C, B = c.tree.B, T = c.tree.n_leaves;
-  c.s_tips[k].reserve((size_t)T * n_pad);
-  c.s_D.reserve(sizeof(double) * (size_t)c.tree.n_slots * C * A * n_pad);
-  c.s_Lc.reserve(sizeof(double) * (size_t)C * n_pad);
-  c.s_invL.reserve(sizeof(double) * n_pad);
-  c.s_loglik.reserve(sizeof(double) * n_pad);
-  c.s_pr[k].reserve(sizeof(double) * n_pad);
-  c.s_rc[k].reserve(sizeof(int32_t) * n_pad);
-  c.s_out[k].reserve(sizeof(double) * (size_t)B * n_pad);
-  MapBuffers b;
-  b.n = n; b.n_pad = n_pad;
-  b.tips = c.s_tips[k].as<uint8_t>();
-  b.D = c.s_D.as<double>(); b.Lc = c.s_Lc.as<double>(); b.invL = c.s_invL.as<double>();
-  b.loglik = c.s_loglik.as<double>(); b.post_rate = c.s_pr[k].as<double>(); b.rate_class = c.s_rc[k].as<int32_t>();
-  b.out = c.s_out[k].as<double>();
-  return b;
 }
 
 void null_load(Context& c, const double* stat_dev, const double* nmin_dev, int64_t n, int K, double nmax) {
@@ -81,6 +42,10 @@ void null_load(Context& c, const double* stat_dev, const double* nmin_dev, int64
   ns.ready = true;
 }
 
+} // namespace cmb
+
+namespace {
+
 // The two simulated alignments of a batch of outer replicates (AnalysisTools.cpp:591-611) live side by side in
 // ONE set of mapping buffers -- columns [0, n) hold batch 1, [half, half + n) batch 2 -- so one down / up launch
 // pair maps both (twice the CTAs per launch: a 125-replicate shard of an 8-GPU run fills 6.6 waves of the grid
@@ -95,10 +60,7 @@ void null_core(Context& c, int stat_id, uint64_t seed, int rep_cpu, int rep_ram,
   const int B = c.tree.B, T = c.tree.n_leaves;
   const int64_t R = rep_ram, nreps = rep_end - rep_begin, total = nreps * R;
   NullState& ns = c.null;
-  ns.ready = false;
-  ns.stat.reserve(sizeof(double) * (size_t)std::max<int64_t>(total, 1));
-  ns.nmin.reserve(sizeof(double) * (size_t)std::max<int64_t>(total, 1));
-  ns.n_samples = total;
+  ns.begin(total);
   // batch as many outer replicates as fit comfortably in free HBM (the answer is cached: cudaMemGetInfo
   // costs a host round trip per call)
   if (c.null_budget_sites <= 0) {
@@ -119,14 +81,9 @@ void null_core(Context& c, int stat_id, uint64_t seed, int rep_cpu, int rep_ram,
   for (int64_t r0 = rep_begin; r0 < rep_end; r0 += rpb) {
     const int64_t nb = std::min<int64_t>(rpb, rep_end - r0), n = nb * R;
     const int64_t half = (n + 255) / 256 * 256, n_pad = pad_sites(half + n);
-    MapBuffers bb = sim_buffers(c, 0, half + n, n_pad);
+    MapBuffers bb = c.sim_buffers(0, half + n, n_pad);
     uint8_t* tips = c.s_tips[0].as<uint8_t>();
-    // the columns between and after the two batches are mapped too (their results are never read): give them
-    // a valid state once per buffer geometry
-    if (c.s_tips_ptr != tips || c.s_tips_pad != n_pad || c.s_tips_n != n) {
-      CMB_CUDA(cudaMemsetAsync(tips, 0, (size_t)T * n_pad, c.stream));
-      c.s_tips_ptr = tips; c.s_tips_pad = n_pad; c.s_tips_n = n;
-    }
+    c.clear_sim_tip_padding(n, n_pad);
     const bool dedup_on = !(getenv("CMB_NULL_DEDUP") && atoi(getenv("CMB_NULL_DEDUP")) == 0);
     const bool dedup = dedup_on && c.A == 4 && !c.map_mode; // the variant kernels walk every column
     int32_t *col_class = nullptr, *col_varied = nullptr;
@@ -240,9 +197,8 @@ void distance_on_device(Context& c, int dist_id, const double* out, int64_t S, i
 void cluster_on_device(Context& c, int linkage, int64_t S) {
   if (linkage < 0 || linkage > 2) fail("unknown clustering method %d", linkage);
   if (S < 2) fail("clustering needs at least 2 sites");
-  auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
-  size_t o_l = 0, o_r = al(4 * S), o_h = al(o_r + 4 * S);
-  c.staging.reserve(al(o_h + 8 * S));
+  size_t o_l = 0, o_r = align256(4 * S), o_h = align256(o_r + 4 * S);
+  c.staging.reserve(align256(o_h + 8 * S));
   unsigned char* sb = c.staging.as<unsigned char>();
   c.prof_begin("cluster");
   int nl = launch_cluster(S, linkage, c.d_dist.as<double>(), c.scratch2, (int32_t*)(sb + o_l), (int32_t*)(sb + o_r),
@@ -263,8 +219,7 @@ void cluster_batch_on_device(Context& c, int linkage, int64_t S, int nb, DevBuf*
                              DendroHost* out) {
   if (linkage < 0 || linkage > 2) fail("unknown clustering method %d", linkage);
   if (S < 2) fail("clustering needs at least 2 sites");
-  auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
-  const size_t o_r = al(4 * S), o_h = al(o_r + 4 * S), per = al(o_h + 8 * S);
+  const size_t o_r = align256(4 * S), o_h = align256(o_r + 4 * S), per = align256(o_h + 8 * S);
   staging.reserve(per * nb);
   unsigned char* sb = staging.as<unsigned char>();
   double* mats[4]; int32_t* l[4]; int32_t* r[4]; double* h[4];
@@ -322,9 +277,8 @@ void groups_of_dendrogram(Context& c, int dist_id, int max_size, int64_t S, int6
   }
   if (dist_id == 1 && !g.height.empty()) {
     const size_t ng = g.height.size();
-    auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
-    size_t o_m = 0, o_o = al(4 * g.members.size()), o_s = al(o_o + 8 * (ng + 1));
-    c.scratch.reserve(al(o_s + 8 * ng));
+    size_t o_m = 0, o_o = align256(4 * g.members.size()), o_s = align256(o_o + 8 * (ng + 1));
+    c.scratch.reserve(align256(o_s + 8 * ng));
     unsigned char* sb = c.scratch.as<unsigned char>();
     CMB_CUDA(cudaMemcpyAsync(sb + o_m, g.members.data(), 4 * g.members.size(), cudaMemcpyHostToDevice, c.stream));
     CMB_CUDA(cudaMemcpyAsync(sb + o_o, g.offsets.data(), 8 * (ng + 1), cudaMemcpyHostToDevice, c.stream));
@@ -337,14 +291,6 @@ void groups_of_dendrogram(Context& c, int dist_id, int max_size, int64_t S, int6
 }
 
 } // namespace
-
-// shared with capi_mica.cu
-namespace cmb {
-MapBuffers sim_batch_buffers(Context& c, int64_t n, int64_t n_pad) { return sim_buffers(c, 0, n, n_pad); }
-void load_null_distribution(Context& c, const double* stat_dev, const double* key_dev, int64_t n, int K, double kmax) {
-  null_load(c, stat_dev, key_dev, n, K, kmax);
-}
-} // namespace cmb
 
 extern "C" {
 
@@ -499,12 +445,10 @@ int cmb_pairs_resident(cmb_ctx* ctx, int32_t stat_id, const cmb_filters* f, int3
     int64_t imin = rows[ti * TS];
     for (int64_t tj = (imin + 1) / TS; tj * TS < S; tj++) tiles.push_back(make_int2((int)ti, (int)tj));
   }
-  const bool any_filter = f && (f->min_rate_class > 0 || f->min_rate > 0. || f->max_rate_class_diff >= 0 ||
-                                f->max_rate_diff >= 0. || f->min_stat > 0.);
-  auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
+  const bool filtered = any_filter(f);
   const size_t nT = std::max<size_t>(total, 1);
-  size_t o_rows = 0, o_roff = al(o_rows + rows.size() * 4), o_tiles = al(o_roff + row_off.size() * 8),
-         o_end = al(o_tiles + tiles.size() * 8);
+  size_t o_rows = 0, o_roff = align256(o_rows + rows.size() * 4), o_tiles = align256(o_roff + row_off.size() * 8),
+         o_end = align256(o_tiles + tiles.size() * 8);
   DevBuf& meta = c.scratch;
   meta.reserve(o_end + 256);
   unsigned char* mb = meta.as<unsigned char>();
@@ -519,11 +463,11 @@ int cmb_pairs_resident(cmb_ctx* ctx, int32_t stat_id, const cmb_filters* f, int3
   // first, PValue / Nsim once the null exists) while earlier ones are still being copied out.
   size_t off[8] = {0}, off2[8] = {0}, cur = 0;
   for (int k = 0; k < 8; k++) {
-    off[k] = cur; cur = al(cur + kColElt[k] * nT);
-    if (any_filter) { off2[k] = cur; cur = al(cur + kColElt[k] * nT); }
+    off[k] = cur; cur = align256(cur + kColElt[k] * nT);
+    if (filtered) { off2[k] = cur; cur = align256(cur + kColElt[k] * nT); }
   }
   size_t o_keep = cur;
-  cur = al(cur + nT);
+  cur = align256(cur + nT);
   if (c.copy_stream && cur + 256 > c.pair_table.cap) CMB_CUDA(cudaStreamSynchronize(c.copy_stream)); // growing frees the old table
   c.pair_table.reserve(cur + 256);
   unsigned char* sb = c.pair_table.as<unsigned char>();
@@ -549,7 +493,7 @@ int cmb_pairs_resident(cmb_ctx* ctx, int32_t stat_id, const cmb_filters* f, int3
     L.min_rate_class = f->min_rate_class; L.max_rate_class_diff = f->max_rate_class_diff;
     L.min_rate = f->min_rate; L.max_rate_diff = f->max_rate_diff; L.min_stat = f->min_stat;
   }
-  L.any_filter = any_filter;
+  L.any_filter = filtered;
   if (use_null) {
     L.K = c.null.K; L.nmax = c.null.nmax;
     L.bin_off = c.null.bin_off_dev.as<int64_t>(); L.sorted = c.null.sorted.as<double>();
@@ -561,7 +505,7 @@ int cmb_pairs_resident(cmb_ctx* ctx, int32_t stat_id, const cmb_filters* f, int3
   c.prof_begin("pairs");
   int nl = 0;
   // only PValue / Nsim asked for and Stat / Nmin of the same table are resident: no Gram tiles
-  const bool pv_only = use_null && !any_filter && (columns & 0x3Fu) == 0 && c.pairs_rows == total &&
+  const bool pv_only = use_null && !filtered && (columns & 0x3Fu) == 0 && c.pairs_rows == total &&
                        c.pairs_col_off[2] == (int64_t)off[2] && c.pairs_col_off[5] == (int64_t)off[5] &&
                        c.pairs_stat_id == stat_id && c.pairs_shard_index == shard_index && c.pairs_shard_count == shard_count;
   if (pv_only) {
@@ -571,7 +515,7 @@ int cmb_pairs_resident(cmb_ctx* ctx, int32_t stat_id, const cmb_filters* f, int3
   } else nl = launch_tiles(L, c.stream);
   c.prof_end(nl);
   int64_t kept = total;
-  if (any_filter && total > 0) {
+  if (filtered && total > 0) {
     int64_t* pos = nullptr;
     kept = compact_positions(total, L.o_keep, c.scratch2, &pos, c.stream);
     for (int k = 0; k < 8; k++) {
@@ -582,8 +526,7 @@ int cmb_pairs_resident(cmb_ctx* ctx, int32_t stat_id, const cmb_filters* f, int3
       c.prof.total_launches += 1;
     }
   }
-  if (any_filter || c.pairs_rows != kept) // filtered tables are only valid as one consistent call
-    for (auto& o : c.pairs_col_off) o = -1;
+  if (filtered || c.pairs_rows != kept) c.drop_pair_table(); // filtered tables are only valid as one consistent call
   for (int k = 0; k < 8; k++)
     if (columns >> k & 1) c.pairs_col_off[k] = (int64_t)off[k];
   c.pairs_rows = kept;
@@ -716,7 +659,7 @@ int cmb_cluster_null(cmb_ctx* ctx, int32_t dist_id, int32_t linkage, uint64_t se
     for (int q = 0; q < nb; q++) {
       const int rep = rep0 + q;
       // ClusterTools.cpp:224-227: simulate sizeOfDataSet sites, re-initialise, map
-      MapBuffers b = sim_buffers(c, 0, S, S_pad);
+      MapBuffers b = c.sim_buffers(0, S, S_pad);
       c.prof_begin("simulate");
       launch_simulate(m, c.sim_stream, seed, (int64_t)rep * S, S, 0, S, S_pad, weighted_classes, c.tree.n_nodes - 1,
                       c.s_tips[0].as<uint8_t>(), nullptr, c.stream);

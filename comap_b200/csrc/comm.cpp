@@ -11,7 +11,6 @@
 #include <mutex>
 
 namespace cmb {
-extern thread_local std::string g_last_error;
 
 namespace {
 // the slice of nccl.h this file needs (NCCL's C ABI is stable across 2.x)
@@ -66,20 +65,6 @@ void comm_all_gather(Context& c, const double* send, double* recv, size_t count)
 } // namespace cmb
 
 using namespace cmb;
-struct cmb_ctx { Context c; };
-
-#define CMB_TRY try {
-#define CMB_CATCH                                   \
-  }                                                 \
-  catch (const std::exception& e) {                 \
-    g_last_error = e.what();                        \
-    return 1;                                       \
-  }                                                 \
-  catch (...) {                                     \
-    g_last_error = "unknown error";                 \
-    return 1;                                       \
-  }                                                 \
-  return 0;
 
 extern "C" {
 

@@ -24,10 +24,21 @@ struct Error : std::runtime_error {
       ::cmb::fail("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__); \
   } while (0)
 
-// Device buffer that only grows (arena-style reuse across batches).
+inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
+
+// Device buffer that only grows (arena-style reuse across batches); frees its memory when destroyed.
 struct DevBuf {
   void* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  DevBuf& operator=(DevBuf&& o) noexcept {
+    if (this != &o) { release(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; }
+    return *this;
+  }
+  ~DevBuf() { release(); }
   void reserve(size_t bytes);
   void release();
   template <class T> T* as() const { return static_cast<T*>(p); }

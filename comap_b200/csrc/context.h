@@ -1,6 +1,9 @@
-// The context object behind cmb_ctx: one GPU, one stream, device arenas.
+// The context object behind cmb_ctx: one GPU, one stream, device arenas; and the scaffolding every C ABI
+// entry point shares (error capture, statistic ids).
 #pragma once
+#include "../../include/comap_b200.h"
 #include "kernels.h"
+#include <algorithm>
 #include <memory>
 
 namespace cmb {
@@ -24,6 +27,12 @@ struct NullState {            // binned, sorted null distribution (device + host
   std::vector<int64_t> bin_off;
   bool ready = false;
   bool nmax_from_map = false;  // nmax was taken from the mapped alignment's max(norm) (nmax < 0 at load time)
+  void begin(int64_t n) {     // a new arena of n raw samples; the binned distribution is stale
+    ready = false;
+    stat.reserve(sizeof(double) * (size_t)std::max<int64_t>(n, 1));
+    nmin.reserve(sizeof(double) * (size_t)std::max<int64_t>(n, 1));
+    n_samples = n;
+  }
 };
 
 struct Context {
@@ -61,7 +70,7 @@ struct Context {
   DevBuf d_tips;                 // [T][S_pad]
   std::vector<uint32_t> code_mask;
   bool have_alignment = false, mapped = false;
-  DevBuf d_D, d_Lc, d_invL, d_loglik, d_pr, d_rc, d_out, d_sum, d_sumsq;
+  DevBuf d_D, d_Lc, d_invL, d_loglik, d_pr, d_rc, d_out;
   double *h_norm = nullptr, *h_loglik = nullptr; // pinned host copies [S] used by null / pairs / the saturation check
   size_t h_cap = 0;
   // cmb_map without host outputs is deferred: enqueued on a side stream so that what the caller enqueues next
@@ -70,19 +79,23 @@ struct Context {
   cudaEvent_t map_begin = nullptr, map_done = nullptr;
   bool map_pending = false;
   DevBuf k1_part_obs;            // per-class partial outputs of the observed alignment's protein mapping
-  void wait_map();               // block until a deferred mapping has left the device (no checks)
+  void cancel_map();             // block until a deferred mapping has left the device and drop it (no checks)
   void finish_map();             // ... and complete it: max norm, saturated sites (throws), ordering of the main stream
   void finalize_map_host();
   double max_norm = 0.;
 
   // scratch for simulated batches
-  DevBuf s_tips[2], s_D, s_Lc, s_invL, s_loglik, s_pr[2], s_rc[2], s_out[2], s_sum[2], s_sumsq[2], s_cls;
+  DevBuf s_tips[2], s_D, s_Lc, s_invL, s_loglik, s_pr[2], s_rc[2], s_out[2], s_cls;
   DevBuf d_identity_mask;
   DevBuf s_cols, s_counts;       // pattern compression of simulated batches: column of every site, {sites to map, varied} per batch
   int s_batches = 0;
   int64_t null_budget_sites = 0;  // simulated sites the null may hold at once (from free memory, cached)
   const void* s_tips_ptr = nullptr;
   int64_t s_tips_pad = -1, s_tips_n = -1; // geometry the simulated tip buffer's padding columns were cleared for
+  MapBuffers sim_buffers(int k, int64_t n, int64_t n_pad); // mapping buffers of n simulated sites, tips in s_tips[k]
+  // s_tips[0] holds two batches of n sites at columns [0, n) and [half, half + n); the columns between and after them
+  // are mapped too (their results are never read): give them a valid state once per buffer geometry
+  void clear_sim_tip_padding(int64_t n, int64_t n_pad);
 
   NullState null;
 
@@ -108,6 +121,7 @@ struct Context {
   cudaEvent_t copy_event = nullptr;
   int64_t pairs_col_off[8] = {-1, -1, -1, -1, -1, -1, -1, -1}; // resident pair columns in `pair_table`
   int64_t pairs_rows = -1;
+  void drop_pair_table() { pairs_rows = -1; for (auto& o : pairs_col_off) o = -1; }
   int pairs_stat_id = -1, pairs_shard_index = -1, pairs_shard_count = -1; // what the resident columns belong to
   DevBuf pairs_mean, pairs_sd, pairs_norm; // per-site mean / sd / norm for the tile kernels
   // corrected correlation (Statistics.h:176-205): mean vector of the mapped alignment and the
@@ -142,5 +156,36 @@ struct Context {
 
 int64_t pad_sites(int64_t n);
 void comm_all_gather(Context& c, const double* send, double* recv, size_t count);
+// bins and sorts n device-resident samples into c.null (nmax < 0: the mapped alignment's max(norm))
+void null_load(Context& c, const double* stat_dev, const double* nmin_dev, int64_t n, int K, double nmax);
+// bytes of device memory one simulated site needs through simulate -> map x2 -> paired
+size_t null_bytes_per_site(const Context& c);
+
+inline void check_stat(int stat_id) {
+  if (stat_id < 0 || stat_id > CMB_STAT_MI_LABEL) fail("unknown statistic id %d", stat_id);
+}
+// whether any of the pair filters can drop a row
+inline bool any_filter(const cmb_filters* f) {
+  return f && (f->min_rate_class > 0 || f->min_rate > 0. || f->max_rate_class_diff >= 0 || f->max_rate_diff >= 0. ||
+               f->min_stat > 0.);
+}
+
+extern thread_local std::string g_last_error; // defined in capi.cu
 
 } // namespace cmb
+
+struct cmb_ctx { cmb::Context c; };
+
+// Every C ABI entry point returns 0, or 1 with the message for cmb_last_error.
+#define CMB_TRY try {
+#define CMB_CATCH                                   \
+  }                                                 \
+  catch (const std::exception& e) {                 \
+    ::cmb::g_last_error = e.what();                 \
+    return 1;                                       \
+  }                                                 \
+  catch (...) {                                     \
+    ::cmb::g_last_error = "unknown error";          \
+    return 1;                                       \
+  }                                                 \
+  return 0;

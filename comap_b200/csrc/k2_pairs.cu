@@ -835,7 +835,7 @@ size_t compress_reserve(int64_t n_pad, DevBuf& tmp, size_t* scan_bytes) {
   if (n_pad > 0x7fffffff) fail("internal: batch too large for 32-bit column indices");
   size_t need = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, need, (const int32_t*)nullptr, (int32_t*)nullptr, (int)n_pad, nullptr);
-  const size_t a = ((size_t)n_pad * 4 + 255) & ~size_t(255);
+  const size_t a = align256((size_t)n_pad * 4);
   tmp.reserve(3 * a + need + 256);
   *scan_bytes = need;
   return a;
@@ -900,7 +900,7 @@ int bin_and_sort(int64_t n, const double* stat, const double* nmin, int K, doubl
   cub::DeviceRadixSort::SortPairs(nullptr, need2, (const uint32_t*)nullptr, (uint32_t*)nullptr, (const double*)nullptr,
                                   (double*)nullptr, (int)n, 0, 32, st);
   size_t need = need1 > need2 ? need1 : need2;
-  size_t a = ((size_t)n * 4 + 255) & ~size_t(255), d = ((size_t)n * 8 + 255) & ~size_t(255);
+  size_t a = align256((size_t)n * 4), d = align256((size_t)n * 8);
   tmp.reserve(2 * a + d + need + 256);
   unsigned char* base = tmp.as<unsigned char>();
   uint32_t* cat = (uint32_t*)base;
@@ -991,7 +991,7 @@ int launch_inter_diagonal(const TilesLaunch& L, cudaStream_t st) {
 int64_t compact_positions(int64_t n, const uint8_t* keep, DevBuf& tmp, int64_t** pos_out, cudaStream_t st) {
   size_t need = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, need, (const int64_t*)nullptr, (int64_t*)nullptr, (int)n, st);
-  size_t a = ((size_t)n * 8 + 255) & ~size_t(255);
+  size_t a = align256((size_t)n * 8);
   tmp.reserve(2 * a + need + 256);
   int64_t* flags = tmp.as<int64_t>();
   int64_t* pos = (int64_t*)(tmp.as<unsigned char>() + a);

@@ -738,12 +738,12 @@ __global__ void k4_group_compensation(int64_t n_groups, const int32_t* __restric
 namespace {
 ClusterParams make_params(int64_t S, int linkage, double* mat, DevBuf& work, int32_t* left_dev, int32_t* right_dev,
                           double* height_dev, cudaStream_t st) {
-  auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
-  size_t o_val = 0, o_idx = al(o_val + 8 * S), o_alive = al(o_idx + 4 * S), o_len = al(o_alive + S),
-         o_nl = al(o_len + 8 * S), o_node = al(o_nl + 4 * S), o_wl = al(o_node + 4 * S), o_wlc = al(o_wl + 8 * S),
-         o_pv = al(o_wlc + 64), o_pi = al(o_pv + 8 * 1024), o_sv = al(o_pi + 4 * 1024), o_si = al(o_sv + 8 * 1024),
-         o_sc = al(o_si + 4 * 1024),
-         o_gv = al(o_sc + 4 * 1024), o_gi = al(o_gv + 8 * 1024), o_gc = al(o_gi + 4 * 1024), o_end = al(o_gc + 4 * 1024);
+  size_t o_val = 0, o_idx = align256(o_val + 8 * S), o_alive = align256(o_idx + 4 * S), o_len = align256(o_alive + S),
+         o_nl = align256(o_len + 8 * S), o_node = align256(o_nl + 4 * S), o_wl = align256(o_node + 4 * S),
+         o_wlc = align256(o_wl + 8 * S), o_pv = align256(o_wlc + 64), o_pi = align256(o_pv + 8 * 1024),
+         o_sv = align256(o_pi + 4 * 1024), o_si = align256(o_sv + 8 * 1024), o_sc = align256(o_si + 4 * 1024),
+         o_gv = align256(o_sc + 4 * 1024), o_gi = align256(o_gv + 8 * 1024), o_gc = align256(o_gi + 4 * 1024),
+         o_end = align256(o_gc + 4 * 1024);
   work.reserve(o_end);
   unsigned char* w = work.as<unsigned char>();
   ClusterParams p;

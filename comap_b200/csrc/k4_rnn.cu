@@ -369,9 +369,8 @@ bool cluster_rnn_selected(int64_t S, int linkage) {
 // creation order.  Returns the number of kernel launches.
 int launch_cluster_rnn(int64_t S, int linkage, double* mat, DevBuf& work, int32_t* left_dev, int32_t* right_dev,
                        double* height_dev, cudaStream_t st) {
-  auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
   size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o = al(o + bytes); return at; };
+  auto take = [&](size_t bytes) { size_t at = o; o = align256(o + bytes); return at; };
   const size_t o_alive = take(S), o_len = take(8 * S), o_nl = take(4 * S), o_node = take(4 * S), o_nv = take(8 * S),
                o_ni = take(4 * S), o_dirty = take(4 * S), o_role = take(8 * S), o_wl = take(8 * S), o_pi = take(4 * (S / 2 + 2)),
                o_pj = take(4 * (S / 2 + 2)), o_pd = take(8 * (S / 2 + 2)), o_w1 = take(8 * (S / 2 + 2)), o_w2 = take(8 * (S / 2 + 2)),

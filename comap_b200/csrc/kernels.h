@@ -11,7 +11,6 @@ struct DevStream {           // an OpStream uploaded to the device
   uint32_t stage_bytes = 0;
   uint32_t blk_off_max[3] = {0, 0, 0};
   void upload(const OpStream& s, cudaStream_t st);
-  void release();
 };
 
 struct ChunkMeta {           // kernel-side view of a DevStream
