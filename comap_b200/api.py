@@ -34,6 +34,7 @@ SYMBOLS = [
     "cmb_mica_sites", "cmb_mica_pairs", "cmb_mica_pair_list", "cmb_mica_permutations", "cmb_mica_null_parametric", "cmb_null_load",
     "cmb_comm_unique_id", "cmb_comm_init", "cmb_comm_init_all", "cmb_comm_set", "cmb_comm_destroy", "cmb_comm_rank",
     "cmb_comm_group_start", "cmb_comm_group_end", "cmb_null_intra_sharded", "cmb_set_continuous_rates",
+    "cmb_mica_permutations_shard", "cmb_mica_null_parametric_range", "cmb_mica_null_parametric_sharded", "cmb_null_inter_range",
 ]
 
 
@@ -225,21 +226,38 @@ class Context:
                                               b.ctypes.data_as(C.POINTER(C.c_int32)), _d(mi), _d(hj)))
         return mi, hj
 
-    def mica_permutations(self, seed, max_permutations=1000):
-        """null.method = permutations (miTest, Mica.cpp:92-118): Perm.p.value and Perm.nb of every pair, mica's order."""
+    def mica_permutations(self, seed, max_permutations=1000, shard_index=0, shard_count=1):
+        """null.method = permutations (miTest, Mica.cpp:92-118): Perm.p.value and Perm.nb of every pair, mica's order.
+        shard_count > 1: only the pairs idx = shard_index + k * shard_count, row k holding pair idx."""
         n = self.S * (self.S - 1) // 2
+        n = max(0, (n - 1 - shard_index) // shard_count + 1) if 0 <= shard_index < shard_count else 0
         pv = np.empty(n); nb = np.empty(n, np.int32)
         k = C.c_int64(0)
-        self._chk(self.lib.cmb_mica_permutations(self.h, C.c_uint64(seed), int(max_permutations), C.c_int64(n), _d(pv),
-                                                 nb.ctypes.data_as(C.POINTER(C.c_int32)), C.byref(k)))
+        self._chk(self.lib.cmb_mica_permutations_shard(self.h, C.c_uint64(seed), int(max_permutations), int(shard_index),
+                                                       int(shard_count), C.c_int64(n), _d(pv), _i32(nb), C.byref(k)))
         assert k.value == n
         return pv, nb
 
-    def mica_null_parametric(self, seed, rep_cpu, rep_ram, K=10, nmax=-1.0, weighted_classes=False):
-        """null.method = parametric-bootstrap (Mica.cpp:470-545); returns the [n][3] rows MI, Hjoint, Nmin."""
-        raw = np.empty((rep_cpu * rep_ram, 3))
-        self._chk(self.lib.cmb_mica_null_parametric(self.h, C.c_uint64(seed), int(rep_cpu), int(rep_ram), int(bool(weighted_classes)),
-                                                    int(K), C.c_double(nmax), _d(raw)))
+    def mica_null_parametric(self, seed, rep_cpu, rep_ram, K=10, nmax=-1.0, weighted_classes=False, rep_begin=0, rep_end=None):
+        """null.method = parametric-bootstrap (Mica.cpp:470-545); returns the [n][3] rows MI, Hjoint, Nmin of the outer
+        replicates [rep_begin, rep_end) (default: all of them)."""
+        rep_end = rep_cpu if rep_end is None else rep_end
+        raw = np.empty((max(0, rep_end - rep_begin) * rep_ram, 3))
+        self._chk(self.lib.cmb_mica_null_parametric_range(self.h, C.c_uint64(seed), int(rep_cpu), int(rep_ram), int(rep_begin),
+                                                          int(rep_end), int(bool(weighted_classes)), int(K), C.c_double(nmax),
+                                                          _d(raw)))
+        return raw
+
+    def mica_null_parametric_sharded(self, seed, rep_cpu, rep_ram, K=10, nmax=-1.0, weighted_classes=False, want_raw=False):
+        """This rank's share of the parametric-bootstrap replicates, all-gather of the (MI, Nmin) samples and binning of
+        the union (cmb_mica_null_parametric_sharded).  want_raw: the rows of this rank's replicates."""
+        raw = None
+        if want_raw:
+            rank, n = self.comm_rank()
+            q, m = divmod(rep_cpu, n)
+            raw = np.empty(((q + (1 if rank < m else 0)) * rep_ram, 3))
+        self._chk(self.lib.cmb_mica_null_parametric_sharded(self.h, C.c_uint64(seed), int(rep_cpu), int(rep_ram),
+                                                            int(bool(weighted_classes)), int(K), C.c_double(nmax), _d(raw)))
         return raw
 
     def null_load(self, stat, key, K, kmax):
@@ -377,12 +395,13 @@ class Context:
         k = nr.value
         return dict(i=oi[:k], j=oj[:k], stat=st[:k], rcmin=rcm[:k], prmin=prm[:k], nmin=nm[:k]), k
 
-    def null_inter(self, other, stat, seed, rep_cpu, rep_ram, weighted_classes=False):
+    def null_inter(self, other, stat, seed, rep_cpu, rep_ram, weighted_classes=False, rep_begin=0, rep_end=None):
         """rep_cpu x rep_ram paired null statistics of the two data sets' simulators
-        (AnalysisTools.cpp:662-735); rows Stat, RCmin, PRmin, Nmin."""
-        raw = np.empty((rep_cpu * rep_ram, 4))
-        self._chk(self.lib.cmb_null_inter(self.h, other.h, STAT[stat], C.c_uint64(seed), rep_cpu, rep_ram,
-                                          int(weighted_classes), _d(raw)))
+        (AnalysisTools.cpp:662-735); rows Stat, RCmin, PRmin, Nmin of the outer replicates [rep_begin, rep_end)."""
+        rep_end = rep_cpu if rep_end is None else rep_end
+        raw = np.empty((max(0, rep_end - rep_begin) * rep_ram, 4))
+        self._chk(self.lib.cmb_null_inter_range(self.h, other.h, STAT[stat], C.c_uint64(seed), rep_cpu, rep_ram,
+                                                rep_begin, rep_end, int(weighted_classes), _d(raw)))
         return raw
 
     COLS = ("i", "j", "stat", "rcmin", "prmin", "nmin", "pvalue", "nsim")

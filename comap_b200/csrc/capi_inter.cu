@@ -6,7 +6,8 @@
 //                    with per-data-set rate thresholds, rows in the reference's order.
 //   cmb_null_inter   replaces AnalysisTools::getNullDistributionInterDR (AnalysisTools.cpp:662-735):
 //                    rep_cpu x { simulate rep_ram sites under each data set's model, map both,
-//                    paired statistic j<->j }, rows Stat RCmin PRmin Nmin.
+//                    paired statistic j<->j }, rows Stat RCmin PRmin Nmin; cmb_null_inter_range
+//                    computes the rows of a range of outer replicates (a GPU's share).
 // Each data set lives in its own context (tree, model, alignment, mapping); both must be on the
 // same device.  The kernels are K2's (rectangle mode of k2_tiles, k2_paired) and K1/K3.
 #include "../../include/comap_b200.h"
@@ -140,14 +141,15 @@ int cmb_pairs_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, const cmb_fil
   CMB_CATCH
 }
 
-int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed, int32_t rep_cpu, int32_t rep_ram,
-                   int32_t weighted_classes, double* raw) {
+int cmb_null_inter_range(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed, int32_t rep_cpu, int32_t rep_ram,
+                         int32_t rep_begin, int32_t rep_end, int32_t weighted_classes, double* raw) {
   CMB_TRY
   Context& c = ctx1->c;
   Context& d = ctx2->c;
   CMB_CUDA(cudaSetDevice(c.device));
   check_stat(stat_id);
   if (rep_ram < 1 || rep_cpu < 0) fail("cmb_null_inter: bad replicate counts");
+  if (rep_begin < 0 || rep_end > rep_cpu || rep_begin > rep_end) fail("cmb_null_inter: bad replicate range");
   if (!raw) fail("cmb_null_inter: raw output buffer required");
   check_pair(c, d, "cmb_null_inter");
   c.ensure_streams();
@@ -156,7 +158,7 @@ int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed,
   const double* mv1 = corrected ? c.mean_vector() : nullptr;
   const double* mv2 = corrected ? d.mean_vector() : nullptr;
   const int B = c.tree.B;
-  const int64_t R = rep_ram, total = (int64_t)rep_cpu * R;
+  const int64_t R = rep_ram, total = (int64_t)(rep_end - rep_begin) * R;
   c.null.begin(total);
   // batch outer replicates: the two data sets' partials are alive at the same time
   size_t freeb = 0, totalb = 0;
@@ -169,8 +171,8 @@ int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed,
   const uint64_t seed2 = seed ^ 0x9E3779B97F4A7C15ull;
   MapModel m1 = c.map_model(), m2 = d.map_model();
   int64_t off = 0;
-  for (int64_t r0 = 0; r0 < rep_cpu; r0 += rpb) {
-    const int64_t nb = std::min<int64_t>(rpb, rep_cpu - r0), n = nb * R;
+  for (int64_t r0 = rep_begin; r0 < rep_end; r0 += rpb) {
+    const int64_t nb = std::min<int64_t>(rpb, rep_end - r0), n = nb * R;
     const int64_t np1 = pad_sites(n), np2 = pad_sites(n);
     MapBuffers b1 = c.sim_buffers(0, n, np1), b2 = d.sim_buffers(0, n, np2);
     c.prof_begin("simulate");
@@ -197,6 +199,11 @@ int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed,
     off += n;
   }
   CMB_CATCH
+}
+
+int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed, int32_t rep_cpu, int32_t rep_ram,
+                   int32_t weighted_classes, double* raw) {
+  return cmb_null_inter_range(ctx1, ctx2, stat_id, seed, rep_cpu, rep_ram, 0, rep_cpu, weighted_classes, raw);
 }
 
 } // extern "C"

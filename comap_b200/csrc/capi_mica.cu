@@ -46,6 +46,55 @@ void ensure_mica(Context& c) {
   c.mica_ready = true;
 }
 
+// Mica.cpp:505-541 over the outer replicates [rep_begin, rep_end): two simulated alignments of rep_ram sites per
+// replicate, their mappings for the norms (computeSubstitutionVectors, whatever nijt.average says), MI and joint
+// entropy of site j with site j.  The simulator is keyed by the global site 2 r rep_ram, so ranges concatenate to the
+// whole null; c.null holds this range's samples, raw (nullable) its rows.
+void mica_null_core(Context& c, uint64_t seed, int rep_cpu, int rep_ram, int rep_begin, int rep_end, int weighted_classes, int K,
+                    double nmax, double* raw) {
+  CMB_CUDA(cudaSetDevice(c.device));
+  c.ensure_streams();
+  if (rep_cpu < 1 || rep_ram < 1) fail("cmb_mica_null_parametric: rep_cpu and rep_ram must be positive");
+  if (rep_begin < 0 || rep_end > rep_cpu || rep_begin > rep_end) fail("cmb_mica_null_parametric: bad replicate range");
+  const int B = c.tree.B, T = c.tree.n_leaves;
+  const int64_t R = rep_ram, total = (int64_t)(rep_end - rep_begin) * R;
+  NullState& ns = c.null;
+  ns.begin(total);
+  MapModel m = c.map_model();
+  const uint32_t* ident = c.d_identity_mask.as<uint32_t>();
+  const int64_t half = (R + 255) / 256 * 256, n_pad = pad_sites(half + R);
+  for (int64_t r = rep_begin; r < rep_end; r++) {
+    const int64_t o = (r - rep_begin) * R;              // this replicate's first sample of the range
+    MapBuffers bb = c.sim_buffers(0, half + R, n_pad);
+    uint8_t* tips = c.s_tips[0].as<uint8_t>();
+    c.clear_sim_tip_padding(R, n_pad);
+    c.prof_begin("simulate");
+    launch_simulate(m, c.sim_stream, seed, 2 * r * R, R, 2 * R, 2 * R, n_pad, weighted_classes, c.tree.n_nodes - 1, tips, nullptr,
+                    c.stream, R, half, R);
+    c.prof_end(1);
+    c.run_map(bb, true, true, false);
+    c.scratch.reserve(sizeof(double) * 4 * (size_t)n_pad);
+    double* prep = c.scratch.as<double>();             // mean | sd | norm of the mapped batch pair
+    launch_prep(B, half + R, n_pad, bb.out, nullptr, prep, prep + n_pad, prep + 2 * n_pad, c.stream);
+    double* hj = prep + 3 * n_pad;
+    c.prof_begin("mica_null");
+    launch_mica_listed(c.A, T, R, tips, n_pad, tips + half, n_pad, nullptr, nullptr, ident, ns.stat.as<double>() + o, hj, c.stream);
+    launch_min2(R, prep + 2 * n_pad, prep + 2 * n_pad + half, ns.nmin.as<double>() + o, c.stream);
+    c.prof_end(3);
+    if (raw) { // rows of null.output.file: MI, Hjoint, Nmin
+      std::vector<double> h_mi(R), h_hj(R), h_nm(R);
+      CMB_CUDA(cudaMemcpyAsync(h_mi.data(), ns.stat.as<double>() + o, sizeof(double) * R, cudaMemcpyDeviceToHost, c.stream));
+      CMB_CUDA(cudaMemcpyAsync(h_hj.data(), hj, sizeof(double) * R, cudaMemcpyDeviceToHost, c.stream));
+      CMB_CUDA(cudaMemcpyAsync(h_nm.data(), ns.nmin.as<double>() + o, sizeof(double) * R, cudaMemcpyDeviceToHost, c.stream));
+      CMB_CUDA(cudaStreamSynchronize(c.stream));
+      for (int64_t j = 0; j < R; j++) { raw[(o + j) * 3] = h_mi[j]; raw[(o + j) * 3 + 1] = h_hj[j]; raw[(o + j) * 3 + 2] = h_nm[j]; }
+    }
+    c.prof.sites_simulated += 2 * R;
+  }
+  if (K > 0) null_load(c, ns.stat.as<double>(), ns.nmin.as<double>(), total, K, nmax);
+  else CMB_CUDA(cudaStreamSynchronize(c.stream));
+}
+
 } // namespace
 
 extern "C" {
@@ -115,15 +164,18 @@ int cmb_mica_pair_list(cmb_ctx* ctx, int64_t n, const int32_t* site1, const int3
   CMB_CATCH
 }
 
-int cmb_mica_permutations(cmb_ctx* ctx, uint64_t seed, int32_t max_permutations, int64_t capacity, double* pvalue, int32_t* nperm,
-                          int64_t* n_rows) {
+int cmb_mica_permutations_shard(cmb_ctx* ctx, uint64_t seed, int32_t max_permutations, int32_t shard_index, int32_t shard_count,
+                                int64_t capacity, double* pvalue, int32_t* nperm, int64_t* n_rows) {
   CMB_TRY
   Context& c = ctx->c;
   CMB_CUDA(cudaSetDevice(c.device));
   if (!c.have_alignment) fail("cmb_mica_permutations: call cmb_set_alignment first");
   if (c.S < 2) fail("mica: at least two sites are needed");
   if (max_permutations < 1) fail("Permutation number should be greater than 0!"); // Mica.cpp:611-614
-  const int64_t n = c.S * (c.S - 1) / 2;
+  if (shard_count < 1 || shard_index < 0 || shard_index >= shard_count)
+    fail("cmb_mica_permutations: bad shard %d of %d", shard_index, shard_count);
+  const int64_t n_pairs = c.S * (c.S - 1) / 2;
+  const int64_t n = shard_index < n_pairs ? (n_pairs - 1 - shard_index) / shard_count + 1 : 0; // idx = shard_index + k shard_count
   if (capacity < n) fail("cmb_mica_permutations: capacity %lld < %lld pairs", (long long)capacity, (long long)n);
   const size_t d = align256(sizeof(double) * (size_t)n), w = align256(sizeof(int32_t) * (size_t)n);
   c.scratch.reserve(d + w + 256);
@@ -132,60 +184,44 @@ int cmb_mica_permutations(cmb_ctx* ctx, uint64_t seed, int32_t max_permutations,
   unsigned long long* next = (unsigned long long*)(c.scratch.as<unsigned char>() + d + w); // the kernel's work counter
   c.prof_begin("mica_perm");
   launch_mica_permutations(c.A, c.tree.n_leaves, c.S, c.S_pad, c.d_tips.as<uint8_t>(), c.d_code_mask.as<uint32_t>(), seed,
-                           max_permutations, next, pv, np, c.stream);
-  c.prof_end(2);
-  if (pvalue) CMB_CUDA(cudaMemcpyAsync(pvalue, pv, sizeof(double) * n, cudaMemcpyDeviceToHost, c.stream));
-  if (nperm) CMB_CUDA(cudaMemcpyAsync(nperm, np, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, c.stream));
+                           max_permutations, shard_index, shard_count, n, next, pv, np, c.stream);
+  c.prof_end(n > 0 ? 2 : 0);
+  if (pvalue && n > 0) CMB_CUDA(cudaMemcpyAsync(pvalue, pv, sizeof(double) * n, cudaMemcpyDeviceToHost, c.stream));
+  if (nperm && n > 0) CMB_CUDA(cudaMemcpyAsync(nperm, np, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, c.stream));
   CMB_CUDA(cudaStreamSynchronize(c.stream));
   if (n_rows) *n_rows = n;
   CMB_CATCH
 }
 
+int cmb_mica_permutations(cmb_ctx* ctx, uint64_t seed, int32_t max_permutations, int64_t capacity, double* pvalue, int32_t* nperm,
+                          int64_t* n_rows) {
+  return cmb_mica_permutations_shard(ctx, seed, max_permutations, 0, 1, capacity, pvalue, nperm, n_rows);
+}
+
+int cmb_mica_null_parametric_range(cmb_ctx* ctx, uint64_t seed, int32_t rep_cpu, int32_t rep_ram, int32_t rep_begin, int32_t rep_end,
+                                   int32_t weighted_classes, int32_t K, double nmax, double* raw) {
+  CMB_TRY
+  mica_null_core(ctx->c, seed, rep_cpu, rep_ram, rep_begin, rep_end, weighted_classes, K, nmax, raw);
+  CMB_CATCH
+}
+
 int cmb_mica_null_parametric(cmb_ctx* ctx, uint64_t seed, int32_t rep_cpu, int32_t rep_ram, int32_t weighted_classes, int32_t K,
                              double nmax, double* raw) {
+  return cmb_mica_null_parametric_range(ctx, seed, rep_cpu, rep_ram, 0, rep_cpu, weighted_classes, K, nmax, raw);
+}
+
+int cmb_mica_null_parametric_sharded(cmb_ctx* ctx, uint64_t seed, int32_t rep_cpu, int32_t rep_ram, int32_t weighted_classes,
+                                     int32_t K, double nmax, double* raw) {
   CMB_TRY
   Context& c = ctx->c;
-  CMB_CUDA(cudaSetDevice(c.device));
-  c.ensure_streams();
-  if (rep_cpu < 1 || rep_ram < 1) fail("cmb_mica_null_parametric: rep_cpu and rep_ram must be positive");
-  const int B = c.tree.B, T = c.tree.n_leaves;
-  const int64_t R = rep_ram, total = (int64_t)rep_cpu * R;
-  NullState& ns = c.null;
-  ns.begin(total);
-  MapModel m = c.map_model();
-  const uint32_t* ident = c.d_identity_mask.as<uint32_t>();
-  // Mica.cpp:505-541, one outer replicate at a time: two simulated alignments of rep_ram sites, their mappings for the
-  // norms (computeSubstitutionVectors, whatever nijt.average says), MI and joint entropy of site j with site j
-  const int64_t half = (R + 255) / 256 * 256, n_pad = pad_sites(half + R);
-  for (int64_t r = 0; r < rep_cpu; r++) {
-    MapBuffers bb = c.sim_buffers(0, half + R, n_pad);
-    uint8_t* tips = c.s_tips[0].as<uint8_t>();
-    c.clear_sim_tip_padding(R, n_pad);
-    c.prof_begin("simulate");
-    launch_simulate(m, c.sim_stream, seed, 2 * r * R, R, 2 * R, 2 * R, n_pad, weighted_classes, c.tree.n_nodes - 1, tips, nullptr,
-                    c.stream, R, half, R);
-    c.prof_end(1);
-    c.run_map(bb, true, true, false);
-    c.scratch.reserve(sizeof(double) * 4 * (size_t)n_pad);
-    double* prep = c.scratch.as<double>();             // mean | sd | norm of the mapped batch pair
-    launch_prep(B, half + R, n_pad, bb.out, nullptr, prep, prep + n_pad, prep + 2 * n_pad, c.stream);
-    double* hj = prep + 3 * n_pad;
-    c.prof_begin("mica_null");
-    launch_mica_listed(c.A, T, R, tips, n_pad, tips + half, n_pad, nullptr, nullptr, ident, ns.stat.as<double>() + r * R, hj, c.stream);
-    launch_min2(R, prep + 2 * n_pad, prep + 2 * n_pad + half, ns.nmin.as<double>() + r * R, c.stream);
-    c.prof_end(3);
-    if (raw) { // rows of null.output.file: MI, Hjoint, Nmin
-      std::vector<double> h_mi(R), h_hj(R), h_nm(R);
-      CMB_CUDA(cudaMemcpyAsync(h_mi.data(), ns.stat.as<double>() + r * R, sizeof(double) * R, cudaMemcpyDeviceToHost, c.stream));
-      CMB_CUDA(cudaMemcpyAsync(h_hj.data(), hj, sizeof(double) * R, cudaMemcpyDeviceToHost, c.stream));
-      CMB_CUDA(cudaMemcpyAsync(h_nm.data(), ns.nmin.as<double>() + r * R, sizeof(double) * R, cudaMemcpyDeviceToHost, c.stream));
-      CMB_CUDA(cudaStreamSynchronize(c.stream));
-      for (int64_t j = 0; j < R; j++) { raw[(r * R + j) * 3] = h_mi[j]; raw[(r * R + j) * 3 + 1] = h_hj[j]; raw[(r * R + j) * 3 + 2] = h_nm[j]; }
-    }
-    c.prof.sites_simulated += 2 * R;
+  if (c.comm_size == 1) { // no communicator: the whole null on this GPU
+    mica_null_core(c, seed, rep_cpu, rep_ram, 0, rep_cpu, weighted_classes, K, nmax, raw);
+    return 0;
   }
-  if (K > 0) null_load(c, ns.stat.as<double>(), ns.nmin.as<double>(), total, K, nmax);
-  else CMB_CUDA(cudaStreamSynchronize(c.stream));
+  int r0, r1;
+  replicate_range(rep_cpu, c.comm_size, c.comm_rank, r0, r1);
+  mica_null_core(c, seed, rep_cpu, rep_ram, r0, r1, weighted_classes, 0, 0., raw);
+  if (K > 0) gather_null_shards(c, rep_cpu, rep_ram, K, nmax);
   CMB_CATCH
 }
 

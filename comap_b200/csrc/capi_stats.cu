@@ -42,6 +42,47 @@ void null_load(Context& c, const double* stat_dev, const double* nmin_dev, int64
   ns.ready = true;
 }
 
+void replicate_range(int rep_cpu, int n_ranks, int rank, int& begin, int& end) {
+  const int q = rep_cpu / n_ranks, r = rep_cpu % n_ranks;
+  begin = rank * q + std::min(rank, r);
+  end = begin + q + (rank < r ? 1 : 0);
+}
+
+__global__ void k_fill_nan(double* p, int64_t n) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) p[i] = nan("");
+}
+
+void gather_null_shards(Context& c, int rep_cpu, int rep_ram, int K, double nmax) {
+  // every rank contributes one block [stat (cap) | nmin (cap)], cap = the largest shard; unused entries carry
+  // Nmin = NaN, which Domain::getIndex rejects, so they fall out of the binning like out-of-range samples
+  const int64_t R = rep_ram, n = c.null.n_samples;
+  const int64_t cap = ((int64_t)(rep_cpu + c.comm_size - 1) / c.comm_size) * R;
+  c.gather_send.reserve(sizeof(double) * 2 * (size_t)cap);
+  c.gather_recv.reserve(sizeof(double) * 2 * (size_t)cap * c.comm_size);
+  double* send = c.gather_send.as<double>();
+  if (n < cap) {
+    k_fill_nan<<<(unsigned)((2 * cap + 255) / 256), 256, 0, c.stream>>>(send, 2 * cap);
+    CMB_CUDA(cudaGetLastError());
+    c.prof.total_launches += 1;
+  }
+  if (n > 0) {
+    CMB_CUDA(cudaMemcpyAsync(send, c.null.stat.p, sizeof(double) * n, cudaMemcpyDeviceToDevice, c.stream));
+    CMB_CUDA(cudaMemcpyAsync(send + cap, c.null.nmin.p, sizeof(double) * n, cudaMemcpyDeviceToDevice, c.stream));
+  }
+  comm_all_gather(c, send, c.gather_recv.as<double>(), 2 * (size_t)cap);
+  // blocks [stat | nmin] per rank -> two contiguous arrays of comm_size * cap samples
+  const int64_t tot = cap * c.comm_size;
+  c.null.stat.reserve(sizeof(double) * (size_t)tot);
+  c.null.nmin.reserve(sizeof(double) * (size_t)tot);
+  CMB_CUDA(cudaMemcpy2DAsync(c.null.stat.p, sizeof(double) * cap, c.gather_recv.p, sizeof(double) * 2 * cap,
+                             sizeof(double) * cap, c.comm_size, cudaMemcpyDeviceToDevice, c.stream));
+  CMB_CUDA(cudaMemcpy2DAsync(c.null.nmin.p, sizeof(double) * cap, c.gather_recv.as<double>() + cap, sizeof(double) * 2 * cap,
+                             sizeof(double) * cap, c.comm_size, cudaMemcpyDeviceToDevice, c.stream));
+  c.null.n_samples = tot;
+  null_load(c, c.null.stat.as<double>(), c.null.nmin.as<double>(), tot, K, nmax);
+}
+
 } // namespace cmb
 
 namespace {
@@ -148,17 +189,6 @@ void null_core(Context& c, int stat_id, uint64_t seed, int rep_cpu, int rep_ram,
   else if (!c.async_null) CMB_CUDA(cudaStreamSynchronize(c.stream));
 }
 
-// This rank's share of the outer replicates: contiguous ranges, the first rep_cpu % n_ranks ranks get one more.
-void replicate_range(int rep_cpu, int n_ranks, int rank, int& begin, int& end) {
-  const int q = rep_cpu / n_ranks, r = rep_cpu % n_ranks;
-  begin = rank * q + std::min(rank, r);
-  end = begin + q + (rank < r ? 1 : 0);
-}
-
-__global__ void k_fill_nan(double* p, int64_t n) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) p[i] = nan("");
-}
 
 struct GroupTable {
   std::vector<int32_t> members;
@@ -338,33 +368,7 @@ int cmb_null_intra_sharded(cmb_ctx* ctx, int32_t stat_id, uint64_t seed, int32_t
   c.async_null = true; // no host wait between the last null kernel and the exchange
   struct Restore { Context& c; bool v; ~Restore() { c.async_null = v; } } restore{c, was_async};
   null_core(c, stat_id, seed, rep_cpu, rep_ram, r0, r1, weighted_classes, 0, 0., raw, nullptr, nullptr);
-  // every rank contributes one block [stat (cap) | nmin (cap)], cap = the largest shard; unused entries carry
-  // Nmin = NaN, which Domain::getIndex rejects, so they fall out of the binning like out-of-range samples
-  const int64_t R = rep_ram, n = (int64_t)(r1 - r0) * R;
-  const int64_t cap = ((int64_t)(rep_cpu + c.comm_size - 1) / c.comm_size) * R;
-  c.gather_send.reserve(sizeof(double) * 2 * (size_t)cap);
-  c.gather_recv.reserve(sizeof(double) * 2 * (size_t)cap * c.comm_size);
-  double* send = c.gather_send.as<double>();
-  if (n < cap) {
-    k_fill_nan<<<(unsigned)((2 * cap + 255) / 256), 256, 0, c.stream>>>(send, 2 * cap);
-    CMB_CUDA(cudaGetLastError());
-    c.prof.total_launches += 1;
-  }
-  if (n > 0) {
-    CMB_CUDA(cudaMemcpyAsync(send, c.null.stat.p, sizeof(double) * n, cudaMemcpyDeviceToDevice, c.stream));
-    CMB_CUDA(cudaMemcpyAsync(send + cap, c.null.nmin.p, sizeof(double) * n, cudaMemcpyDeviceToDevice, c.stream));
-  }
-  comm_all_gather(c, send, c.gather_recv.as<double>(), 2 * (size_t)cap);
-  // blocks [stat | nmin] per rank -> two contiguous arrays of comm_size * cap samples
-  const int64_t tot = cap * c.comm_size;
-  c.null.stat.reserve(sizeof(double) * (size_t)tot);
-  c.null.nmin.reserve(sizeof(double) * (size_t)tot);
-  CMB_CUDA(cudaMemcpy2DAsync(c.null.stat.p, sizeof(double) * cap, c.gather_recv.p, sizeof(double) * 2 * cap,
-                             sizeof(double) * cap, c.comm_size, cudaMemcpyDeviceToDevice, c.stream));
-  CMB_CUDA(cudaMemcpy2DAsync(c.null.nmin.p, sizeof(double) * cap, c.gather_recv.as<double>() + cap, sizeof(double) * 2 * cap,
-                             sizeof(double) * cap, c.comm_size, cudaMemcpyDeviceToDevice, c.stream));
-  c.null.n_samples = tot;
-  null_load(c, c.null.stat.as<double>(), c.null.nmin.as<double>(), tot, K, nmax);
+  gather_null_shards(c, rep_cpu, rep_ram, K, nmax);
   CMB_CATCH
 }
 

@@ -160,6 +160,11 @@ void comm_all_gather(Context& c, const double* send, double* recv, size_t count)
 void null_load(Context& c, const double* stat_dev, const double* nmin_dev, int64_t n, int K, double nmax);
 // bytes of device memory one simulated site needs through simulate -> map x2 -> paired
 size_t null_bytes_per_site(const Context& c);
+// This rank's share of rep_cpu outer replicates: contiguous ranges, the first rep_cpu % n_ranks ranks get one more.
+void replicate_range(int rep_cpu, int n_ranks, int rank, int& begin, int& end);
+// The exchange of a sharded null: this rank's c.null samples (its replicate_range) are all-gathered over the
+// communicator in blocks padded with Nmin = NaN, and every rank bins and sorts the union into c.null.
+void gather_null_shards(Context& c, int rep_cpu, int rep_ram, int K, double nmax);
 
 inline void check_stat(int stat_id) {
   if (stat_id < 0 || stat_id > CMB_STAT_MI_LABEL) fail("unknown statistic id %d", stat_id);

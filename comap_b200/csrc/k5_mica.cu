@@ -290,8 +290,13 @@ __global__ void __launch_bounds__(128) k5_listed(int T, int64_t n, const uint8_t
 // word for word in the oracle (orc_mica_permutation_test).
 // The observed and the shuffled MIs come from the same call site, so equal joint tables give equal bits and
 // `rep >= mi` sees the exact ties a discrete statistic produces.
+//
+// A shard (shard_index, shard_count) owns the pairs idx = shard_index + k shard_count, k = 0 .. n_rows - 1: the counter
+// hands out k, the outputs are written at k.  Shuffle q of pair idx depends on (seed, idx, q) only, so a shard's rows
+// are bit for bit the same rows of the whole table (shard_count = 1).
 template <int A, int MIN_CTAS>
-__global__ void __launch_bounds__(128, MIN_CTAS) k5_permutations(int T, int64_t S, int64_t n_pairs, int64_t n_pad,
+__global__ void __launch_bounds__(128, MIN_CTAS) k5_permutations(int T, int64_t S, int64_t n_rows, int shard_index,
+                                                       int shard_count, int64_t n_pad,
                                                        const uint8_t* __restrict__ tips, const uint32_t* __restrict__ cmask,
                                                        uint64_t seed, int max_perm, int use_filter,
                                                        unsigned long long* __restrict__ next, double* __restrict__ pvalue,
@@ -321,8 +326,9 @@ __global__ void __launch_bounds__(128, MIN_CTAS) k5_permutations(int T, int64_t 
     __syncwarp();
     unsigned long long got = 0;
     if (lane == 0) got = atomicAdd(next, 1ull);
-    const int64_t idx = (int64_t)__shfl_sync(ALL, got, 0);
-    if (idx >= n_pairs) break;
+    const int64_t row = (int64_t)__shfl_sync(ALL, got, 0);
+    if (row >= n_rows) break;
+    const int64_t idx = shard_index + row * (int64_t)shard_count;
     // idx = i S - i (i + 1) / 2 + (j - i - 1): row i from the root of the quadratic, then one step either way
     const double b = 2. * (double)S - 1.;
     int64_t i = (int64_t)((b - sqrt(b * b - 8. * (double)idx)) * 0.5);
@@ -346,7 +352,7 @@ __global__ void __launch_bounds__(128, MIN_CTAS) k5_permutations(int T, int64_t 
     lo2 = __reduce_min_sync(ALL, lo2); hi2 = __reduce_max_sync(ALL, hi2);
     amb = __any_sync(ALL, amb);
     if (lo1 >= hi1 || lo2 >= hi2) {              // one character at most (none: lo = 2^32 - 1 > hi = 0)
-      if (lane == 0) { pvalue[idx] = 1.; nperm[idx] = 0; }
+      if (lane == 0) { pvalue[row] = 1.; nperm[row] = 0; }
       continue;
     }
     for (int t = lane; t < T; t += 32) {
@@ -440,7 +446,7 @@ __global__ void __launch_bounds__(128, MIN_CTAS) k5_permutations(int T, int64_t 
       }
       count += c;
     }
-    if (lane == 0) { pvalue[idx] = (double)(count + 1) / (double)(shuffles + 1); nperm[idx] = shuffles; }
+    if (lane == 0) { pvalue[row] = (double)(count + 1) / (double)(shuffles + 1); nperm[row] = shuffles; }
   }
 }
 
@@ -508,11 +514,11 @@ void launch_mica_listed(int A, int T, int64_t n, const uint8_t* t1, int64_t np1,
   CMB_CUDA(cudaGetLastError());
 }
 void launch_mica_permutations(int A, int T, int64_t S, int64_t n_pad, const uint8_t* tips, const uint32_t* cmask, uint64_t seed,
-                              int max_perm, unsigned long long* next, double* pvalue, int32_t* nperm, cudaStream_t st) {
-  if (S < 2) return;
+                              int max_perm, int shard_index, int shard_count, int64_t n_rows, unsigned long long* next,
+                              double* pvalue, int32_t* nperm, cudaStream_t st) {
+  if (S < 2 || n_rows == 0) return;
   if (T < 2) fail("mica permutations: at least two sequences are needed");
   if (T > 65535) fail("mica: %d sequences exceed the 16-bit cells of the joint table", T);
-  const int64_t n_pairs = S * (S - 1) / 2;
   const size_t T4 = ((size_t)T + 3) / 4;
   const size_t q_bytes = ((size_t)(T + 1) * 16 + 15) & ~(size_t)15;
   auto bytes = [&](int nt) { return 1024 + q_bytes + (size_t)(nt / 32) * 8 * T4 + 8 * T4 * nt; };  // masks | c / T, (c / T) ln(c / T) | warps' pairs | private copies
@@ -532,12 +538,13 @@ void launch_mica_permutations(int A, int T, int64_t S, int64_t n_pad, const uint
   CMB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   CMB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, nt, smem));
   if (per_sm < 1) fail("mica permutations: the kernel does not fit an SM (T = %d)", T);
-  // persistent warps, one wave; pairs are handed out by a counter: no more warps than pairs
-  const int64_t ctas = std::min<int64_t>((int64_t)sms * per_sm, (n_pairs + nt / 32 - 1) / (nt / 32));
+  // persistent warps, one wave; the shard's pairs are handed out by a counter: no more warps than pairs
+  const int64_t ctas = std::min<int64_t>((int64_t)sms * per_sm, (n_rows + nt / 32 - 1) / (nt / 32));
   CMB_CUDA(cudaMemsetAsync(next, 0, sizeof(unsigned long long), st));
   // CMB_K5_FILTER=0: every shuffle through the reference's formula (same table; for A/B runs and tests)
   static const int use_filter = [] { const char* e = getenv("CMB_K5_FILTER"); return e ? atoi(e) : 1; }();
-  kernel<<<(unsigned)ctas, nt, smem, st>>>(T, S, n_pairs, n_pad, tips, cmask, seed, max_perm, use_filter, next, pvalue, nperm);
+  kernel<<<(unsigned)ctas, nt, smem, st>>>(T, S, n_rows, shard_index, shard_count, n_pad, tips, cmask, seed, max_perm, use_filter,
+                                           next, pvalue, nperm);
   CMB_CUDA(cudaGetLastError());
 }
 void launch_mica_average(int64_t S, const double* mi, double* avg, cudaStream_t st) {

@@ -93,8 +93,10 @@ void launch_mica_pairs(int A, int T, int64_t S, int64_t n_pad, const uint8_t* ti
 // site a[r] of tip matrix t1 against site b[r] of t2 (a / b nullptr: r itself)
 void launch_mica_listed(int A, int T, int64_t n, const uint8_t* t1, int64_t np1, const uint8_t* t2, int64_t np2, const int32_t* a,
                         const int32_t* b, const uint32_t* cmask, double* mi, double* hj, cudaStream_t st);
+// the pairs idx = shard_index + k shard_count of the upper triangle, k < n_rows, written at k
 void launch_mica_permutations(int A, int T, int64_t S, int64_t n_pad, const uint8_t* tips, const uint32_t* cmask, uint64_t seed,
-                              int max_perm, unsigned long long* next, double* pvalue, int32_t* nperm, cudaStream_t st);
+                              int max_perm, int shard_index, int shard_count, int64_t n_rows, unsigned long long* next,
+                              double* pvalue, int32_t* nperm, cudaStream_t st);
 void launch_mica_average(int64_t S, const double* mi, double* avg, cudaStream_t st);
 void launch_mica_rows(int64_t S, const double* entropy, const double* norm, int32_t* oi, int32_t* oj, double* hmin, double* nmin,
                       cudaStream_t st);

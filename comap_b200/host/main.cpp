@@ -471,25 +471,49 @@ int mica_main(Inputs& in, const char* argv0) {
   if (S < 2) throw Error("at least two sites are needed");
   uint64_t seed = in.app.seed;
   if (!in.app.seed_given) seed = ((uint64_t)std::random_device{}() << 32) ^ std::random_device{}();
-  cmb_ctx* ctx = nullptr;
-  chk(cmb_ctx_create(-1, nullptr, &ctx));
-  chk(cmb_set_tree(ctx, (int32_t)in.tree.parent.size(), in.tree.parent.data(), in.tree.brlen.data()));
+  // a context on `device` (-1: the current one) holding the tree, the model and the alignment
+  auto load = [&](int device) {
+    cmb_ctx* c = nullptr;
+    chk(cmb_ctx_create(device, nullptr, &c));
+    chk(cmb_set_tree(c, (int32_t)in.tree.parent.size(), in.tree.parent.data(), in.tree.brlen.data()));
+    if (with_model) { // Mica.cpp:303-339: likelihood, then the mapping (Uniformization, total counts) for the norms
+      chk(cmb_set_model(c, in.model.A, in.model.Q.data(), in.model.pi.data(), (int32_t)in.rdist.rates.size(),
+                        in.rdist.rates.data(), in.rdist.probs.data(), CMB_COUNT_UNIFORMIZATION, nullptr));
+    } else { // the library wants a model before it takes an alignment; a uniform one, never used
+      const int A = (int)in.alpha.states.size();
+      std::vector<double> Q((size_t)A * A, 1. / (A - 1)), pi(A, 1. / A);
+      for (int x = 0; x < A; x++) Q[(size_t)x * A + x] = -1.;
+      const double one = 1.;
+      chk(cmb_set_model(c, A, Q.data(), pi.data(), 1, &one, &one, CMB_COUNT_NAIVE, nullptr));
+    }
+    chk(cmb_set_alignment(c, S, in.codes.data(), (int32_t)in.code_mask.size(), in.code_mask.data()));
+    return c;
+  };
+  cmb_ctx* ctx = load(-1);
   std::vector<double> norms;
-  if (with_model) { // Mica.cpp:303-339: likelihood, then the mapping (Uniformization, total counts) for the norms
-    chk(cmb_set_model(ctx, in.model.A, in.model.Q.data(), in.model.pi.data(), (int32_t)in.rdist.rates.size(),
-                      in.rdist.rates.data(), in.rdist.probs.data(), CMB_COUNT_UNIFORMIZATION, nullptr));
-  } else { // the library wants a model before it takes an alignment; a uniform one, never used
-    const int A = (int)in.alpha.states.size();
-    std::vector<double> Q((size_t)A * A, 1. / (A - 1)), pi(A, 1. / A);
-    for (int x = 0; x < A; x++) Q[(size_t)x * A + x] = -1.;
-    const double one = 1.;
-    chk(cmb_set_model(ctx, A, Q.data(), pi.data(), 1, &one, &one, CMB_COUNT_NAIVE, nullptr));
-  }
-  chk(cmb_set_alignment(ctx, S, in.codes.data(), (int32_t)in.code_mask.size(), in.code_mask.data()));
   if (with_model) {
     norms.resize(S);
     chk(cmb_map(ctx, nullptr, norms.data(), nullptr, nullptr, nullptr));
   }
+  // comap_b200.gpus = N: the permutation test's pairs and the parametric bootstrap's replicates are spread over
+  // contexts on devices 0..N-1 holding the same tree, model and alignment; the other null methods build their samples
+  // on the host and, like the table, stay on context 0
+  const int n_gpus = (int)get_int(P, "comap_b200.gpus", 1);
+  if (n_gpus < 1) throw Error("comap_b200.gpus must be at least 1");
+  const std::string method = get_string(P, "null.method", "none");
+  const bool parametric = method == "parametric-bootstrap";
+  std::vector<cmb_ctx*> ctxs{ctx};
+  if (n_gpus > 1 && (method == "permutations" || (parametric && with_model))) {
+    display_result("GPUs", n_gpus);
+    ctxs.resize(n_gpus, nullptr);
+    on_all(n_gpus, [&](int r) {
+      if (r == 0) return;
+      ctxs[r] = load(r);
+      if (parametric) chk(cmb_map(ctxs[r], nullptr, nullptr, nullptr, nullptr, nullptr));
+    });
+    if (parametric) chk(cmb_comm_init_all(ctxs.data(), n_gpus));
+  }
+  const int n_dev = (int)ctxs.size();
   const std::string path = get_path(P, "output.file", "none");
   if (path == "none") throw Error("output.file is not set");
   display_result("Output file", path);
@@ -506,7 +530,6 @@ int mica_main(Inputs& in, const char* argv0) {
   const int key = with_model ? CMB_MICA_KEY_NMIN : CMB_MICA_KEY_HMIN;
 
   // null distribution (Mica.cpp:369-628)
-  const std::string method = get_string(P, "null.method", "none");
   display_result("Null distribution", method);
   bool compute_p = false;
   int64_t max_perm = 0;
@@ -560,13 +583,20 @@ int mica_main(Inputs& in, const char* argv0) {
       display_result("Rate distribution for simulations", continuous_sim ? "continuous" : "discrete");
       if (continuous_sim) {
         if (in.rdist.cont_kind == 0) throw Error("simulations.continuous=yes is available for Constant, Gamma and Invariant(dist=Gamma) rate distributions");
-        chk(cmb_set_continuous_rates(ctx, in.rdist.cont_kind, in.rdist.alpha, in.rdist.p_inv));
+        for (cmb_ctx* c : ctxs) chk(cmb_set_continuous_rates(c, in.rdist.cont_kind, in.rdist.alpha, in.rdist.p_inv));
       }
       display_message("Computing null distribution............: ");
       const int64_t n = (int64_t)rep_cpu * rep_ram;
       std::vector<double> raw(to_file ? (size_t)n * 3 : 0);
-      chk(cmb_mica_null_parametric(ctx, seed, rep_cpu, rep_ram, get_bool(P, "simulations.weighted_classes", false) ? 1 : 0,
-                                   compute_p ? K : 0, kmax, to_file ? raw.data() : nullptr));
+      const int weighted = get_bool(P, "simulations.weighted_classes", false) ? 1 : 0;
+      if (n_dev == 1)
+        chk(cmb_mica_null_parametric(ctx, seed, rep_cpu, rep_ram, weighted, compute_p ? K : 0, kmax, to_file ? raw.data() : nullptr));
+      else // outer replicates sharded over the GPUs; rank r's rows start at its first replicate
+        on_all(n_dev, [&](int r) {
+          const int q = rep_cpu / n_dev, m = rep_cpu % n_dev, r0 = r * q + std::min(r, m);
+          chk(cmb_mica_null_parametric_sharded(ctxs[r], seed, rep_cpu, rep_ram, weighted, compute_p ? K : 0, kmax,
+                                               to_file ? raw.data() + (size_t)r0 * rep_ram * 3 : nullptr));
+        });
       if (to_file) {
         display_result("Null output file", simpath);
         std::ofstream so(simpath);
@@ -605,7 +635,18 @@ int mica_main(Inputs& in, const char* argv0) {
   std::vector<int32_t> perm_nb;
   if (max_perm > 0) {
     perm_p.resize(n_pairs); perm_nb.resize(n_pairs);
-    chk(cmb_mica_permutations(ctx, seed, (int32_t)std::min<int64_t>(max_perm, INT32_MAX), n_pairs, perm_p.data(), perm_nb.data(), nullptr));
+    const int32_t mp = (int32_t)std::min<int64_t>(max_perm, INT32_MAX);
+    if (n_dev == 1) chk(cmb_mica_permutations(ctx, seed, mp, n_pairs, perm_p.data(), perm_nb.data(), nullptr));
+    else { // GPU r tests the pairs r, r + N, r + 2N, ...; its rows are scattered back into the table's order
+      on_all(n_dev, [&](int r) {
+        const int64_t cap = r < n_pairs ? (n_pairs - 1 - r) / n_dev + 1 : 0;
+        std::vector<double> p(cap);
+        std::vector<int32_t> nb(cap);
+        int64_t got = 0;
+        chk(cmb_mica_permutations_shard(ctxs[r], seed, mp, r, n_dev, cap, p.data(), nb.data(), &got));
+        for (int64_t k = 0; k < got; k++) { perm_p[r + k * n_dev] = p[k]; perm_nb[r + k * n_dev] = nb[k]; }
+      });
+    }
   }
   {
     std::ofstream out(path);
@@ -634,7 +675,7 @@ int mica_main(Inputs& in, const char* argv0) {
       return (int)(q - p);
     });
   }
-  chk(cmb_ctx_destroy(ctx));
+  for (cmb_ctx* c : ctxs) chk(cmb_ctx_destroy(c));
   display_message("\nBye bye ;-)");
   return 0;
 }
@@ -805,6 +846,28 @@ int main(int argc, char** argv) {
           chk(cmb_set_continuous_rates(m2.ctx, in2.rdist.cont_kind, in2.rdist.alpha, in2.rdist.p_inv));
         }
         const int64_t S2 = (int64_t)in2.cols.size();
+        // comap_b200.gpus = N: data set 2 on every GPU too, mapped there (the corrected correlation of the null needs
+        // both observed mean vectors on each GPU); the rectangle of statistics stays on GPU 0
+        std::vector<cmb_ctx*> ctxs2{m2.ctx};
+        if (n_gpus > 1) {
+          if (get_path(P2, "input.vectors.file", "none") != "none")
+            throw Error("comap_b200.gpus > 1 cannot be combined with input.vectors.file2");
+          ctxs2.resize(n_gpus, nullptr);
+          on_all(n_gpus, [&](int r) {
+            if (r == 0) return;
+            chk(cmb_ctx_create(r, nullptr, &ctxs2[r]));
+            chk(cmb_set_tree(ctxs2[r], (int32_t)in2.tree.parent.size(), in2.tree.parent.data(), in2.tree.brlen.data()));
+            chk(cmb_set_model(ctxs2[r], in2.model.A, in2.model.Q.data(), in2.model.pi.data(), (int32_t)in2.rdist.rates.size(),
+                              in2.rdist.rates.data(), in2.rdist.probs.data(), in2.count_method,
+                              in2.weights.empty() ? nullptr : in2.weights.data()));
+            chk(cmb_set_map_mode(ctxs2[r], in2.average, in2.joint));
+            chk(cmb_set_alignment(ctxs2[r], S2, in2.codes.data(), (int32_t)in2.code_mask.size(), in2.code_mask.data()));
+            Procedure st = parse_procedure(get_string(P2, "statistic", "Correlation"));
+            if (st.name == "MI") chk(cmb_set_mi_threshold(ctxs2[r], get_double(st.args, "threshold", 0.99)));
+            if (continuous_sim) chk(cmb_set_continuous_rates(ctxs2[r], in2.rdist.cont_kind, in2.rdist.alpha, in2.rdist.p_inv));
+            chk(cmb_map(ctxs2[r], nullptr, nullptr, nullptr, nullptr, nullptr));
+          });
+        }
         display_message("\n\n-*- Compute statistics -*-\n");
         display_message("Compares data set 1 with data set 2.");
         const bool indep = get_bool(P, "independant_comparisons", false);
@@ -851,7 +914,14 @@ int main(int argc, char** argv) {
           const int rep_ram = (int)get_int(P, "statistic.null.nb_rep_RAM", 1000);
           display_message("Compute statistic under null hypothesis...");
           std::vector<double> raw((size_t)rep_cpu * rep_ram * 4);
-          chk(cmb_null_inter(m1.ctx, m2.ctx, stat_id, seed, rep_cpu, rep_ram, weighted_classes ? 1 : 0, raw.data()));
+          if (n_gpus == 1)
+            chk(cmb_null_inter(m1.ctx, m2.ctx, stat_id, seed, rep_cpu, rep_ram, weighted_classes ? 1 : 0, raw.data()));
+          else // outer replicates in contiguous ranges over the GPUs, each range's rows at its first replicate
+            on_all(n_gpus, [&](int r) {
+              const int q = rep_cpu / n_gpus, m = rep_cpu % n_gpus, r0 = r * q + std::min(r, m), r1 = r0 + q + (r < m ? 1 : 0);
+              chk(cmb_null_inter_range(ctxs[r], ctxs2[r], stat_id, seed, rep_cpu, rep_ram, r0, r1, weighted_classes ? 1 : 0,
+                                       raw.data() + (size_t)r0 * rep_ram * 4));
+            });
           std::ofstream out(null_path);
           out << "Stat\tRCmin\tPRmin\tNmin\n";
           write_rows_parallel(out, (int64_t)rep_cpu * rep_ram, 80, [&](int64_t r, char* p) {
@@ -864,8 +934,8 @@ int main(int argc, char** argv) {
           });
           display_result("Wrote null distribution to", null_path);
         }
-        chk(cmb_ctx_destroy(m2.ctx));
-        chk(cmb_ctx_destroy(ctx));
+        for (cmb_ctx* c : ctxs2) chk(cmb_ctx_destroy(c));
+        for (cmb_ctx* c : ctxs) chk(cmb_ctx_destroy(c));
         double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
         std::cout << "Total execution time: " << secs << "s" << std::endl;
         std::cout << "Bye bye ;-)" << std::endl;

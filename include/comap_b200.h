@@ -258,6 +258,12 @@ int cmb_pairs_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, const cmb_fil
  * draws from the stream keyed seed ^ 0x9E3779B97F4A7C15 at the same site indices. */
 int cmb_null_inter(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed, int32_t rep_cpu,
                    int32_t rep_ram, int32_t weighted_classes, double* raw);
+/* cmb_null_inter over the outer replicates [rep_begin, rep_end) only (one GPU's share of a multi-GPU
+ * run; cmb_null_inter is the range [0, rep_cpu)).  raw is [(rep_end-rep_begin)*rep_ram][4], the rows of
+ * the whole call for those replicates bit for bit: both simulators are keyed by the global site index. */
+int cmb_null_inter_range(cmb_ctx* ctx1, cmb_ctx* ctx2, int32_t stat_id, uint64_t seed, int32_t rep_cpu,
+                         int32_t rep_ram, int32_t rep_begin, int32_t rep_end, int32_t weighted_classes,
+                         double* raw);
 
 /* Candidate groups (analysis=candidates): replaces CandidateGroup::computeStatisticValue /
  * computeNormRanges (CoMap.cpp:663-667; CoETools.h:106-128) and
@@ -324,11 +330,29 @@ int cmb_mica_pair_list(cmb_ctx* ctx, int64_t n, const int32_t* site1, const int3
  * (the same distribution) and is a function of (seed, pair, shuffle number) only -- see DESIGN.md s4 K5. */
 int cmb_mica_permutations(cmb_ctx* ctx, uint64_t seed, int32_t max_permutations, int64_t capacity, double* pvalue, int32_t* nperm,
                           int64_t* n_rows);
+/* One shard of cmb_mica_permutations (one GPU's share of a multi-GPU run; needs no communicator): the pairs
+ * idx = shard_index + k shard_count, k = 0, 1, ... of cmb_mica_pairs' order, row k of the outputs holding pair idx.  Each
+ * row is bit for bit the row idx of cmb_mica_permutations (shard_count = 1).  0 <= shard_index < shard_count; a shard
+ * past the last pair has 0 rows.  The shards interleave so that each gets its part of the pairs that run all their
+ * shuffles, wherever they sit in the table. */
+int cmb_mica_permutations_shard(cmb_ctx* ctx, uint64_t seed, int32_t max_permutations, int32_t shard_index, int32_t shard_count,
+                                int64_t capacity, double* pvalue, int32_t* nperm, int64_t* n_rows);
 /* null.method = parametric-bootstrap (Mica.cpp:470-545): per outer replicate two simulated alignments of rep_ram sites,
  * mapped for their norms (computeSubstitutionVectors), MI of site j with site j, binned by min norm over [0, nmax)
  * (nmax < 0: the mapped alignment's largest norm).  raw: nullable [rep_cpu * rep_ram][3] = MI, Hjoint, Nmin. */
 int cmb_mica_null_parametric(cmb_ctx* ctx, uint64_t seed, int32_t rep_cpu, int32_t rep_ram, int32_t weighted_classes, int32_t K,
                              double nmax, double* raw);
+/* cmb_mica_null_parametric over the outer replicates [rep_begin, rep_end) (cmb_mica_null_parametric is [0, rep_cpu)):
+ * raw holds this range's [(rep_end - rep_begin) * rep_ram][3] rows, and K > 0 bins this range's samples only.  Replicate r
+ * simulates the global sites from 2 r rep_ram, so the ranges concatenate to the whole null. */
+int cmb_mica_null_parametric_range(cmb_ctx* ctx, uint64_t seed, int32_t rep_cpu, int32_t rep_ram, int32_t rep_begin,
+                                   int32_t rep_end, int32_t weighted_classes, int32_t K, double nmax, double* raw);
+/* cmb_mica_null_parametric over the communicator, as cmb_null_intra_sharded: this rank scores its contiguous share of the
+ * replicates (the r0, r1 documented there), the (MI, Nmin) samples are all-gathered, and every rank bins and sorts the
+ * union, so cmb_mica_pairs on any rank sees the single-GPU null.  raw (nullable): the rows of THIS rank's replicates.
+ * K = 0: no binning and no exchange.  Without a communicator it is cmb_mica_null_parametric. */
+int cmb_mica_null_parametric_sharded(cmb_ctx* ctx, uint64_t seed, int32_t rep_cpu, int32_t rep_ram, int32_t weighted_classes,
+                                     int32_t K, double nmax, double* raw);
 /* A null distribution from host arrays -- n statistics and the key they are conditioned on, K bins over [0, kmax) -- for
  * the null methods whose samples the caller builds (Mica.cpp:401-468 nonparametric bootstrap, :546-606 z-score). */
 int cmb_null_load(cmb_ctx* ctx, const double* stat, const double* key, int64_t n, int32_t K, double kmax);
