@@ -9,8 +9,8 @@
 //
 // Layout: the alignment is the tip matrix K1 reads, [T][S_pad] codes with the 256-entry code -> state-mask table.
 // k5_pairs / k5_listed / k5_entropy: one thread per pair (site); T byte loads per column (coalesced over the 32 pairs of
-// a warp, which share site i and walk consecutive sites j), then the table's A^2 cells.  For A <= 4 and no ambiguous
-// character the joint table sits in packed registers, otherwise in local memory (pair_stats below).  Not a tiled
+// a warp, which share site i and walk consecutive sites j), then the table's A^2 cells.  For A <= 4, T <= 65535 and no
+// ambiguous character the joint table sits in packed registers, otherwise in local memory (pair_stats below).  Not a tiled
 // kernel: the work per pair is a histogram, not a dot product.
 // k5_permutations (null.method = permutations, up to 1000 evaluations per pair): one warp per pair, see there.
 #include "kernels.h"
@@ -115,33 +115,36 @@ __device__ __noinline__ void pair_stats_generic(const C1 c1, const C2 c2, int T,
 // A <= 4 and no ambiguous character in either column (almost every pair of a real alignment, every pair of a simulated
 // one): the joint table never leaves the registers.  Counts sit in packed 16-bit fields, one 64-bit word per state of the
 // first column, so no register is indexed by data; integers convert exactly, so the result is bit for bit the generic
-// path's.  A pair that does hold an ambiguous character takes the generic path.
+// path's.  A pair that does hold an ambiguous character takes the generic path, and so does every pair of an alignment of
+// more than 65535 sequences: a cell counts up to T sequences, and a 65536th would carry into the next state's field.
 template <int A, class C1, class C2>
 __device__ __forceinline__ void pair_stats(const C1 c1, const C2 c2, int T, const uint32_t* __restrict__ cmask, double& mi, double& hj) {
   if constexpr (A <= 4) {
-    constexpr uint32_t full = (1u << A) - 1u;
-    unsigned long long w[A];
+    if (T <= 65535) {
+      constexpr uint32_t full = (1u << A) - 1u;
+      unsigned long long w[A];
 #pragma unroll
-    for (int x = 0; x < A; x++) w[x] = 0ull;
-    bool ambiguous = false;
-    for (int t = 0; t < T; t++) {
-      const uint32_t m1 = cmask[c1[t]] & full, m2 = cmask[c2[t]] & full;
-      const int k1 = __popc(m1), k2 = __popc(m2);
-      if (k1 == 1 && k2 == 1) {
-        const unsigned long long inc = 1ull << (16 * (__ffs(m2) - 1));
+      for (int x = 0; x < A; x++) w[x] = 0ull;
+      bool ambiguous = false;
+      for (int t = 0; t < T; t++) {
+        const uint32_t m1 = cmask[c1[t]] & full, m2 = cmask[c2[t]] & full;
+        const int k1 = __popc(m1), k2 = __popc(m2);
+        if (k1 == 1 && k2 == 1) {
+          const unsigned long long inc = 1ull << (16 * (__ffs(m2) - 1));
 #pragma unroll
-        for (int x = 0; x < A; x++) w[x] += (m1 >> x) & 1u ? inc : 0ull;
-      } else if (k1 && k2) ambiguous = true;
-    }
-    if (!ambiguous) {
-      const double n = (double)T;
-      table_stats<A>([&](int x, int y) {
-        unsigned long long r = w[0];
+          for (int x = 0; x < A; x++) w[x] += (m1 >> x) & 1u ? inc : 0ull;
+        } else if (k1 && k2) ambiguous = true;
+      }
+      if (!ambiguous) {
+        const double n = (double)T;
+        table_stats<A>([&](int x, int y) {
+          unsigned long long r = w[0];
 #pragma unroll
-        for (int i = 1; i < A; i++) r = x == i ? w[i] : r;
-        return (double)(unsigned)((r >> (16 * y)) & 0xffffull) / n;
-      }, mi, hj);
-      return;
+          for (int i = 1; i < A; i++) r = x == i ? w[i] : r;
+          return (double)(unsigned)((r >> (16 * y)) & 0xffffull) / n;
+        }, mi, hj);
+        return;
+      }
     }
   }
   pair_stats_generic<A, C1, C2>(c1, c2, T, cmask, mi, hj);

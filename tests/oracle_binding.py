@@ -149,6 +149,17 @@ def mica_permutations(codes, A, code_mask, seed, max_perm):
     return pv, nb, cl
 
 
+def mica_permutation_test(c1, c2, A, code_mask, seed, pair, max_perm):
+    """miTest of one pair of columns with the shuffle stream of pair index `pair` (idx = i S - i (i + 1) / 2 + j - i - 1
+    in mica's order): (MI, p-value, number of shuffles, smallest |shuffled MI - MI|)."""
+    c1 = np.ascontiguousarray(c1, dtype=np.uint8); c2 = np.ascontiguousarray(c2, dtype=np.uint8)
+    m = np.ascontiguousarray(code_mask, dtype=np.uint32)
+    mi, pv, nb, cl = C.c_double(), C.c_double(), C.c_int(), C.c_double()
+    lib().orc_mica_permutation_test(len(c1), _p(c1, C.c_uint8), _p(c2, C.c_uint8), A, len(m), _p(m, C.c_uint32), C.c_uint64(seed),
+                                    C.c_uint64(pair), int(max_perm), C.byref(mi), C.byref(pv), C.byref(nb), C.byref(cl))
+    return mi.value, pv.value, nb.value, cl.value
+
+
 def set_mi_threshold(t):
     lib().orc_set_mi_threshold(C.c_double(t))
 
