@@ -99,6 +99,16 @@ void Context::ensure_streams() {
     OpStream os;
     build_sim_stream(os, tree, tables);
     sim_stream.upload(os, stream);
+    std::vector<int32_t> walk; // the tips in the order k3_simulate writes them: per record child a, then b
+    for (uint32_t r = 0; r < os.n_records; r++) {
+      const int32_t* x = &os.aux[8 * (size_t)r];
+      if (x[0] & kUpTipA) walk.push_back(x[1]);
+      if (x[0] & kUpTipB) walk.push_back(x[2]);
+    }
+    if ((int)walk.size() != tree.n_leaves) fail("internal: the simulation walk reaches %zu of %d leaves", walk.size(), tree.n_leaves);
+    d_leaf_walk.reserve(sizeof(int32_t) * walk.size());
+    CMB_CUDA(cudaMemcpyAsync(d_leaf_walk.p, walk.data(), sizeof(int32_t) * walk.size(), cudaMemcpyHostToDevice, stream));
+    CMB_CUDA(cudaStreamSynchronize(stream));
   }
   {
     std::vector<double> ev, R, L, spec;
@@ -633,15 +643,15 @@ int cmb_profile_get(cmb_ctx* ctx, const char* name, double* ms, int64_t* launche
   ctx->c.prof_collect();
   if (std::string(name) == "sites_simulated" || std::string(name) == "sites_mapped_null") {
     // counters, returned through `ms`: simulated sites handed to the null's mapping since the reset, and how many
-    // of them (varied columns + the A constant patterns per batch) the mapping kernels actually walked
+    // columns the mapping kernels actually walked (the distinct columns of each pattern-compressed batch)
     Context& c = ctx->c;
     double v = (double)c.prof.sites_simulated;
     if (std::string(name) == "sites_mapped_null") {
       if (c.s_batches > 0 && c.s_counts.p) {
-        std::vector<int32_t> h(2 * (size_t)c.s_batches);
+        std::vector<int32_t> h((size_t)c.s_batches);
         CMB_CUDA(cudaMemcpy(h.data(), c.s_counts.p, sizeof(int32_t) * h.size(), cudaMemcpyDeviceToHost));
         v = 0.;
-        for (int k = 0; k < c.s_batches; k++) v += h[2 * k];
+        for (int32_t x : h) v += x;
       }
     }
     if (ms) *ms = v;

@@ -14,7 +14,9 @@ size_t null_bytes_per_site(const Context& c) {
   size_t out = (size_t)c.tree.B * 8 * 2;
   size_t tips = (size_t)c.tree.n_leaves * 2;
   const size_t part = c.protein_mma ? (size_t)c.C * c.tree.B * 8 : 0; // per-class partial outputs of k1_mma20.cu
-  return D + out + tips + part + (size_t)c.C * 8 + 16 * 8;
+  // pattern compression (ColumnKeys): packed tips, hash + column twice over, representative, scan value + sum, s_cols
+  const size_t keys = c.A == 4 ? (size_t)(c.tree.n_leaves + 15) / 16 * 4 + 2 * (8 + 4) + 4 + 2 * 8 + 4 : 0;
+  return D + out + tips + part + keys + (size_t)c.C * 8 + 16 * 8;
 }
 
 void null_load(Context& c, const double* stat_dev, const double* nmin_dev, int64_t n, int K, double nmax) {
@@ -87,6 +89,16 @@ void gather_null_shards(Context& c, int rep_cpu, int rep_ram, int K, double nmax
 
 namespace {
 
+// Pattern compression merges the columns of a pattern only when it occurs at least this often in a batch: every
+// member then reads the pattern's vector out of the band of merged columns instead of its own coalesced column,
+// and k2_paired pays for those scattered reads.  B200, config 4 (one step, 2 000 000 simulated columns):
+//   min run      2      4      8     16     32   (constant columns only: 1 734 385 walked)
+//   walked    1.555  1.558  1.568  1.595  1.644  M columns
+//   K1 ms     33.8   33.7   34.2   34.6   35.9   (37.8)
+//   paired ms  7.8    7.3    6.6    5.5    4.6   (4.3)
+//   step ms   52.4   51.7   51.2   50.9   51.0   (52.5)
+constexpr int kMinMergedRun = 16;
+
 // The two simulated alignments of a batch of outer replicates (AnalysisTools.cpp:591-611) live side by side in
 // ONE set of mapping buffers -- columns [0, n) hold batch 1, [half, half + n) batch 2 -- so one down / up launch
 // pair maps both (twice the CTAs per launch: a 125-replicate shard of an 8-GPU run fills 6.6 waves of the grid
@@ -127,8 +139,9 @@ void null_core(Context& c, int stat_id, uint64_t seed, int rep_cpu, int rep_ram,
     c.clear_sim_tip_padding(n, n_pad);
     const bool dedup_on = !(getenv("CMB_NULL_DEDUP") && atoi(getenv("CMB_NULL_DEDUP")) == 0);
     const bool dedup = dedup_on && c.A == 4 && !c.map_mode; // the variant kernels walk every column
-    int32_t *col_class = nullptr, *col_varied = nullptr;
-    bool classified = false;
+    ColumnKeys keys{};
+    if (dedup) keys = column_key_buffers(T, n, n_pad, c.scratch2);
+    bool keyed = false;
     if (sim1) {
       for (int k = 0; k < 2; k++) {
         const uint8_t* src = k == 0 ? sim1 : sim2;
@@ -137,34 +150,33 @@ void null_core(Context& c, int stat_id, uint64_t seed, int rep_cpu, int rep_ram,
                                      cudaMemcpyHostToDevice, c.stream));
       }
     } else { // both batches in one launch: threads >= n simulate the second alignment's sites into the columns from `half`
-      if (dedup && m.cont_kind == 0) { // the simulator classifies its columns while it writes them
-        compress_class_buffers(n_pad, c.scratch2, &col_class, &col_varied);
-        classified = true;
-      }
+      keyed = dedup && m.cont_kind == 0; // the discrete simulator keys its columns while it writes them
       c.prof_begin("simulate");
       launch_simulate(m, c.sim_stream, seed, 2 * r0 * R, R, 2 * R, 2 * n, n_pad, weighted, c.tree.n_nodes - 1, tips, nullptr,
-                      c.stream, n, half, R, col_class, col_varied);
+                      c.stream, n, half, R, keyed ? &keys : nullptr);
       c.prof_end(1);
     }
-    // Pattern compression (nucleotides): columns whose tips all carry the same state -- 16 % of the simulated
-    // sites of config 4 -- are mapped once per state, as Bio++ maps distinct site patterns and copies
-    // (LegacySubstitutionMappingTools::computeSubstitutionVectors over getNumberOfDistinctSites()).  The varied
-    // columns are packed to the front of a second tip buffer with the A constant patterns behind them, the
-    // mapping kernels stop at the packed count (a device scalar: no host round trip), and the paired statistic
-    // reads each site's vector through a column index.
+    // Pattern compression (nucleotides): identical columns of the batch's two alignments are mapped once, as Bio++
+    // maps distinct site patterns and copies (LegacySubstitutionMappingTools::computeSubstitutionVectors over
+    // getNumberOfDistinctSites()); a column's vector depends only on its tips.  Patterns that occur at least
+    // kMinMergedRun times in the batch are mapped once; one column per pattern is packed into a second tip buffer
+    // (the merged patterns in a band behind the others), the mapping kernels stop at the packed count (a device
+    // scalar: no host round trip), and the paired statistic reads each site's vector through a column index.
     const int32_t *col1 = nullptr, *col2 = nullptr;
     if (dedup) {
       c.s_tips[1].reserve((size_t)T * n_pad);
       c.s_cols.reserve(sizeof(int32_t) * (size_t)n_pad + 256);
-      c.s_counts.reserve(sizeof(int32_t) * 2 * 4096);
+      c.s_counts.reserve(sizeof(int32_t) * 4096);
       if (c.s_batches >= 4096) c.s_batches = 0;
-      int32_t* counts = c.s_counts.as<int32_t>() + 2 * c.s_batches;
+      int32_t* count = c.s_counts.as<int32_t>() + c.s_batches;
+      const char* hb = getenv("CMB_NULL_DEDUP_HASH_BITS"); // tests: a short hash makes the collision path common
+      const char* mr = getenv("CMB_NULL_DEDUP_MIN_RUN"); // tests: 2 merges every repeated column
       c.prof_begin("compress");
-      const int nl = launch_compress_constant(c.A, T, n, half, n_pad, tips, c.s_tips[1].as<uint8_t>(), c.s_cols.as<int32_t>(), counts,
-                                              c.scratch2, c.stream, classified);
+      const int nl = launch_compress_patterns(T, n, half, n_pad, tips, c.d_leaf_walk.as<int32_t>(), keyed, hb ? atoi(hb) : 64,
+                                              mr ? atoi(mr) : kMinMergedRun, keys, c.s_tips[1].as<uint8_t>(), c.s_cols.as<int32_t>(), count, c.stream);
       c.prof_end(nl);
       bb.tips = c.s_tips[1].as<uint8_t>();
-      bb.n_active = counts;
+      bb.n_active = count;
       col1 = c.s_cols.as<int32_t>(); col2 = col1 + half;
       c.s_batches++;
     }

@@ -52,6 +52,7 @@ struct Context {
   // device-resident model + op streams
   DevBuf d_code_mask, d_pi, d_rates, d_probs;
   DevStream down_stream, up_stream, sim_stream;
+  DevBuf d_leaf_walk;            // int32 [T]: alignment row of the j-th leaf the simulation walk reaches (column keys)
   DevStream up_stream_hi; // scalar protein up pass above kScalarUpClasses classes: classes [kScalarUpClasses, C)
   int cont_kind = 0;             // continuous-rate simulation (cmb_set_continuous_rates)
   double cont_alpha = 1., cont_pinv = 0.;
@@ -87,7 +88,7 @@ struct Context {
   // scratch for simulated batches
   DevBuf s_tips[2], s_D, s_Lc, s_invL, s_loglik, s_pr[2], s_rc[2], s_out[2], s_cls;
   DevBuf d_identity_mask;
-  DevBuf s_cols, s_counts;       // pattern compression of simulated batches: column of every site, {sites to map, varied} per batch
+  DevBuf s_cols, s_counts;       // pattern compression of simulated batches: column of every site, columns to map per batch
   int s_batches = 0;
   int64_t null_budget_sites = 0;  // simulated sites the null may hold at once (from free memory, cached)
   const void* s_tips_ptr = nullptr;

@@ -130,6 +130,20 @@ __host__ __device__ __forceinline__ void philox_u01x2(uint64_t seed, uint64_t si
   u1 = (double)((((uint64_t)c[2] << 32) | c[3]) >> 11) * (1.0 / 9007199254740992.0);
 }
 
+// Key of a nucleotide column for the null's pattern compression (k2_pairs.cu launch_compress_patterns): the tips
+// at 2 bits each, 16 to a 32-bit word in the order the simulation walk reaches the leaves, and a 64-bit hash of
+// those words folded in the same order.  k3_simulate and k2_column_keys must produce the same key.
+constexpr uint64_t kColumnHashInit = 0x243F6A8885A308D3ull;
+__device__ __forceinline__ uint64_t column_hash_step(uint64_t h, uint32_t w) {
+  h = (h ^ w) * 0xFF51AFD7ED558CCDull;
+  return h ^ (h >> 32);
+}
+__device__ __forceinline__ uint64_t column_hash_final(uint64_t h) { // MurmurHash3's fmix64
+  h ^= h >> 33; h *= 0xFF51AFD7ED558CCDull;
+  h ^= h >> 33; h *= 0xC4CEB9FE1A85EC53ull;
+  return h ^ (h >> 33);
+}
+
 // Continuous site rate (simulations.continuous = yes; NonHomogeneousSequenceSimulator::enableContinuousRates,
 // CoMap.cpp:209-219 -> rDist->randC()): Gamma(alpha, beta = alpha) by Marsaglia & Tsang's squeeze method with
 // Box-Muller normals, every uniform from the site's Philox stream (node = root, tags 98.. ), so a site's rate

@@ -11,8 +11,10 @@
 //                   = cov/(sd sd) with the unbiased factors kept as the reference has them.
 //  * null binning + per-bin sort (Domain.cpp:113-122, CoETools.cpp:650-652) with CUB radix
 //    sorts (library code, not a hot step: 1e6 keys).
+#include "device_utils.cuh"
 #include "kernels.h"
 #include <cub/cub.cuh>
+#include <cuda/functional>
 #include <cstdlib>
 
 namespace cmb {
@@ -234,50 +236,96 @@ __global__ void k2_raw_rows(int64_t n, const double* stat, const double* nmin, c
 }
 
 // ---------------------------------------------------------------------------- pattern compression
-// state of a column whose tips all agree, else -1; sites outside the two batches: -2 (not mapped at all)
-__global__ void k2_classify_columns(int T, int64_t n, int64_t half, int64_t n_pad, const uint8_t* __restrict__ tips,
-                                    int32_t* __restrict__ cls, int32_t* __restrict__ varied, int classified) {
-  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (s >= n_pad) return;
-  const bool real = s < n || (s >= half && s < half + n);
-  if (real && classified) return; // k3_simulate wrote these while it produced the column
-  int c = -2;
-  if (real) {
-    const uint8_t s0 = tips[s];
-    bool same = true;
+// launch_compress_patterns.  Entry k of the keys belongs to column k of the first batch, or to column half + k - n
+__device__ __forceinline__ int64_t key_column(int64_t k, int64_t n, int64_t half) { return k < n ? k : half + k - n; }
+__device__ __forceinline__ bool batch_column(int64_t s, int64_t n, int64_t half) { return s < n || (s >= half && s < half + n); }
+
+// The key of every column of a batch the simulator did not key (host alignments, continuous rates): the same words
+// and hash as k3_simulate, the rows taken in its walk order (loads coalesced across the warp)
+__global__ void k2_column_keys(int T, int64_t n, int64_t half, int64_t n_pad, const uint8_t* __restrict__ tips,
+                               const int32_t* __restrict__ leaf_rows, uint64_t* __restrict__ hash, int32_t* __restrict__ col,
+                               uint32_t* __restrict__ packed) {
+  const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= 2 * n) return;
+  const int64_t s = key_column(k, n, half);
+  uint64_t h = kColumnHashInit;
+  for (int w = 0; 16 * w < T; w++) {
+    const int m = min(16, T - 16 * w);
+    uint32_t word = 0;
 #pragma unroll 16
-    for (int t = 1; t < T; t++) same &= tips[(size_t)t * n_pad + s] == s0; // independent loads: 16 in flight
-    c = same ? (int)s0 : -1;
+    for (int j = 0; j < m; j++) word |= (uint32_t)tips[(size_t)__ldg(leaf_rows + 16 * w + j) * n_pad + s] << (2 * j);
+    packed[(size_t)w * n_pad + s] = word;
+    h = column_hash_step(h, word);
   }
-  cls[s] = c;
-  varied[s] = c == -1 ? 1 : 0;
+  hash[k] = column_hash_final(h);
+  col[k] = (int32_t)s;
 }
-__global__ void k2_compress_counts(int A, int64_t n_pad, const int32_t* pos, const int32_t* varied, int32_t* counts) {
-  const int32_t nv = pos[n_pad - 1] + varied[n_pad - 1];
-  counts[1] = nv;
-  counts[0] = nv + A;
+// sorted entry i opens a run of equal (masked) hashes: i, else 0 -- a max-scan then gives every entry its run's start
+__global__ void k2_run_starts(int64_t m, const uint64_t* __restrict__ hs, uint64_t mask, int32_t* __restrict__ start) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  start[i] = (i == 0 || ((hs[i] ^ hs[i - 1]) & mask) != 0) ? (int32_t)i : 0;
 }
-__global__ void k2_compact_columns(int A, int T, int64_t n_pad, const uint8_t* __restrict__ tips, const int32_t* __restrict__ cls,
-                                   const int32_t* __restrict__ pos, const int32_t* __restrict__ counts, uint8_t* __restrict__ tips_c,
-                                   int32_t* __restrict__ col) {
+// rep[column] = the column heading its run (the stable sort put the lowest column first), stored as ~head for the
+// head itself; the columns of runs shorter than min_run represent themselves
+__global__ void k2_run_heads(int64_t m, int min_run, const int32_t* __restrict__ run_start, const int32_t* __restrict__ cs,
+                             int32_t* __restrict__ rep) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  const int64_t st = run_start[i];
+  const bool merged = st + min_run - 1 < m && run_start[st + min_run - 1] == st;
+  const int32_t h = cs[st];
+  rep[cs[i]] = !merged ? cs[i] : st == i ? ~h : h;
+}
+// A column joins its run's head only if their packed tips are equal; otherwise it represents itself.  Scan value
+// of a representative: 1 << 32 for the head of a run with other members, 1 for any other.
+__global__ void k2_pick_representatives(int W, int64_t n, int64_t half, int64_t n_pad, const uint32_t* __restrict__ packed,
+                                        int32_t* __restrict__ rep, int64_t* __restrict__ val) {
   const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= n_pad) return;
-  const int32_t nv = counts[1];
-  const int c = cls[s];
-  if (c == -1) {
-    const int32_t d = pos[s];
+  int64_t v = 0;
+  if (batch_column(s, n, half)) {
+    const int32_t h = rep[s];
+    if (h < 0) {
+      rep[s] = ~h;
+      v = (int64_t)1 << 32;
+    } else if (h != s) {
+      bool joins = true;
+#pragma unroll 8
+      for (int w = 0; w < W; w++) joins &= packed[(size_t)w * n_pad + s] == packed[(size_t)w * n_pad + h];
+      if (!joins) { rep[s] = (int32_t)s; v = 1; }
+    } else v = 1;
+  }
+  val[s] = v;
+}
+// packed column of representative r: the columns mapped for themselves alone first, the heads of runs behind them
+__device__ __forceinline__ int32_t packed_column(int64_t r, const int64_t* __restrict__ val, const int64_t* __restrict__ pos,
+                                                 int32_t n_alone) {
+  return val[r] == 1 ? (int32_t)pos[r] : n_alone + (int32_t)(pos[r] >> 32);
+}
+// The heads of merged runs sit together behind the other representatives: k2_paired reads a shared vector for every
+// member, and a narrow band of columns keeps those reads in fewer pages and in L2 (B200, config 4, every repeated
+// column merged: k2_paired 7.8 ms with the band, 10.7 ms with the heads in column order, 4.3 ms uncompressed).
+__global__ void k2_compact_columns(int T, int64_t n, int64_t half, int64_t n_pad, const uint8_t* __restrict__ tips,
+                                   const int32_t* __restrict__ rep, const int64_t* __restrict__ val,
+                                   const int64_t* __restrict__ pos, uint8_t* __restrict__ tips_c, int32_t* __restrict__ col,
+                                   int32_t* __restrict__ count) {
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n_pad) return;
+  const int64_t tot = pos[n_pad - 1] + val[n_pad - 1];
+  const int32_t n_alone = (int32_t)(tot & 0xffffffff), nr = n_alone + (int32_t)(tot >> 32);
+  if (s == 0) *count = nr;
+  if (batch_column(s, n, half)) {
+    const int32_t r = rep[s], d = packed_column(r, val, pos, n_alone);
+    if (r == s) {
 #pragma unroll 16
-    for (int t = 0; t < T; t++) tips_c[(size_t)t * n_pad + d] = tips[(size_t)t * n_pad + s];
-    col[s] = d;
-  } else col[s] = c >= 0 ? nv + c : 0;
-  // the A constant patterns behind the varied columns, then one CTA's worth of valid filler
-  if (s < A + 256) {
-    const int64_t d = (int64_t)nv + s;
-    if (d < n_pad) {
-      const uint8_t v = s < A ? (uint8_t)s : 0;
-      for (int t = 0; t < T; t++) tips_c[(size_t)t * n_pad + d] = v;
+      for (int t = 0; t < T; t++) tips_c[(size_t)t * n_pad + d] = tips[(size_t)t * n_pad + s];
     }
-  }
+    col[s] = d;
+  } else col[s] = 0;
+  // one CTA's worth of valid filler behind the representatives
+  if (s < 256 && nr + s < n_pad)
+    for (int t = 0; t < T; t++) tips_c[(size_t)t * n_pad + nr + s] = 0;
 }
 
 // ---------------------------------------------------------------------------- binning
@@ -830,39 +878,58 @@ void launch_pair_list(int stat_id, double thr, int B, int64_t n_pad, const doubl
   k2_pair_list<<<(unsigned)((n_pairs + 127) / 128), 128, 0, st>>>(stat_id, thr, B, n_pad, out, mv, pairs, n_pairs, stat);
   CMB_CUDA(cudaGetLastError());
 }
-namespace {
-size_t compress_reserve(int64_t n_pad, DevBuf& tmp, size_t* scan_bytes) {
+ColumnKeys column_key_buffers(int T, int64_t n, int64_t n_pad, DevBuf& tmp) {
   if (n_pad > 0x7fffffff) fail("internal: batch too large for 32-bit column indices");
-  size_t need = 0;
-  cub::DeviceScan::ExclusiveSum(nullptr, need, (const int32_t*)nullptr, (int32_t*)nullptr, (int)n_pad, nullptr);
-  const size_t a = align256((size_t)n_pad * 4);
-  tmp.reserve(3 * a + need + 256);
-  *scan_bytes = need;
-  return a;
+  const int m = (int)(2 * n);
+  size_t sort_bytes = 0, max_bytes = 0, sum_bytes = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr, (const int32_t*)nullptr,
+                                  (int32_t*)nullptr, m, 0, 64);
+  cub::DeviceScan::InclusiveScan(nullptr, max_bytes, (const int32_t*)nullptr, (int32_t*)nullptr, cuda::maximum<int32_t>(), m);
+  cub::DeviceScan::ExclusiveSum(nullptr, sum_bytes, (const int64_t*)nullptr, (int64_t*)nullptr, (int)n_pad);
+  const size_t a8 = align256(8 * (size_t)m), a4 = align256(4 * (size_t)m), c4 = align256(4 * (size_t)n_pad);
+  const size_t c8 = align256(8 * (size_t)n_pad);
+  const size_t pk = align256(4 * (size_t)((T + 15) / 16) * n_pad);
+  ColumnKeys k;
+  k.cub_bytes = std::max(sort_bytes, std::max(max_bytes, sum_bytes));
+  tmp.reserve(2 * a8 + 2 * a4 + pk + c4 + 2 * c8 + k.cub_bytes);
+  unsigned char* p = tmp.as<unsigned char>();
+  k.hash = (uint64_t*)p; p += a8;
+  k.hash_sorted = (uint64_t*)p; p += a8;
+  k.col = (int32_t*)p; p += a4;
+  k.col_sorted = (int32_t*)p; p += a4;
+  k.packed = (uint32_t*)p; p += pk;
+  k.rep = (int32_t*)p; p += c4;
+  k.val = (int64_t*)p; p += c8;
+  k.pos = (int64_t*)p; p += c8;
+  k.cub_tmp = p;
+  return k;
 }
-} // namespace
-void compress_class_buffers(int64_t n_pad, DevBuf& tmp, int32_t** col_class, int32_t** col_varied) {
-  size_t need;
-  const size_t a = compress_reserve(n_pad, tmp, &need);
-  *col_class = (int32_t*)tmp.as<unsigned char>();
-  *col_varied = (int32_t*)(tmp.as<unsigned char>() + a);
-}
-int launch_compress_constant(int A, int T, int64_t n, int64_t half, int64_t n_pad, const uint8_t* tips, uint8_t* tips_c,
-                             int32_t* col, int32_t* counts, DevBuf& tmp, cudaStream_t st, bool classified) {
-  size_t need = 0;
-  const size_t a = compress_reserve(n_pad, tmp, &need);
-  unsigned char* base = tmp.as<unsigned char>();
-  int32_t* cls = (int32_t*)base;
-  int32_t* varied = (int32_t*)(base + a);
-  int32_t* pos = (int32_t*)(base + 2 * a);
-  void* ctemp = base + 3 * a;
-  const unsigned g = (unsigned)((n_pad + 255) / 256);
-  k2_classify_columns<<<g, 256, 0, st>>>(T, n, half, n_pad, tips, cls, varied, classified ? 1 : 0);
-  CMB_CUDA(cub::DeviceScan::ExclusiveSum(ctemp, need, varied, pos, (int)n_pad, st));
-  k2_compress_counts<<<1, 1, 0, st>>>(A, n_pad, pos, varied, counts);
-  k2_compact_columns<<<g, 256, 0, st>>>(A, T, n_pad, tips, cls, pos, counts, tips_c, col);
+int launch_compress_patterns(int T, int64_t n, int64_t half, int64_t n_pad, const uint8_t* tips, const int32_t* leaf_rows,
+                             bool keyed, int hash_bits, int min_run, const ColumnKeys& k, uint8_t* tips_c, int32_t* col,
+                             int32_t* count, cudaStream_t st) {
+  if (hash_bits < 1 || hash_bits > 64) fail("internal: %d hash bits", hash_bits);
+  if (min_run < 2) fail("internal: runs of %d columns", min_run);
+  const int64_t m = 2 * n;
+  const unsigned gm = (unsigned)((m + 255) / 256), g = (unsigned)((n_pad + 255) / 256);
+  int nl = 7; // the sort and the scans counted once each
+  if (!keyed) {
+    k2_column_keys<<<gm, 256, 0, st>>>(T, n, half, n_pad, tips, leaf_rows, k.hash, k.col, k.packed);
+    nl++;
+  }
+  size_t bytes = k.cub_bytes;
+  CMB_CUDA(cub::DeviceRadixSort::SortPairs(k.cub_tmp, bytes, k.hash, k.hash_sorted, k.col, k.col_sorted, (int)m, 0, hash_bits, st));
+  int32_t* start = reinterpret_cast<int32_t*>(k.hash); // the unsorted hashes are spent
+  k2_run_starts<<<gm, 256, 0, st>>>(m, k.hash_sorted, hash_bits == 64 ? ~0ull : (1ull << hash_bits) - 1, start);
+  bytes = k.cub_bytes;
+  int32_t* run_start = reinterpret_cast<int32_t*>(k.pos);
+  CMB_CUDA(cub::DeviceScan::InclusiveScan(k.cub_tmp, bytes, start, run_start, cuda::maximum<int32_t>(), (int)m, st));
+  k2_run_heads<<<gm, 256, 0, st>>>(m, min_run, run_start, k.col_sorted, k.rep);
+  k2_pick_representatives<<<g, 256, 0, st>>>((T + 15) / 16, n, half, n_pad, k.packed, k.rep, k.val);
+  bytes = k.cub_bytes;
+  CMB_CUDA(cub::DeviceScan::ExclusiveSum(k.cub_tmp, bytes, k.val, k.pos, (int)n_pad, st));
+  k2_compact_columns<<<g, 256, 0, st>>>(T, n, half, n_pad, tips, k.rep, k.val, k.pos, tips_c, col, count);
   CMB_CUDA(cudaGetLastError());
-  return 4;
+  return nl;
 }
 
 void launch_raw_rows(int64_t n, const double* stat, const double* nmin, const int32_t* rc1, const int32_t* rc2,

@@ -33,9 +33,11 @@ struct SimParams {
   const double *pi, *probs;
   uint8_t* tips;
   int32_t* classes;
-  // pattern compression of the null (k2_pairs.cu launch_compress_constant), fused: per column the state all its tips
-  // share (or -1) and the "varied" flag, written while the column is produced instead of re-read (nullable)
-  int32_t *col_class, *col_varied;
+  // pattern compression of the null (k2_pairs.cu launch_compress_patterns), fused: the column's key, built in
+  // registers while the column is produced instead of re-read from the tip matrix (nullable; A = 4)
+  uint64_t* key_hash;
+  int32_t* key_col;
+  uint32_t* key_packed;
 };
 
 // Philox4x32-10 with the key schedule taken from the launch parameters: the round keys depend on the seed only,
@@ -118,10 +120,21 @@ __global__ void __launch_bounds__(NT) k3_simulate(const __grid_constant__ SimPar
 
   uint8_t stk[kMaxStack];
   int sp = 0;
-  int first = -1;
-  bool same = true;
   uint8_t* const tip_col = p.tips + idx;
   const uint32_t npad32 = (uint32_t)p.n_pad;
+  // column key: 16 tips per word in walk order (every thread counts the same tips: the branches are uniform)
+  const bool keyed = AT == 4 && p.key_hash != nullptr;
+  uint64_t hash = kColumnHashInit;
+  uint32_t word = 0, n_tips = 0;
+  uint32_t* const packed_col = keyed ? p.key_packed + idx : nullptr;
+  auto key_tip = [&](int s) {
+    word |= (uint32_t)s << (2 * (n_tips & 15));
+    if ((++n_tips & 15) == 0) {
+      if (live) packed_col[(uint64_t)(n_tips / 16 - 1) * npad32] = word;
+      hash = column_hash_step(hash, word);
+      word = 0;
+    }
+  };
   const size_t tab = (size_t)C * AA;
   for (uint32_t k = 0; k < p.n_chunks; k++) {
     const unsigned char* rp = cs.wait(k);
@@ -148,13 +161,11 @@ __global__ void __launch_bounds__(NT) k3_simulate(const __grid_constant__ SimPar
       // row * n_pad as one 32 x 32 -> 64 bit multiply (rows and padded site counts are below 2^32)
       if (flags & kUpTipA) {
         if (live) tip_col[(uint64_t)(uint32_t)h0.y * npad32] = (uint8_t)sa;
-        same = same && (first < 0 || sa == first);
-        first = first < 0 ? sa : first;
+        if (keyed) key_tip(sa);
       }
       if (flags & kUpTipB) {
         if (live) tip_col[(uint64_t)(uint32_t)h0.z * npad32] = (uint8_t)sb;
-        same = same && (first < 0 || sb == first);
-        first = first < 0 ? sb : first;
+        if (keyed) key_tip(sb);
       }
       if (flags & kUpTakeA) {
         if (flags & kUpPush) stk[sp++] = (uint8_t)sb;
@@ -164,9 +175,13 @@ __global__ void __launch_bounds__(NT) k3_simulate(const __grid_constant__ SimPar
     }
     cs.release(k);
   }
-  if (live && p.col_class) {
-    p.col_class[idx] = same ? first : -1;
-    p.col_varied[idx] = same ? 0 : 1;
+  if (keyed && live) {
+    if (n_tips & 15) {
+      packed_col[(uint64_t)(n_tips / 16) * npad32] = word;
+      hash = column_hash_step(hash, word);
+    }
+    p.key_hash[tid] = column_hash_final(hash);
+    p.key_col[tid] = (int32_t)idx;
   }
 }
 
@@ -265,7 +280,7 @@ __global__ void __launch_bounds__(NT) k3_simulate_cont(SimParams p, ContParams c
 void launch_simulate(const MapModel& m, const DevStream& s, uint64_t seed, int64_t base, int64_t group,
                      int64_t stride, int64_t n, int64_t n_pad, int weighted, int root_node, uint8_t* tips,
                      int32_t* classes, cudaStream_t st, int64_t half_n, int64_t half_col, int64_t half_shift,
-                     int32_t* col_class, int32_t* col_varied) {
+                     const ColumnKeys* keys) {
   if (n_pad >= ((int64_t)1 << 32)) fail("internal: simulated batch of %lld padded sites", (long long)n_pad);
   SimParams p;
   p.half_n = half_n; p.half_col = half_col; p.half_shift = half_shift;
@@ -278,8 +293,10 @@ void launch_simulate(const MapModel& m, const DevStream& s, uint64_t seed, int64
   }
   p.base = base; p.group = group; p.stride = stride; p.n = n; p.n_pad = n_pad;
   p.pi = m.pi; p.probs = m.probs; p.tips = tips; p.classes = classes;
-  p.col_class = col_class; p.col_varied = col_varied;
-  if (col_class && m.cont_kind != 0) fail("internal: fused column classes need the discrete simulator");
+  p.key_hash = keys ? keys->hash : nullptr;
+  p.key_col = keys ? keys->col : nullptr;
+  p.key_packed = keys ? keys->packed : nullptr;
+  if (keys && (m.cont_kind != 0 || m.A != 4)) fail("internal: fused column keys need the discrete nucleotide simulator");
   size_t smem = 128 + 2 * (size_t)s.cap;
   if (m.cont_kind != 0) {
     if (!m.spec) fail("internal: continuous simulation without the generator's spectrum");

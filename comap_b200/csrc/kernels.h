@@ -80,10 +80,13 @@ __host__ __device__ inline size_t d_chunk(int64_t chunk, int slot, int n_slots, 
 }
 
 // site id of thread idx = base + (idx / group) * stride + idx % group
+// keys (nullable; A = 4, discrete rates): the column keys of the pattern compression (ColumnKeys), written while
+// each column is produced; entry `idx` of keys->hash / keys->col belongs to thread idx
+struct ColumnKeys;
 void launch_simulate(const MapModel& m, const DevStream& s, uint64_t seed, int64_t base, int64_t group,
                      int64_t stride, int64_t n, int64_t n_pad, int weighted, int root_node, uint8_t* tips,
                      int32_t* classes, cudaStream_t st, int64_t half_n = 0, int64_t half_col = 0, int64_t half_shift = 0,
-                     int32_t* col_class = nullptr, int32_t* col_varied = nullptr);
+                     const ColumnKeys* keys = nullptr);
 
 // ---- K5: Mica's column statistics (k5_mica.cu)
 void launch_mica_entropy(int A, int T, int64_t n, int64_t n_pad, const uint8_t* tips, const uint32_t* cmask, double* entropy,
@@ -108,16 +111,34 @@ void launch_min2(int64_t n, const double* a, const double* b, double* out, cudaS
 void launch_paired(int stat_id, double thr, int B, int64_t n, int64_t n_pad, int64_t n_pad2, const double* o1, const double* o2,
                    const double* mv, const double* mv2, double* stat, double* nmin, cudaStream_t st,
                    const int32_t* col1 = nullptr, const int32_t* col2 = nullptr);
-// Pattern compression of a simulated alignment (what Bio++ does through its distinct-site patterns): columns whose
-// tips all carry the same state are mapped ONCE per state.  cls[site] = state or -1 (varied) for the sites of
-// the two batches [0, n) and [half, half + n); tips_c receives the varied columns packed from 0 and the A constant
-// patterns after them; col[site] = where the site's vector will be; counts[0] = sites to map (varied + A),
-// counts[1] = varied sites.  tmp: scan scratch.
-// classified: the simulator already wrote the class / varied flag of every simulated column (compress_class_buffers of
-// the same tmp and n_pad handed to launch_simulate); only the columns outside the two batches are filled in here
-int launch_compress_constant(int A, int T, int64_t n, int64_t half, int64_t n_pad, const uint8_t* tips, uint8_t* tips_c,
-                             int32_t* col, int32_t* counts, DevBuf& tmp, cudaStream_t st, bool classified = false);
-void compress_class_buffers(int64_t n_pad, DevBuf& tmp, int32_t** col_class, int32_t** col_varied);
+// Pattern compression of a simulated nucleotide batch (what Bio++ does through its distinct-site patterns): a set of
+// identical columns among the two batches [0, n) and [half, half + n) is mapped ONCE.  Each of the 2n
+// columns gets a key (device_utils.cuh column_hash_step): packed tips [W][n_pad], W = (T + 15) / 16, and a 64-bit
+// hash; entry k < n of hash / col is column k, entry k >= n column half + k - n.  The rest is scratch of
+// launch_compress_patterns.  column_key_buffers reserves all of it in `tmp` (call it before the simulation
+// that writes the keys; nothing may reserve `tmp` in between).
+struct ColumnKeys {
+  uint64_t *hash, *hash_sorted;  // [2n]
+  int32_t *col, *col_sorted;     // [2n]
+  uint32_t* packed;              // [W][n_pad]
+  int32_t* rep;                  // [n_pad] representative column
+  int64_t *val, *pos;            // [n_pad] scan value of a representative / its exclusive sum (launch_compress_patterns)
+  void* cub_tmp;
+  size_t cub_bytes;
+};
+ColumnKeys column_key_buffers(int T, int64_t n, int64_t n_pad, DevBuf& tmp);
+// keyed: the simulator wrote the keys (launch_simulate's `keys`); else k2_column_keys computes them from `tips`,
+// reading row leaf_rows[j] for the j-th leaf the simulation walk reaches.  Columns are grouped by hash (radix sort of
+// (hash, column): the lowest column heads each run of equal hashes); a column joins its run's head only if their
+// packed tips are equal, so a hash collision costs a lost merge, never a wrong vector.  hash_bits < 64 keeps only
+// the low bits of the hash (tests: makes collisions common).  Runs shorter than min_run (>= 2) are not merged: each
+// of their columns represents itself.  The representatives are packed into tips_c from
+// column 0, in column order: first those mapped for their own column alone, then the heads of runs with other
+// members; 256 columns of valid filler follow.  col[site] = packed column of the site's representative;
+// *count = representatives (the mapping kernels stop there).  Returns the launches.
+int launch_compress_patterns(int T, int64_t n, int64_t half, int64_t n_pad, const uint8_t* tips, const int32_t* leaf_rows,
+                             bool keyed, int hash_bits, int min_run, const ColumnKeys& k, uint8_t* tips_c, int32_t* col,
+                             int32_t* count, cudaStream_t st);
 // statistic of listed column pairs of one [B][n_pad] matrix (candidate-group statistics)
 void launch_pair_list(int stat_id, double thr, int B, int64_t n_pad, const double* out, const double* mv, const int2* pairs,
                       int64_t n_pairs, double* stat, cudaStream_t st);
