@@ -665,8 +665,7 @@ int cmb_cluster_null(cmb_ctx* ctx, int32_t dist_id, int32_t linkage, uint64_t se
   size_t held = 0;
   for (int q = 0; q < 4; q++) held += c.cn_dists[q].cap + c.cn_outs[q].cap + c.cn_works[q].cap;
   const size_t per_rep = sizeof(double) * ((size_t)S * S + (size_t)B * S_pad) + ((size_t)64 << 20);
-  int NB = (int)std::min<size_t>(4, std::max<size_t>(1, (size_t)(0.6 * (double)(free_b + held)) / per_rep));
-  if (const char* e = std::getenv("CMB_K4_BATCH")) NB = std::max(1, std::min(4, atoi(e)));
+  const int NB = (int)std::min<size_t>(4, std::max<size_t>(1, (size_t)(0.6 * (double)(free_b + held)) / per_rep));
   DevBuf *dists = c.cn_dists, *works = c.cn_works, *outs = c.cn_outs;
   std::vector<double> h_norms[4];
   DendroHost dendro[4];

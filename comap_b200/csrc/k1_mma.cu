@@ -27,7 +27,6 @@
 // chunk (C * 4 KB) into the stage ring.  Measured on B200 at config 4 (517 k sites): down 4.2 ms
 // (5.1 TB/s of stores), up 10.8 ms.
 #include <algorithm>
-#include <cstdlib>
 #include <type_traits>
 #include "device_utils.cuh"
 #include "kernels.h"
@@ -405,7 +404,6 @@ bool try_up_mma(const MapModel& m, const MapBuffers& b, const DevStream& s, cuda
   stage = (stage + 127) & ~size_t(127);
   const size_t fixed = 128;
   if ((size_t)max_smem < fixed + 2 * stage) return false;
-  static const int stage_cap = getenv("CMB_UP_STAGES") ? atoi(getenv("CMB_UP_STAGES")) : kMaxStages;
   UpMmaParams up;
   up.stream = s.bytes.as<unsigned char>();
   up.rec_off = s.off.as<uint32_t>();
@@ -413,17 +411,15 @@ bool try_up_mma(const MapModel& m, const MapBuffers& b, const DevStream& s, cuda
   up.refs = s.aux.as<int4>();
   up.n_nodes = s.n_records;
   up.stage_bytes = (uint32_t)stage;
-  up.n_stages = (int)std::min<size_t>(std::min(kMaxStages, stage_cap), ((size_t)max_smem - fixed) / stage);
+  up.n_stages = (int)std::min<size_t>(kMaxStages, ((size_t)max_smem - fixed) / stage);
   // Shared memory is carved out of the 256 KB it shares with L1, and the consumers' message stack and
   // register spills live in local memory behind that L1: a third stage at C = 4 (2 x 111 KB of shared
   // memory, ~28 KB of L1) ran 41 ms per step instead of 33.  Keep a CTA's ring within 80 KB.
-  static const size_t ring_kb = getenv("CMB_UP_RING_KB") ? (size_t)atoi(getenv("CMB_UP_RING_KB")) : 80;
-  if (MINB > 1) up.n_stages = (int)std::max<size_t>(2, std::min<size_t>(up.n_stages, (ring_kb * 1024) / stage));
+  constexpr size_t kRingBytes = 80 * 1024;
+  if (MINB > 1) up.n_stages = (int)std::max<size_t>(2, std::min<size_t>(up.n_stages, kRingBytes / stage));
   const size_t smem = fixed + (size_t)up.n_stages * stage;
   constexpr int threads = 32 * (SG / (8 * NG) + 1);
   CMB_CUDA(cudaFuncSetAttribute(k1_up_mma<NG, C, SG, MINB, STATES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  if (getenv("CMB_UP_CARVEOUT"))
-    CMB_CUDA(cudaFuncSetAttribute(k1_up_mma<NG, C, SG, MINB, STATES>, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(getenv("CMB_UP_CARVEOUT"))));
   k1_up_mma<NG, C, SG, MINB, STATES><<<(unsigned)(b.n_pad / SG), threads, smem, st>>>(m, b, up);
   CMB_CUDA(cudaGetLastError());
   return true;
@@ -437,8 +433,6 @@ bool narrow_batch(const MapBuffers& b) {
     CMB_CUDA(cudaGetDevice(&dev));
     CMB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   }
-  static const int force = getenv("CMB_K1_NARROW") ? atoi(getenv("CMB_K1_NARROW")) : -1; // experiment switch
-  if (force >= 0) return force != 0;
   return b.n_pad / kWideSG < sms;
 }
 
@@ -451,11 +445,8 @@ bool up_mma_for(const MapModel& m, const MapBuffers& b, const DevStream& s, cuda
     if (m.states_only ? try_up_mma<2, C, kNarrowSG, 2, true>(m, b, s, st) : try_up_mma<2, C, kNarrowSG, 2, false>(m, b, s, st)) return true;
   }
   // device-simulated batches: 64-site CTAs, three per SM (12 consumer warps at 128 registers, a 3-stage ring each):
-  // 26.6 ms per config-4 step against 27.7 for 128-site CTAs x 2 (CMB_UP_SG=128 selects those)
-  {
-    static const int sg = getenv("CMB_UP_SG") ? atoi(getenv("CMB_UP_SG")) : 64; // experiment switch
-    if (m.states_only && sg == 64 && try_up_mma<2, C, 64, 3, true>(m, b, s, st)) return true;
-  }
+  // 26.6 ms per config-4 step against 27.7 for 128-site CTAs x 2
+  if (m.states_only && try_up_mma<2, C, 64, 3, true>(m, b, s, st)) return true;
   if (m.states_only) return try_up_mma<2, C, kWideSG, 2, true>(m, b, s, st) || try_up_mma<2, C, kWideSG, 1, true>(m, b, s, st);
   return try_up_mma<2, C, kWideSG, 2, false>(m, b, s, st) || try_up_mma<2, C, kWideSG, 1, false>(m, b, s, st);
 }

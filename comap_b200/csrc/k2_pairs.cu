@@ -561,98 +561,6 @@ __device__ __forceinline__ void pair_epilogue(const TileParams& p, int64_t ri, i
   }
 }
 
-// Opt-in tensor-core flavour of the correlation / covariance / cosinus Gram tiles (CMB_K2_DMMA=1): the same
-// 64 x 64 tile, centred in the tile load, accumulated by DMMA m8n8k4 (warp = 32 x 16 outputs = 4 x 2 MMA tiles,
-// 8 DMMAs per 4 branches).  It is NOT the default: the tensor core fuses and reorders the sums, so given the
-// same vectors the statistics differ from the reference's summation order in the last bits and the p-value
-// counts of tied pairs move (measured in DESIGN.md s4, K2), while the tile kernel is 6 % of the step.
-__device__ __forceinline__ void dmma_acc(double& d0, double& d1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
-}
-template <int STAT>
-__global__ void __launch_bounds__(256) k2_tiles_dmma(TileParams p) {
-  constexpr int LD = TS + 4;                     // row stride = 4 mod 16 doubles: conflict-free fragment loads
-  __shared__ __align__(16) double As[BK][LD];
-  __shared__ __align__(16) double Bs[BK][LD];
-  const int2 t = p.tiles[blockIdx.x];
-  const int64_t i0 = (int64_t)t.x * TS, j0 = (int64_t)t.y * TS;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int r0 = (warp >> 2) * 32, c0 = (warp & 3) * 16;   // warp tile
-  const int lk = tid >> 4, lc = (tid & 15) * 4;
-  int64_t ai[4], bj[4];
-  double am[4], bm[4];
-#pragma unroll
-  for (int u = 0; u < 4; u++) {
-    int64_t ri = i0 + lc + u;
-    ai[u] = ri < p.n_rows ? (p.rows ? p.rows[ri] : ri) : -1;
-    int64_t cj = j0 + lc + u;
-    bj[u] = cj < p.S2 ? cj : -1;
-    am[u] = ai[u] >= 0 ? p.mean[ai[u]] : 0.;
-    bm[u] = bj[u] >= 0 ? p.mean2[bj[u]] : 0.;
-  }
-  double acc[4][2][2];
-#pragma unroll
-  for (int mi = 0; mi < 4; mi++)
-#pragma unroll
-    for (int ni = 0; ni < 2; ni++) acc[mi][ni][0] = acc[mi][ni][1] = 0.;
-  for (int k0 = 0; k0 < p.B; k0 += BK) {
-    const int k = k0 + lk;
-    const double* rowp = p.out + (size_t)k * p.S_pad;
-    const double* colp = p.out2 + (size_t)k * p.S2_pad;
-    const double mvk = (STAT == 0 && p.mv && k < p.B) ? p.mv[k] : 0.;
-    const double mvk2 = (STAT == 0 && p.mv && k < p.B) ? p.mv2[k] : 0.;
-#pragma unroll
-    for (int u = 0; u < 4; u++) {
-      double a = 0., b = 0.;
-      if (k < p.B) {
-        if (STAT == 0 && p.mv) {
-          if (ai[u] >= 0) a = tile_load<STAT>(add_(rowp[ai[u]], -mvk), am[u]);
-          if (bj[u] >= 0) b = tile_load<STAT>(add_(colp[bj[u]], -mvk2), bm[u]);
-        } else {
-          if (ai[u] >= 0) a = tile_load<STAT>(rowp[ai[u]], am[u], p.thr);
-          if (bj[u] >= 0) b = tile_load<STAT>(colp[bj[u]], bm[u], p.thr);
-        }
-      }
-      As[lk][lc + u] = a;
-      Bs[lk][lc + u] = b;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int ks = 0; ks < BK / 4; ks++) {
-      double af[4], bf[2];
-#pragma unroll
-      for (int mi = 0; mi < 4; mi++) af[mi] = As[ks * 4 + (lane & 3)][r0 + 8 * mi + (lane >> 2)];
-#pragma unroll
-      for (int ni = 0; ni < 2; ni++) bf[ni] = Bs[ks * 4 + (lane & 3)][c0 + 8 * ni + (lane >> 2)];
-#pragma unroll
-      for (int mi = 0; mi < 4; mi++)
-#pragma unroll
-        for (int ni = 0; ni < 2; ni++) dmma_acc(acc[mi][ni][0], acc[mi][ni][1], af[mi], bf[ni]);
-    }
-    __syncthreads();
-  }
-#pragma unroll
-  for (int mi = 0; mi < 4; mi++) {
-    const int64_t ri = i0 + r0 + 8 * mi + (lane >> 2);
-    if (ri >= p.n_rows) continue;
-    const int64_t i = p.rows ? p.rows[ri] : ri;
-#pragma unroll
-    for (int ni = 0; ni < 2; ni++)
-#pragma unroll
-      for (int h = 0; h < 2; h++) {
-        const int64_t j = j0 + c0 + 8 * ni + (lane & 3) * 2 + h;
-        if (j >= p.S2 || (p.mode != MODE_RECT && j <= i)) continue;
-        pair_epilogue<STAT>(p, ri, i, j, acc[mi][ni][h]);
-      }
-  }
-  if (p.mode == MODE_DIST && t.x == t.y) { // zero diagonal
-    for (int d = tid; d < TS; d += blockDim.x) {
-      int64_t i = i0 + d;
-      if (i < p.S) p.mat[(size_t)i * p.S + i] = 0.;
-    }
-  }
-}
-
 template <int STAT>
 __global__ void __launch_bounds__(256) k2_tiles(TileParams p) {
   __shared__ __align__(16) double stage[2][BK][TS];
@@ -1009,14 +917,6 @@ int launch_tiles(const TilesLaunch& L, cudaStream_t st) {
   p.dist_is_stat = L.dist_is_stat;
   if (L.n_tiles == 0) return 0;
   unsigned g = (unsigned)L.n_tiles;
-  const char* dm = getenv("CMB_K2_DMMA"); // opt-in tensor-core Gram tiles (not bit-exact with the reference's summation order)
-  if (dm && atoi(dm) && L.stat_id <= 2) {
-    if (L.stat_id == 0) k2_tiles_dmma<0><<<g, 256, 0, st>>>(p);
-    else if (L.stat_id == 1) k2_tiles_dmma<1><<<g, 256, 0, st>>>(p);
-    else k2_tiles_dmma<2><<<g, 256, 0, st>>>(p);
-    CMB_CUDA(cudaGetLastError());
-    return 1;
-  }
   switch (L.stat_id) {
     case 0: k2_tiles<0><<<g, 256, 0, st>>>(p); break;
     case 1: k2_tiles<1><<<g, 256, 0, st>>>(p); break;

@@ -14,8 +14,6 @@
 // in the common case -- with the reference's tie-breaking preserved exactly.
 #include "kernels.h"
 #include <algorithm>
-#include <cstdlib>
-#include <string>
 #include <cooperative_groups.h>
 
 namespace cg = cooperative_groups;
@@ -122,8 +120,8 @@ __global__ void __launch_bounds__(CT) k4_init_rows(ClusterParams p) {
 // cached minimum pointed at a or b for a rescan, and reduces the new row a's own minimum on the
 // fly (per-CTA partial); grid sync; (B) bookkeeping, row a's minimum from the partials, rescans;
 // grid sync.  ncu / clock64 on config 5 (S = 20 000) before this layout: 73 us per merge, of
-// which 21 us in (1) and 47 us in serial rescans of row a and ~40 queued rows.  Now (-DCMB_K4_TIMING,
-// cycles per merge on a mid-grid CTA): scan 3300 | barrier 2800 | combine 3400 | update 1400 |
+// which 21 us in (1) and 47 us in serial rescans of row a and ~40 queued rows.  Now (cycles per
+// merge on a mid-grid CTA): scan 3300 | barrier 2800 | combine 3400 | update 1400 |
 // barrier 6400 (waits for CTA 0's 4000) | rescans 2800 (slowest CTA 8200) | barrier 10000.  A barrier
 // costs ~2500 cycles and a round trip to data another SM has just written ~1000, whatever the grid
 // size (16..148 CTAs measured the same).  A two-barrier variant that rescans a queued row inside the
@@ -179,16 +177,7 @@ __global__ void __launch_bounds__(CT) k4_cluster(const __grid_constant__ Cluster
   const int G = (int)gridDim.x;
   const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, gsz = (int64_t)G * blockDim.x;
   const int64_t per = (S + G - 1) / G, lo = (int64_t)blockIdx.x * per, hi = lo + per < S ? lo + per : S;
-#ifdef CMB_K4_TIMING
-  long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, t0 = 0, t1 = 0;
-#define K4_T(slot) { t1 = clock64(); tacc[slot] += t1 - t0; t0 = t1; }
-#else
-#define K4_T(slot)
-#endif
   for (int64_t step = 0; step + 2 < S; step++) {
-#ifdef CMB_K4_TIMING
-    t0 = clock64();
-#endif
     // (1) first global minimum of the cached row minima: every CTA scans its slice (the loads of
     //     all problems are issued together), publishes (value, row, column), grid barrier, then all
     //     CTAs reduce the per-CTA partials
@@ -220,9 +209,7 @@ __global__ void __launch_bounds__(CT) k4_cluster(const __grid_constant__ Cluster
       if (threadIdx.x == 0) { B.p[q].scan_val[blockIdx.x] = b[q].v; B.p[q].scan_idx[blockIdx.x] = b[q].i; }
       if (my_i[q] >= 0 && my_i[q] == b[q].i) B.p[q].scan_col[blockIdx.x] = my_col[q]; // a row belongs to one thread
     }
-    K4_T(0)
     grid.sync();
-    K4_T(1)
     // the column travels with the partial, so no load depends on the reduced row index
     {
       int pi0[NP], pc0[NP]; double pv0[NP];
@@ -268,7 +255,6 @@ __global__ void __launch_bounds__(CT) k4_cluster(const __grid_constant__ Cluster
         w1[q] = na / (na + nb); w2[q] = nb / (na + nb); w4[q] = 0.;
       }
     }
-    K4_T(2)
     // (A) new distances to the merged cluster (slot a).  After the barrier the cached minimum of row k is
     //     read and written by the thread that owns k only, so a row that only sees a new column compares in
     //     place; rows whose minimum pointed at a or bb are queued; the new row a's own minimum is reduced on
@@ -322,9 +308,7 @@ __global__ void __launch_bounds__(CT) k4_cluster(const __grid_constant__ Cluster
 #pragma unroll
       for (int q = 0; q < NP; q++) { B.p[q].part_val[blockIdx.x] = ra[q].v; B.p[q].part_idx[blockIdx.x] = ra[q].i; }
     }
-    K4_T(3)
     grid.sync();
-    K4_T(4)
     // (B) bookkeeping and row a's cached minimum from the per-CTA partials (block 0), queued rescans
     int n_wl[NP], n_all = 0;
 #pragma unroll
@@ -421,15 +405,8 @@ __global__ void __launch_bounds__(CT) k4_cluster(const __grid_constant__ Cluster
       }
       __syncthreads();
     }
-    K4_T(5)
     grid.sync();
-    K4_T(6)
   }
-#ifdef CMB_K4_TIMING
-  if (threadIdx.x == 0 && (blockIdx.x == 0 || blockIdx.x == 77 || blockIdx.x == gridDim.x - 1))
-    printf("k4 timing cta %d: scan %lld sync1 %lld combine %lld update %lld sync2 %lld rescans %lld sync3 %lld (cycles per step of %d merges)\n",
-           blockIdx.x, tacc[0] / (S - 2), tacc[1] / (S - 2), tacc[2] / (S - 2), tacc[3] / (S - 2), tacc[4] / (S - 2), tacc[5] / (S - 2), tacc[6] / (S - 2), NP);
-#endif
   // finalStep: join the last two clusters at d/2
   if (gtid < NP) {
     const ClusterParams& p = B.p[gtid];
@@ -441,260 +418,6 @@ __global__ void __launch_bounds__(CT) k4_cluster(const __grid_constant__ Cluster
     p.right[S - 2] = p.node[i2];
     p.height[S - 2] = p.len[i1] + (d - p.len[i1]);
   }
-}
-
-// ---- the same merge loop inside ONE thread-block cluster ----------------------------------
-// A grid barrier costs ~2500 cycles and every exchange through global memory ~1000 more; a merge
-// has three of each.  Sixteen CTAs of one cluster hold the cached row minima in their shared memory
-// (slice r of the rows in CTA r), exchange partial minima and the rescan queue with remote
-// shared-memory stores and meet at cluster barriers; only the matrix itself stays in HBM / L2.
-// Per merge: (P1) slice argmin -> partial to every CTA; barrier; (P2) every CTA reduces the 16
-// partials, updates row / column a for the rows of its slice (cached minima local), sends its
-// partial of the new row a to that row's owner and its queued rows to everybody; barrier; (P3) queued
-// rows are dealt round-robin, each rescanned by one CTA, result stored into the owner's cache;
-// barrier.  Measured (S = 20 000, cycles per merge): slice argmin 2100 | barrier 1100 | reduce 1250 | update 3600 |
-// publish 2700 | barrier 1500+ | rescans up to 13 000 on the CTAs that hold a row | barrier: 16 us per merge.
-// Splitting every queued row over the 16 CTAs (as the grid kernel does) is the missing step; until then the
-// grid kernel is the default and this one is selected with CMB_K4_LAYOUT=cluster.
-constexpr int NC = 16, NT = 1024, QMAX = 8;
-
-struct DsmLayout {
-  int per; size_t o_rv, o_pv, o_rav, o_ri, o_pi, o_pc, o_rai, o_rn, o_rl, o_ovf, o_alive, bytes;
-  __host__ __device__ explicit DsmLayout(int64_t S) {
-    per = (int)((S + NC - 1) / NC);
-    size_t o = 0;
-    o_rv = o; o += 8 * (size_t)per; o_pv = o; o += 8 * NC; o_rav = o; o += 8 * NC;
-    o_ri = o; o += 4 * (size_t)per; o_pi = o; o += 4 * NC; o_pc = o; o += 4 * NC; o_rai = o; o += 4 * NC;
-    o_rn = o; o += 4 * NC; o_rl = o; o += 4 * NC * QMAX; o_ovf = o; o += 4 * (size_t)per;
-    o_alive = o; o += (size_t)S; bytes = (o + 15) & ~size_t(15);
-  }
-};
-
-__device__ Best scan_row_dsm(const double* __restrict__ row, const uint8_t* alive_s, int r, int64_t S, Best* sh) {
-  constexpr int U = 10; // 10 240 columns per batch of loads
-  Best b{0., -1};
-  for (int64_t base = r + 1; base < S; base += (int64_t)NT * U) {
-    double v[U];
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-      const int64_t j = base + (int64_t)u * NT + threadIdx.x;
-      v[u] = j < S ? row[j] : 0.;
-    }
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-      const int64_t j = base + (int64_t)u * NT + threadIdx.x;
-      if (j < S && alive_s[j] && !(v[u] != v[u]) && better(v[u], (int)j, b)) { b.v = v[u]; b.i = (int)j; }
-    }
-  }
-  return block_best(b, sh);
-}
-
-__global__ void __launch_bounds__(NT, 1) k4_cluster_dsm(ClusterParams p) {
-  cg::cluster_group cluster = cg::this_cluster();
-  const int rank = (int)cluster.block_rank(), tid = (int)threadIdx.x;
-  extern __shared__ __align__(16) unsigned char dsm[];
-  __shared__ Best sh[32];
-  __shared__ int sh_col, sh_a, sh_bb, rs_n, sh_ntot, sh_list[NC * QMAX], rs_loc[QMAX];
-  __shared__ double sh_d;
-  const int64_t S = p.S;
-  const DsmLayout L(S);
-  const int per = L.per, lo = rank * per, hi = (int)((int64_t)lo + per < S ? lo + per : S);
-  double* rv = (double*)(dsm + L.o_rv); double* pv = (double*)(dsm + L.o_pv); double* rav = (double*)(dsm + L.o_rav);
-  int* ri = (int*)(dsm + L.o_ri); int* pi = (int*)(dsm + L.o_pi); int* pc = (int*)(dsm + L.o_pc);
-  int* rai = (int*)(dsm + L.o_rai); int* rn = (int*)(dsm + L.o_rn); int* rl = (int*)(dsm + L.o_rl);
-  int* ovf = (int*)(dsm + L.o_ovf); uint8_t* alive_s = dsm + L.o_alive;
-  for (int i = lo + tid; i < hi; i += NT) { rv[i - lo] = p.rmin_val[i]; ri[i - lo] = p.rmin_idx[i]; }
-  for (int64_t i = tid; i < S; i += NT) alive_s[i] = 1;
-  __syncthreads();
-  cluster.sync(); // every CTA of the cluster is running: remote shared memory may be written
-#ifdef CMB_K4_TIMING
-  long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, t0 = 0, t1 = 0;
-#endif
-  for (int64_t step = 0; step + 2 < S; step++) {
-#ifdef CMB_K4_TIMING
-    t0 = clock64();
-#endif
-    // (P1) first minimum of this CTA's slice of the cached row minima, published to every CTA
-    Best b{0., -1};
-    int my_col = -1;
-    for (int i = lo + tid; i < hi; i += NT) {
-      const int ix = ri[i - lo];
-      const double v = rv[i - lo];
-      if (ix >= 0 && better(v, i, b)) { b.v = v; b.i = i; my_col = ix; }
-    }
-    const int my_i = b.i;
-    b = block_best(b, sh);
-    if (my_i >= 0 && my_i == b.i) sh_col = my_col; // a row belongs to one thread: one writer
-    __syncthreads();
-    if (tid < NC) {
-      cluster.map_shared_rank(pv, tid)[rank] = b.v;
-      cluster.map_shared_rank(pi, tid)[rank] = b.i;
-      cluster.map_shared_rank(pc, tid)[rank] = b.i >= 0 ? sh_col : -1;
-    }
-    K4_T(0)
-    cluster.sync();
-    K4_T(1)
-    // (P2) every CTA reduces the 16 partials
-    if (tid < 32) {
-      Best c{0., -1};
-      int col = -1;
-      if (tid < NC) { c.v = pv[tid]; c.i = pi[tid]; col = pc[tid]; }
-      const Best w = warp_best(c);
-      if (w.i < 0) { if (tid == 0) sh_a = -1; }
-      else if (c.i == w.i) { sh_a = w.i; sh_bb = col; sh_d = w.v; } // rows are unique across the partials
-      if (tid == 0) rs_n = 0;
-    }
-    __syncthreads();
-    const int a = sh_a;
-    if (a < 0) return; // nothing mergeable (NaN distances), the same in every CTA: host reports the error
-    const int bb = sh_bb;
-    const double dab = sh_d;
-    double w1, w2, w4;
-    if (p.linkage == 1) { w1 = .5; w2 = .5; w4 = -.5; }
-    else if (p.linkage == 0) { w1 = .5; w2 = .5; w4 = .5; }
-    else {
-      double na = (double)p.nleaves[a], nb = (double)p.nleaves[bb];
-      w1 = na / (na + nb); w2 = nb / (na + nb); w4 = 0.;
-    }
-    // dendrogram bookkeeping (rank 0, thread 0): loads now, stores in (P3)
-    double len_a = 0.; int node_a = 0, node_b = 0, nl_a = 0, nl_b = 0;
-    if (rank == 0 && tid == 0) { len_a = p.len[a]; node_a = p.node[a]; node_b = p.node[bb]; nl_a = p.nleaves[a]; nl_b = p.nleaves[bb]; }
-    if (tid == 0) alive_s[bb] = 0; // every CTA keeps its own copy of the liveness bytes
-    K4_T(2)
-    Best ra{0., -1}; // first minimum of the new row a over live columns k > a (this slice)
-    for (int k = lo + tid; k < hi; k += NT) {
-      const int kl = k - lo;
-      const uint8_t live = alive_s[k];
-      const double d1 = p.mat[(size_t)a * S + k], d2 = p.mat[(size_t)bb * S + k];
-      const int ci = ri[kl];
-      const double cv = rv[kl];
-      if (k == bb) { ri[kl] = -1; continue; } // dead rows drop out of (P1)
-      if (k == a || !live) continue;
-      // left-to-right, unfused, as the reference's C++ expression evaluates
-      const double nd = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(w1, d1), __dmul_rn(w2, d2)), __dmul_rn(0., dab)),
-                                  __dmul_rn(w4, fabs(__dadd_rn(d1, -d2))));
-      p.mat[(size_t)a * S + k] = nd;
-      p.mat[(size_t)k * S + a] = nd;
-      bool rescan = false;
-      if (k > a) {
-        if (!(nd != nd) && better(nd, k, ra)) { ra.v = nd; ra.i = k; }
-        rescan = k < bb && ci == bb;                                     // lost its minimum's column
-      } else {
-        if (ci == a || ci == bb) rescan = true;                         // minimum pointed at a merged slot
-        else if (!(nd != nd) && (ci < 0 || nd < cv || (nd == cv && a < ci))) { rv[kl] = nd; ri[kl] = a; }
-      }
-      if (rescan) {
-        const int q = atomicAdd(&rs_n, 1);
-        if (q < QMAX) rs_loc[q] = k; else ovf[q - QMAX] = k;
-      }
-    }
-    K4_T(3)
-    ra = block_best(ra, sh); // its barriers also publish the queue and this CTA's column-a stores to the CTA
-    const int n_found = rs_n, n_q = n_found < QMAX ? n_found : QMAX;
-    if (tid == 0) {
-      const int oa = a / per;
-      cluster.map_shared_rank(rav, oa)[rank] = ra.v;
-      cluster.map_shared_rank(rai, oa)[rank] = ra.i;
-    }
-    if (tid < NC) {
-      cluster.map_shared_rank(rn, tid)[rank] = n_q;
-      int* dst = cluster.map_shared_rank(rl, tid) + rank * QMAX;
-      for (int q = 0; q < n_q; q++) dst[q] = rs_loc[q];
-    }
-    // more than QMAX queued rows in one slice (rare): rescanned here; row k changes only in column a,
-    // which this CTA has just written
-    for (int q = QMAX; q < n_found; q++) {
-      __syncthreads();
-      const int r = ovf[q - QMAX];
-      const Best t = scan_row_dsm(p.mat + (size_t)r * S, alive_s, r, S, sh);
-      if (tid == 0) { rv[r - lo] = t.v; ri[r - lo] = t.i; }
-    }
-    K4_T(4)
-    cluster.sync();
-    K4_T(5)
-    // (P3) row a's minimum at its owner, queued rows dealt round-robin, bookkeeping
-    if (a / per == rank && tid < 32) {
-      Best c{0., -1};
-      if (tid < NC) { c.v = rav[tid]; c.i = rai[tid]; }
-      c = warp_best(c);
-      if (tid == 0) { rv[a - lo] = c.v; ri[a - lo] = c.i; }
-    }
-    if (tid < NC * QMAX) {
-      const int src = tid / QMAX, q = tid % QMAX;
-      int pos = q, tot = 0;
-      for (int r2 = 0; r2 < NC; r2++) { const int c = rn[r2]; if (r2 < src) pos += c; tot += c; }
-      if (q < rn[src]) sh_list[pos] = rl[tid];
-      if (tid == 0) sh_ntot = tot;
-    }
-    __syncthreads();
-    const int n_tot = sh_ntot;
-    for (int w = rank; w < n_tot; w += NC) {
-      const int r = sh_list[w];
-      const Best t = scan_row_dsm(p.mat + (size_t)r * S, alive_s, r, S, sh);
-      if (tid == 0) {
-        const int o = r / per;
-        cluster.map_shared_rank(rv, o)[r - o * per] = t.v;
-        cluster.map_shared_rank(ri, o)[r - o * per] = t.i;
-      }
-      __syncthreads();
-    }
-    if (rank == 0 && tid == 0) {
-      const double half = dab / 2.;
-      const double d0 = half - len_a;
-      p.left[step] = node_a;
-      p.right[step] = node_b;
-      p.height[step] = len_a + d0;
-      p.node[a] = (int32_t)(S + step);
-      p.len[a] = len_a + d0;
-      p.nleaves[a] = nl_a + nl_b;
-    }
-    K4_T(6)
-    cluster.sync();
-    K4_T(7)
-  }
-#ifdef CMB_K4_TIMING
-  if (tid == 0 && (rank == 0 || rank == 7 || rank == 15))
-    printf("k4 dsm timing rank %d: scan %lld b1 %lld reduce %lld update %lld publish %lld b2 %lld rescans %lld b3 %lld (cycles per merge)\n",
-           rank, tacc[0] / (S - 2), tacc[1] / (S - 2), tacc[2] / (S - 2), tacc[3] / (S - 2), tacc[4] / (S - 2), tacc[5] / (S - 2), tacc[6] / (S - 2), tacc[7] / (S - 2));
-#endif
-  // finalStep: join the last two clusters at d/2
-  if (rank == 0 && tid == 0) {
-    int i1 = -1, i2 = -1;
-    for (int64_t i = 0; i < S; i++)
-      if (alive_s[i]) { if (i1 < 0) i1 = (int)i; else i2 = (int)i; }
-    const double d = p.mat[(size_t)i1 * S + i2] / 2;
-    p.left[S - 2] = p.node[i1];
-    p.right[S - 2] = p.node[i2];
-    p.height[S - 2] = p.len[i1] + (d - p.len[i1]);
-  }
-}
-
-// launches the cluster kernel when its shared-memory caches fit and the device can place the cluster
-bool try_cluster_dsm(ClusterParams& p, cudaStream_t st) {
-  // opt-in (CMB_K4_LAYOUT=cluster): parity-green, but at S = 20 000 it needs 16 us per merge against 12 us for
-  // the grid kernel -- a queued row is rescanned by ONE CTA (13 000 cycles) while the other 15 wait
-  const char* e = std::getenv("CMB_K4_LAYOUT");
-  if (!e || std::string(e) != "cluster") return false;
-  const DsmLayout L(p.S);
-  if (L.bytes > 200 * 1024) return false;
-  if (cudaFuncSetAttribute(k4_cluster_dsm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.bytes) != cudaSuccess ||
-      cudaFuncSetAttribute(k4_cluster_dsm, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess) {
-    cudaGetLastError();
-    return false;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(NC); cfg.blockDim = dim3(NT); cfg.dynamicSmemBytes = L.bytes; cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = NC; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  cfg.attrs = at; cfg.numAttrs = 1;
-  int n_clusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&n_clusters, k4_cluster_dsm, &cfg) != cudaSuccess || n_clusters < 1) {
-    cudaGetLastError();
-    return false;
-  }
-  CMB_CUDA(cudaLaunchKernelEx(&cfg, k4_cluster_dsm, p));
-  return true;
 }
 
 __global__ void k4_init_state(ClusterParams p) {
@@ -791,7 +514,6 @@ int launch_cluster_batch(int np, int64_t S, int linkage, double* const* mats, De
     CMB_CUDA(cudaGetLastError());
   }
   for (int q = np; q < kMaxBatch; q++) B.p[q] = B.p[0];
-  if (np == 1 && try_cluster_dsm(B.p[0], st)) return 3;
   if (np == 1) launch_batch_kernel<1>(B, grid, st);
   else if (np == 2) launch_batch_kernel<2>(B, grid, st);
   else if (np == 3) launch_batch_kernel<3>(B, grid, st);

@@ -62,7 +62,7 @@ struct RnnParams {
   double* seg_v;        // [grid] partial minima of row segments (a stale row may be scanned by several CTAs)
   int32_t *seg_i, *seg_cnt;
   int32_t* counters;    // [0..1] pairs of even / odd rounds, [2..3] stale rows queued for even / odd rounds,
-                        // [4..6] the last two slots and their counter, [8] rounds, [9] error, [10..12] us per phase
+                        // [4..6] the last two slots and their counter, [9] error
   int32_t *m_left, *m_right, *m_i, *m_j; // [S - 1] merge records in creation order
   double *m_height, *m_d;
 };
@@ -163,9 +163,6 @@ __global__ void __launch_bounds__(RT) k4r_rounds(RnnParams p) {
   volatile int32_t* cnt = p.counters;
   int64_t merged = 0;
   int round = 0;
-  unsigned long long t_prev = 0, t_a = 0, t_b = 0, t_c = 0;
-  auto now = [&]() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; };
-  if (gtid == 0) t_prev = now();
   for (; merged < S - 1; round++) {
     const int par = round & 1;
     // ---- (A) first minimum of every stale row over the live columns k != r (NaN entries are skipped)
@@ -218,7 +215,6 @@ __global__ void __launch_bounds__(RT) k4r_rounds(RnnParams p) {
       if (gtid == 0) { cnt[par] = 0; cnt[4] = -1; cnt[5] = -1; cnt[6] = 0; } // this round's pair counter, the last-two slots
     }
     grid.sync();
-    if (gtid == 0) { const unsigned long long t = now(); t_a += t - t_prev; t_prev = t; }
     // ---- (B) reciprocal first minima (i, j), i < j, nn(i) = j and nn(j) = i; per-CTA first global minimum
     const bool last2 = (S - merged) == 2;
     {
@@ -248,7 +244,6 @@ __global__ void __launch_bounds__(RT) k4r_rounds(RnnParams p) {
       if (gtid == 0) cnt[2 + (par ^ 1)] = 0; // the queue the next round scans is filled in (C)
     }
     grid.sync();
-    if (gtid == 0) { const unsigned long long t = now(); t_b += t - t_prev; t_prev = t; }
     // ---- merges of this round: the reciprocal pairs, else the reference's next merge (first global minimum in
     //      (i, j) order), else -- two clusters left -- their join whatever the distance (finalStep upstream)
     int n_pairs = cnt[par];
@@ -347,11 +342,6 @@ __global__ void __launch_bounds__(RT) k4r_rounds(RnnParams p) {
     }
     merged += n_pairs;
     grid.sync();
-    if (gtid == 0) { const unsigned long long t = now(); t_c += t - t_prev; t_prev = t; }
-  }
-  if (gtid == 0) {
-    cnt[8] = round;
-    cnt[10] = (int32_t)(t_a / 1000); cnt[11] = (int32_t)(t_b / 1000); cnt[12] = (int32_t)(t_c / 1000); // us per phase
   }
 }
 
@@ -410,9 +400,6 @@ int launch_cluster_rnn(int64_t S, int linkage, double* mat, DevBuf& work, int32_
     CMB_CUDA(cudaMemsetAsync(left_dev, 0xff, 4 * (S - 1), st));
     return launches;
   }
-  if (getenv("CMB_K4_DEBUG"))
-    fprintf(stderr, "k4 rnn: %d rounds for %lld sites on %d CTAs; us per phase: scan %d, pairs %d, update %d\n", h_cnt[8], (long long)S,
-            grid, h_cnt[10], h_cnt[11], h_cnt[12]);
   // ---- the reference's creation order: children before parents, smallest (distance, i, j) first
   const int64_t M = S - 1;
   std::vector<int32_t> ml(M), mr(M), mi(M), mj(M);

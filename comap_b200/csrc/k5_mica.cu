@@ -297,6 +297,8 @@ __global__ void __launch_bounds__(128) k5_listed(int T, int64_t n, const uint8_t
 // A shard (shard_index, shard_count) owns the pairs idx = shard_index + k shard_count, k = 0 .. n_rows - 1: the counter
 // hands out k, the outputs are written at k.  Shuffle q of pair idx depends on (seed, idx, q) only, so a shard's rows
 // are bit for bit the same rows of the whole table (shard_count = 1).
+// Register budget: MIN_CTAS = 5 CTAs of 128 per SM, 95 registers, nothing spilled (6 and 8 measured: DESIGN.md s4, K5).
+// The budget stays in the template arguments so that the kernel keeps its name, k5_permutations<A, 5>.
 template <int A, int MIN_CTAS>
 __global__ void __launch_bounds__(128, MIN_CTAS) k5_permutations(int T, int64_t S, int64_t n_rows, int shard_index,
                                                        int shard_count, int64_t n_pad,
@@ -529,11 +531,7 @@ void launch_mica_permutations(int A, int T, int64_t S, int64_t n_pad, const uint
   while (nt > 32 && bytes(nt) > 64 * 1024) nt >>= 1;
   const size_t smem = bytes(nt);
   if (smem > 200 * 1024) fail("mica permutations: %d sequences exceed the shared memory of a one-warp CTA", T);
-  // register budget: 5 CTAs of 128 per SM (95 registers, nothing spilled; default), 6 (80) or 8 (64, ~300 B spilled);
-  // CMB_K5_CTAS picks one for A/B runs -- before the interval filter the three measured the same
-  static const int want = [] { const char* e = getenv("CMB_K5_CTAS"); return e ? atoi(e) : 5; }();
-  auto kernel = A == 4 ? (want <= 5 ? k5_permutations<4, 5> : want <= 6 ? k5_permutations<4, 6> : k5_permutations<4, 8>)
-                : A == 20 ? k5_permutations<20, 5> : nullptr;
+  auto kernel = A == 4 ? k5_permutations<4, 5> : A == 20 ? k5_permutations<20, 5> : nullptr;
   if (!kernel) fail("mica kernels are built for A = 4 and A = 20 (got %d)", A);
   CMB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int dev = 0, sms = 0, per_sm = 0;

@@ -45,3 +45,17 @@ def test_product_never_touches_oracle():
             if f.endswith((".py", ".cu", ".cuh", ".cpp", ".h")):
                 txt = open(os.path.join(dp, f)).read()
                 assert "liboracle" not in txt and "comap_oracle" not in txt and "oracle_binding" not in txt, f
+
+
+# Environment switches the library may read: each forces a path production inputs also reach, or gives a test its
+# reference (DESIGN.md s4, "Test switches").  A tuning choice is decided by measurement, not left to a switch.
+TEST_SWITCHES = {"CMB_NULL_DEDUP", "CMB_NULL_DEDUP_HASH_BITS", "CMB_NULL_DEDUP_MIN_RUN", "CMB_K5_FILTER",
+                 "CMB_K4_ALGO", "CMB_K1_PROTEIN", "CMB_DOWN_GLOBAL_TIPS"}
+
+
+def test_library_reads_only_the_test_switches():
+    csrc = os.path.join(ROOT, "comap_b200", "csrc")
+    read = set()
+    for f in os.listdir(csrc):
+        read |= set(re.findall(r'getenv\("(CMB_\w+)"\)', open(os.path.join(csrc, f)).read()))
+    assert read == TEST_SWITCHES

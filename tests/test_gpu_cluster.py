@@ -95,18 +95,6 @@ def test_cluster_tiny_alignments(ctx, S):
         assert np.array_equal(gr["stat"], og["stat"])
 
 
-@pytest.mark.parametrize("linkage", ["complete", "single", "average"])
-def test_cluster_dsmem_layout_equals_oracle(ctx, linkage, monkeypatch):
-    """The opt-in 16-CTA thread-block-cluster kernel (CMB_K4_LAYOUT=cluster, cached minima in
-    distributed shared memory) gives the same dendrogram as the oracle, ties included."""
-    monkeypatch.setenv("CMB_K4_LAYOUT", "cluster")
-    c, r = _setup(ctx, T=24, S=700, seed=31)
-    mat = ctx.distance_matrix("correlation")
-    left, right, height = ctx.cluster(linkage)
-    ol, orr, oh = O.hclust(linkage, mat)
-    assert np.array_equal(left, ol) and np.array_equal(right, orr) and np.array_equal(height, oh)
-
-
 @pytest.mark.parametrize("linkage", ["complete", "average"])
 @pytest.mark.parametrize("keep_constant", [False, True])
 def test_cluster_reciprocal_rounds_vs_oracle(ctx, linkage, keep_constant, monkeypatch):

@@ -10,10 +10,7 @@ import contextlib
 import json
 import os
 import re
-import subprocess
-import sys
 import tempfile
-import textwrap
 
 import numpy as np
 import pytest
@@ -22,11 +19,10 @@ from comap_b200 import synthetic as syn
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-9
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 # ------------------------------------------------------------------------------------------ kernel recorder
 _K1 = re.compile(r"\b(k1_\w+?)(<[^()]*>)?\(")
-SEEN = set()          # every K1 instance this module launched (subprocesses included)
+SEEN = set()          # every K1 instance this module launched
 
 
 def instance_of(kernel_name):
@@ -464,69 +460,6 @@ def test_protein_scalar_kernels(ctx, monkeypatch, C):
     assert not rec.instances("k1_up<") and not rec.instances("k1_down<"), rec
 
 
-# ------------------------------------------------------------------------------------------ switches read once
-SWITCH_SCRIPT = textwrap.dedent("""
-    import json, sys
-    import numpy as np
-    sys.path[:0] = [{root!r}, {tests!r}]
-    import test_gpu_k1_shapes as K
-    from comap_b200 import api, synthetic as syn
-    out = sys.argv[1]
-    ctx = api.Context()
-    m = K.dna_model(*syn.random_tree(20, 1618, 0.08), 4)
-    K.set_model(ctx, m)
-    codes = K.with_ambiguity(ctx.simulate(21, 0, K.narrow_max() + 1)[0], 0.02, 5)
-    res, launches = {{}}, {{}}
-    for case, cols in (("wide", codes), ("narrow", codes[:, :5000])):
-        ctx.set_alignment(np.ascontiguousarray(cols), K.DNA_MASK)
-        with K.recorded() as rec:
-            r = ctx.map()
-        launches[case] = rec
-        res.update({{case + "_" + k: v for k, v in r.items()}})
-    with K.recorded() as rec:
-        res["null"] = ctx.null_intra("correlation", 11, 4, 2500, K=10, nmax=40.0, want_raw=True)
-    launches["null"] = rec
-    ctx.close()
-    np.savez(out + ".npz", **res)
-    json.dump({{k: list(v) for k, v in launches.items()}}, open(out + ".json", "w"))
-""")
-
-SWITCHES = {"default": {}, "narrow1": {"CMB_K1_NARROW": "1"}, "narrow0": {"CMB_K1_NARROW": "0"},
-            "up_sg128": {"CMB_UP_SG": "128"}, "up_stages2": {"CMB_UP_STAGES": "2"}, "ring40": {"CMB_UP_RING_KB": "40"}}
-
-
-def test_switches_read_once_per_process_leave_results_unchanged(tmp_path):
-    """CMB_K1_NARROW, CMB_UP_SG, CMB_UP_STAGES and CMB_UP_RING_KB are read into statics on first use, so each
-    setting runs in a fresh process: the same wide and narrow mappings and wide device null, bit for bit, while
-    the recorder shows the instance or ring size each switch changes."""
-    script = tmp_path / "run.py"
-    script.write_text(SWITCH_SCRIPT.format(root=ROOT, tests=os.path.join(ROOT, "tests")))
-    res, logs = {}, {}
-    for name, extra in SWITCHES.items():
-        env = {k: v for k, v in os.environ.items() if not k.startswith("CMB_")}
-        env.update(extra)
-        p = subprocess.run([sys.executable, str(script), str(tmp_path / name)], env=env, cwd=str(tmp_path),
-                           capture_output=True, text=True, timeout=300)
-        assert p.returncode == 0, p.stderr[-3000:]
-        res[name] = dict(np.load(tmp_path / (name + ".npz")))
-        logs[name] = {k: Launches(tuple(x) for x in v) for k, v in json.load(open(tmp_path / (name + ".json"))).items()}
-        SEEN.update(*[v.instances() for v in logs[name].values()])
-    for name in SWITCHES:
-        for k, v in res["default"].items():
-            assert np.array_equal(res[name][k], v, equal_nan=True), (name, k)
-    d = logs["default"]
-    assert d["wide"].args("k1_up_mma") == {(2, 4, 128, 2, False)} and d["narrow"].args("k1_up_mma") == {(2, 4, 32, 2, False)}
-    assert d["null"].args("k1_up_mma") == {(2, 4, 64, 3, True)} and d["null"].args("k1_down_mma") == {(2, 4, 128, 2, True)}
-    for case in ("wide", "null"):
-        assert {a[2] for a in logs["narrow1"][case].args("k1_up_mma") | logs["narrow1"][case].args("k1_down_mma")} == {32}
-    assert logs["narrow0"]["narrow"].args("k1_up_mma") == {(2, 4, 128, 2, False)}
-    assert logs["narrow0"]["narrow"].args("k1_down_mma") == {(2, 4, 128, 2, False)}
-    assert logs["up_sg128"]["null"].args("k1_up_mma") == {(2, 4, 128, 2, True)}
-    for name, case in (("up_stages2", "narrow"), ("up_stages2", "null"), ("ring40", "null")):
-        assert logs[name][case].args("k1_up_mma") == d[case].args("k1_up_mma")
-        assert max(logs[name][case].smem("k1_up_mma")) < min(d[case].smem("k1_up_mma")), (name, case)
-
-
 # ------------------------------------------------------------------------------------------ coverage
 def all_instances():
     """Every K1 instance the launchers can select (k1_mma.cu, k1_mma20.cu, k1_map.cu)."""
@@ -559,14 +492,13 @@ def _not_run():
         for C in range(1, 7):
             out["k1_up_mma<2,%d,128,1,%s>" % (C, st)] = (
                 "the largest up stage at C <= 6 (two stored 128-site chunks, 55 KB) fits two stages at MINB=2")
-    for C in range(1, 9):
-        if C != 4:
-            out["k1_up_mma<2,%d,128,2,true>" % C] = ("device-simulated batches take the 64-site up pass unless "
-                                                     "CMB_UP_SG=128; the switch test runs that at C = 4")
+    for C in range(1, 8):
+        out["k1_up_mma<2,%d,128,2,true>" % C] = ("device-simulated batches take the 64-site, 3-CTA up pass, "
+                                                 "which always fits at C <= 7")
     out["k1_up_mma<2,8,128,2,true>"] = ("C = 8 and a tree with two stored children: neither 64/3 nor 128/2 "
                                         "fits; without such nodes the 64-site pass fits")
-    out["k1_up_mma<2,7,128,1,true>"] = ("C = 7: the 64-site, 3-CTA up pass always fits (36 KB stages); only "
-                                        "CMB_UP_SG=128 reaches this one")
+    out["k1_up_mma<2,7,128,1,true>"] = ("C = 7: the 64-site, 3-CTA up pass always fits (36 KB stages), so no "
+                                        "batch falls back to this one")
     for st in ("false", "true"):
         out["k1_up_mma20<1,%s>" % st] = ("the protein up stage (44 KB: one class, two stored 64-site chunks) "
                                          "always fits two stages at MINB=2")

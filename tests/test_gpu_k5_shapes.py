@@ -1,13 +1,13 @@
 """Every launch shape of Mica's kernels (K5) against the CPU oracle.
 
 The permutation launcher picks its CTA width and dynamic shared memory from the number of sequences T, and the kernel
-draws one or two shuffle indices per generator word depending on T; CMB_K5_CTAS picks the register budget of the A = 4
-instance.  Each permutation test here records, with torch.profiler, the instance, CTA width and shared memory of the
-launch, asserts them against a Python restatement of launch_mica_permutations, and compares Perm.p.value / Perm.nb of
-every pair with the oracle's replay of the same shuffle stream.  The table kernels (k5_entropy, k5_pairs, k5_average,
-k5_rows, k5_listed) are compared at the edges of their grids and above 65535 sequences, where the packed 16-bit joint
-table of pair_stats no longer holds a cell.  The last test checks that the file ran every instance the launchers can
-select, except those listed in NOT_RUN with the reason they are not reached."""
+draws one or two shuffle indices per generator word depending on T. Each permutation test here records, with
+torch.profiler, the instance, CTA width and shared memory of the launch, asserts them against a Python restatement of
+launch_mica_permutations, and compares Perm.p.value / Perm.nb of every pair with the oracle's replay of the same
+shuffle stream. The table kernels (k5_entropy, k5_pairs, k5_average, k5_rows, k5_listed) are compared at the edges of
+their grids and above 65535 sequences, where the packed 16-bit joint table of pair_stats no longer holds a cell. The
+last test checks that the file ran every instance the launchers can select, except those listed in NOT_RUN with the
+reason they are not reached."""
 import json
 import math
 import os
@@ -145,11 +145,9 @@ def perm_shape(T):
     return None if size(nt) > SMEM_CAP else (nt, size(nt))
 
 
-def perm_instance(A, ctas=5):
-    """CMB_K5_CTAS (read once per process) picks the A = 4 register budget; A = 20 has one instance."""
-    if A == 20:
-        return "k5_permutations<20,5>"
-    return "k5_permutations<4,%d>" % (5 if ctas <= 5 else 6 if ctas <= 6 else 8)
+def perm_instance(A):
+    """One permutation instance per alphabet, at the register budget of 5 CTAs per SM."""
+    return "k5_permutations<%d,5>" % A
 
 
 def pair_index(i, j, S):
@@ -488,18 +486,17 @@ SWITCH_SCRIPT = textwrap.dedent("""
     json.dump(launches, open(out + ".json", "w"))
 """)
 SWITCH_T = (100, 300, 600)
-SWITCHES = {"default": ({}, 5), "ctas6": ({"CMB_K5_CTAS": "6"}, 6), "ctas8": ({"CMB_K5_CTAS": "8"}, 8),
-            "filter0": ({"CMB_K5_FILTER": "0"}, 5)}
+SWITCHES = {"default": {}, "filter0": {"CMB_K5_FILTER": "0"}}
 
 
 def test_switches_read_once_per_process_leave_results_unchanged(tmp_path):
-    """CMB_K5_CTAS=6 / 8 (the <4,6> and <4,8> instances) and CMB_K5_FILTER=0 (every shuffle through the reference's
-    formula) are read into statics on first use, so each runs in a fresh process at T = 100, 300 and 600 (CTA widths
-    128, 64, 32): the same table bit for bit, with the instance each setting selects."""
+    """CMB_K5_FILTER=0 (every shuffle through the reference's formula) is read into a static on first use, so each
+    setting runs in a fresh process at T = 100, 300 and 600 (CTA widths 128, 64, 32): the same table bit for bit, from
+    the same instance."""
     script = tmp_path / "run.py"
     script.write_text(SWITCH_SCRIPT.format(root=ROOT, tests=os.path.join(ROOT, "tests")))
     res = {}
-    for name, (extra, ctas) in SWITCHES.items():
+    for name, extra in SWITCHES.items():
         env = {k: v for k, v in os.environ.items() if not k.startswith("CMB_")}
         env.update(extra)
         p = subprocess.run([sys.executable, str(script), str(tmp_path / name)], env=env, cwd=str(tmp_path),
@@ -509,7 +506,7 @@ def test_switches_read_once_per_process_leave_results_unchanged(tmp_path):
         logs = json.load(open(tmp_path / (name + ".json")))
         for T in SWITCH_T:
             rec = Launches(tuple(x) for x in logs[str(T)])
-            assert rec.shapes("k5_permutations") == {(perm_instance(4, ctas),) + perm_shape(T)}, (name, T, rec)
+            assert rec.shapes("k5_permutations") == {(perm_instance(4),) + perm_shape(T)}, (name, T, rec)
             SEEN.update(rec.keys())
     for name in SWITCHES:
         for k, v in res["default"].items():
@@ -520,10 +517,10 @@ def test_switches_read_once_per_process_leave_results_unchanged(tmp_path):
 # ------------------------------------------------------------------------------------------ coverage
 def all_instances():
     """Every K5 instance the launchers can select (k5_mica.cu), each permutation instance at every CTA width its T
-    range allows (T <= 2484: 128, 64 and 32 for all four)."""
+    range allows (T <= 2484: 128, 64 and 32 for both)."""
     out = {"k5_%s<%d>" % (k, A) for k in ("entropy", "pairs", "listed") for A in (4, 20)}
     out |= {"k5_average", "k5_rows", "k5_min2"}
-    for inst in ("k5_permutations<4,5>", "k5_permutations<4,6>", "k5_permutations<4,8>", "k5_permutations<20,5>"):
+    for inst in ("k5_permutations<4,5>", "k5_permutations<20,5>"):
         out |= {"%s@%d" % (inst, w) for w in (128, 64, 32)}
     return out
 

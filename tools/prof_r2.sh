@@ -22,7 +22,4 @@ done
 python tools/k4dbg.py > $O/${T}_k4_plain.log 2>&1 || exit 1
 ncu --set full --clock-control none --import-source on -k regex:k4r_rounds -c 1 -f -o $O/${T}_k4r_rounds python tools/k4dbg.py > $O/${T}_ncu_k4r.log 2>&1
 summ ${T}_k4r_rounds
-python tools/k2_dmma_eval.py > $O/${T}_k2_dmma_eval.json 2> $O/${T}_k2_dmma_eval.err
-CMB_K2_DMMA=1 ncu --set full --clock-control none -k regex:k2_tiles_dmma -s 2 -c 1 -f -o $O/${T}_k2_tiles_dmma $SS > $O/${T}_ncu_k2_tiles_dmma.log 2>&1
-summ ${T}_k2_tiles_dmma
 tail -c 300 $O/${T}_plain.log

@@ -6,7 +6,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OBJ = os.path.join(ROOT, "comap_b200", "build")
 WANT = [("k1_mma.cu.o", r"k1_up_mmaILi2ELi4ELi128ELi2ELb1E"), ("k1_mma.cu.o", r"k1_down_mmaILi2ELi4ELi128ELi2E"),
         ("k1_mma.cu.o", r"k1_up_mmaILi2ELi4ELi32ELi2ELb0E"), ("k1_mma20.cu.o", r"k1_up_mma20ILi2ELb1E"),
-        ("k1_mma20.cu.o", r"k1_down_mma20ILi2ELb1E"), ("k2_pairs.cu.o", r"k2_tilesILi0E"), ("k2_pairs.cu.o", r"k2_tiles_dmmaILi0E"),
+        ("k1_mma20.cu.o", r"k1_down_mma20ILi2ELb1E"), ("k2_pairs.cu.o", r"k2_tilesILi0E"),
         ("k2_pairs.cu.o", r"k2_pairedILi0E"), ("k3_simulate.cu.o", r"k3_simulate"), ("k4_rnn.cu.o", r"k4r_rounds"),
         ("k4_cluster.cu.o", r"k4_clusterILi1E"), ("k5_mica.cu.o", r"k5_permutationsILi4ELi5E"), ("k5_mica.cu.o", r"k5_pairsILi4E"),
         ("k5_mica.cu.o", r"k5_pairsILi20E")]
